@@ -5,17 +5,18 @@ Our arm (default)
   step      ONE launch of the fused env-step kernel over one batch of `--envs` environments per GPU (default 65,536 =
             BASELINE configs[1], "batched fixed-wing physics step only, random actions"): 8 physics substeps at 240 Hz per
             env, actions drawn in-kernel from Philox, motor noise on, auto-reset on ground/dome.
-  value     envs * n_gpus / (device time of one step).  A timed REGION is the K-launch CUDA graph sequence replayed R times
-            so that it lasts >= 50 ms on the device (`timed_launches` = R*K per region); 5 regions, median; CUDA events are
-            recorded in the enqueue order behind a warm launch, so host launch latency is outside the region; MAX over
-            ranks.  (K = 20 launches alone are 0.4 ms -- a window in which host jitter, not the GPU, sets the number.)
+  value     envs * n_gpus / (device time of one step).  The timed region is exactly `--steps` launches (a CUDA graph
+            sequence), after `--warmup` untimed ones and one untimed call that builds the graphs of the timed call; its CUDA
+            events are recorded in the enqueue order behind a warm launch, so host launch latency is outside the region;
+            MAX over ranks.  Ask for enough steps that the region lasts tens of milliseconds (`ms_per_step` shows the
+            length of one): a shorter window measures the clock as much as the kernel.
   L2        the per-batch state (~7 MB) would sit in the 126 MB L2 between launches, so the loop rotates over enough
             independent env batches that the working set exceeds 2x L2 ("l2" in config).  The launches of the graph are
             chained by programmatic dependent launch edges: consecutive launches step different batches, so the next one
             places its blocks while the previous one drains (its tail otherwise idles 54 % of the schedulers).
   e2e       the same metric through the reference-facing host call FixedwingVecEnv.step_arrays(actions) (VecEnv.step seam;
             C ABI fw_step_host) on the Fixedwing-Waypoints-v3 task with HOST buffers: H2D of the actions and D2H of
-            obs/reward/flags inside the timed region (wall clock, >= 50 ms regions, median of 5).
+            obs/reward/flags inside the timed region (wall clock over `--steps` steps after `--warmup` untimed ones).
   roofline  dominant kernel fw_step_kernel.  `bound` names the pipe that binds it -- FP32 issue (SURVEY 8d: 6,400 flop per
             physics env-step against an FMA-chain peak measured in the same run); the HBM view (152 algorithmic bytes per
             env-step against MEASURED_PEAKS.json) rides along as `roofline.hbm`.
@@ -24,6 +25,12 @@ Our arm (default)
             A (n_steps 2048, batch 128: 65,536 optimiser steps per epoch) -- and configs[3], Waypoint-ObjLock at 65,536
             envs/GPU, n_steps 64.
   cpu_baseline  the fp64 oracle (kind "port") on the host cores, bounded sample, rank 0 at N=1 only.
+  --dump-outputs DIR  what the timed steps computed, rank 0's, as DIR/<name>.npy (float32; float64 and integer data as float64):
+            step_<field> = state of the env batch the last timed launch stepped, e2e_obs / e2e_reward / e2e_flags = what the
+            last e2e step returned, ppo_<workload>_theta / _obs_rms = policy parameters and observation moments after each
+            PPO measurement.  Per-env rows are a seeded sample (env_index.npy) when all of them would pass 64 MB.  Every
+            input is seeded and every step count fixed by the command line, so two builds run with the same arguments can
+            be compared output for output.
 
 Reference arm (--impl reference): the reference's CPU path.  PyFlyt/pybullet/SB3 cannot be installed offline and the
 reference has no compilable sources, so this times the oracle port (all host threads) on the workload of our arm's `e2e`
@@ -35,7 +42,6 @@ from __future__ import annotations
 import argparse
 import json
 import os
-import statistics
 import subprocess
 import sys
 import threading
@@ -52,8 +58,7 @@ UNIT = "env-steps/s"
 BYTES_PER_STEP = {"physics_only": 152, "waypoints_v3": 332, "waypoint_objlock": 400, "lowlevel": 276, "objlock_duck": 836}
 FLOPS_PER_STEP = {"physics_only": 6400, "waypoints_v3": 7000, "waypoint_objlock": 7000, "lowlevel": 1750, "objlock_duck": 7000}
 L2_BYTES = 126 * 1024 * 1024
-REGION_MS = 50.0          # minimum device time of one timed region
-N_REGIONS = 5
+DUMP_BYTES = 63 * 10**6   # --dump-outputs: array bytes, leaving room for the .npy headers under 64 MB
 E2E_WORKLOAD = "waypoints_v3"
 # reference's PPO hyper-parameters (train_Fixedwing_Waypoints_v3.py:27-55, train_Fixedwing_Waypoints_ObjLock.py:35-57)
 PPO_HP = dict(learning_rate=3e-4, gamma=0.99, gae_lambda=0.95, clip_range=0.2, ent_coef=0.001, vf_coef=0.5, max_grad_norm=0.5)
@@ -85,7 +90,13 @@ def parse_args():
     ap.add_argument("--steps-per-launch", type=int, default=1,
                     help="env-steps fused into one launch (state kept in registers); a bench step is one launch")
     ap.add_argument("--no-graph", action="store_true", help="issue launches from the host loop instead of a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed steps computed as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what our arm's timed steps computed; the reference arm has none to write")
+    return args
 
 
 def measured_peaks():
@@ -204,7 +215,7 @@ def bench_config(args) -> dict:
                                   "reports the physics-only rate beside it",
             "ppo_workloads": ["configs[2] waypoints_v3 4096 envs/GPU: variant B n_steps 128 x 4 minibatches, variant A n_steps "
                               "2048 / batch 128", "configs[3] waypoint_objlock 65536 envs/GPU n_steps 64 x 4 minibatches"],
-            "timing": f">= {REGION_MS:.0f} ms regions (the K-step sequence replayed), median of {N_REGIONS}"}
+            "timing": f"one region of {args.steps} timed steps after {max(3, args.warmup)} untimed warm-up steps"}
 
 
 # ----------------------------------------------------------------------------------------------------------- CPU arm
@@ -346,6 +357,29 @@ def run_reference(args, rank: int, world: int):
 
 
 # ----------------------------------------------------------------------------------------------------------- our arm
+def dump_outputs(directory: str, per_env: dict, whole: dict) -> None:
+    """Write every array as `directory`/<name>.npy in float32 (float64 for float64 and integer data).  `per_env` arrays
+    have the env index as first axis and share one seeded sample of rows (saved as env_index) when all rows would pass
+    DUMP_BYTES; `whole` arrays are written in full."""
+    import numpy as np
+
+    def wide(a):
+        a = np.asarray(a)
+        return a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    per_env = {k: wide(v) for k, v in per_env.items()}
+    whole = {k: wide(v) for k, v in whole.items()}
+    os.makedirs(directory, exist_ok=True)
+    if per_env:
+        n = len(next(iter(per_env.values())))
+        row_bytes = sum(v[0].nbytes for v in per_env.values()) + 8
+        keep = min(n, (DUMP_BYTES - sum(v.nbytes for v in whole.values())) // row_bytes)
+        rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        whole["env_index"] = rows.astype(np.float64)
+        per_env = {k: v[rows] for k, v in per_env.items()}
+    for name, a in {**per_env, **whole}.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def _max_over_ranks(x: float, world: int) -> float:
     import torch
     import torch.distributed as dist
@@ -357,11 +391,13 @@ def _max_over_ranks(x: float, world: int) -> float:
 
 
 def ppo_measure(preset: str, n_envs: int, n_steps: int, batch_size: int, n_epochs: int, rank: int, local_rank: int,
-                world: int, iters: int = 2, warm: int = 1, epochs_run: int | None = None) -> dict:
+                world: int, iters: int = 2, warm: int = 1, epochs_run: int | None = None, outputs: dict | None = None,
+                name: str = "") -> dict:
     """One PPO workload: `warm` untimed iterations (the second one captures the rollout CUDA graph), then `iters` timed
     iterations of rollout + update between barriers, device-synchronised on both sides, MAX over ranks.  The NCCL
     all-reduce of the 49 KB gradient runs inside the update of every optimiser step when world > 1.
-    epochs_run < n_epochs: the update runs only that many of the n_epochs epochs (variant A's bounded default)."""
+    epochs_run < n_epochs: the update runs only that many of the n_epochs epochs (variant A's bounded default).
+    `outputs`: receives ppo_<name>_theta and ppo_<name>_obs_rms (mean, var, count) as left by the timed iterations."""
     import torch
     import torch.distributed as dist
     from pyflyt_drone_b200.ppo import PPO
@@ -379,6 +415,9 @@ def ppo_measure(preset: str, n_envs: int, n_steps: int, batch_size: int, n_epoch
     model.learn(iters * per_iter)
     torch.cuda.synchronize()
     dt = _max_over_ranks(time.perf_counter() - t0, world)
+    if outputs is not None:
+        outputs[f"ppo_{name}_theta"] = model.policy.theta.detach().float().cpu().numpy()
+        outputs[f"ppo_{name}_obs_rms"] = model.vecnorm.obs_stats.cpu().numpy()
     st = model.stats
     rollout_s = _max_over_ranks(st.rollout_s, world) / iters
     update_s = _max_over_ranks(st.update_s, world) / iters
@@ -475,7 +514,7 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     replicas = max(2, int(np.ceil(2 * L2_BYTES / state_bytes)))
     envs = [FixedwingVecEnv(N, config=cfg, device=local_rank, seed=1234, env_id0=(rank * replicas + r) * N)
             for r in range(replicas)]
-    K, W = max(1, args.steps), max(3, args.warmup)
+    K, W = args.steps, max(3, args.warmup)
     graph = not args.no_graph
     spl = max(1, args.steps_per_launch)
 
@@ -488,37 +527,27 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         return torch.cuda.Event(enable_timing=True)
 
     FixedwingVecEnv.rollout_random(envs, W, spl, use_graph=False)                 # W untimed warm-up steps
-    FixedwingVecEnv.rollout_random(envs, replicas, spl, use_graph=graph)          # builds + instantiates the launch graph
-    # calibrate R: how many times the K-step sequence is replayed so that a region lasts >= REGION_MS on the device
-    c0, c1 = ev(), ev()
-    torch.cuda.synchronize()
-    c0.record()
-    FixedwingVecEnv.rollout_random(envs, K * 4, spl, use_graph=graph)
-    c1.record(); torch.cuda.synchronize()
-    est_ms = max(c0.elapsed_time(c1) / (K * 4), 1e-4)
-    R = max(1, int(np.ceil(REGION_MS * 1.15 / (est_ms * K))))
-    R = int(_max_over_ranks(R, world))
+    FixedwingVecEnv.rollout_random(envs, K, spl, use_graph=graph)                 # builds + instantiates the graphs of K launches
     launches0 = sum(e.launch_count for e in envs)
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    region_ms = []
     barrier()
     if sampler:
         sampler.start()
-    for _ in range(N_REGIONS):
-        e0, e1 = ev(), ev()
-        FixedwingVecEnv.rollout_random(envs, replicas, spl, use_graph=graph)       # warm launch: the GPU is busy ...
-        e0.record()                                                                # ... so the region opens behind it, in enqueue order
-        FixedwingVecEnv.rollout_random(envs, K * R, spl, use_graph=graph)
-        e1.record()
-        barrier()
-        region_ms.append(e0.elapsed_time(e1))
-    clocks = sampler.stop() if sampler else None        # sampled during the timed regions only
+    e0, e1 = ev(), ev()
+    FixedwingVecEnv.rollout_random(envs, replicas, spl, use_graph=graph)           # warm launch: the GPU is busy ...
+    e0.record()                                                                    # ... so the region opens behind it, in enqueue order
+    FixedwingVecEnv.rollout_random(envs, K, spl, use_graph=graph)
+    e1.record()
+    barrier()
+    region_ms = e0.elapsed_time(e1)
+    clocks = sampler.stop() if sampler else None        # sampled during the timed region only
     launches = sum(e.launch_count for e in envs) - launches0
-    med = statistics.median(region_ms)
-    step_ms = _max_over_ranks(med / (K * R), world)      # MAX over ranks of each rank's median
-    best_ms = _max_over_ranks(min(region_ms) / (K * R), world)
+    step_ms = _max_over_ranks(region_ms / K, world)
     value = N * spl * world / (step_ms * 1e-3)
     kernel_ms = step_ms          # back-to-back launches of one kernel: the mean launch-to-launch duration
+    env_outputs, outputs = {}, ({} if args.dump_outputs else None)
+    if args.dump_outputs:        # every call of rollout_random starts at envs[0]: the last timed launch stepped this batch
+        env_outputs = {f"step_{k}": v for k, v in envs[(K - 1) % replicas].get_state().items()}
     for e in envs:
         e.close()
     envs = []
@@ -533,24 +562,20 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     acts = [b.numpy() for b in pinned]
     for a in acts:
         a[:] = rng.uniform(-1, 1, (N, 4)).astype(np.float32)
-    t0 = time.perf_counter()
-    for s in range(8):
+    for s in range(W):
         venv.step_arrays(acts[s % 4], want_terminal_obs=False)
-    e2e_steps = max(8, int(np.ceil(REGION_MS * 1.1e-3 / ((time.perf_counter() - t0) / 8))))
-    e2e_steps = int(_max_over_ranks(e2e_steps, world))
-    e2e_dt = []
-    for _ in range(N_REGIONS):
-        barrier()
-        t0 = time.perf_counter()
-        for s in range(e2e_steps):
-            venv.step_arrays(acts[s % 4], want_terminal_obs=False)
-        torch.cuda.synchronize()
-        e2e_dt.append(time.perf_counter() - t0)
-    e2e_step_s = _max_over_ranks(statistics.median(e2e_dt) / e2e_steps, world)
+    barrier()
+    t0 = time.perf_counter()
+    for s in range(K):
+        obs, rew, flags, _ = venv.step_arrays(acts[s % 4], want_terminal_obs=False)
+    torch.cuda.synchronize()
+    e2e_step_s = _max_over_ranks((time.perf_counter() - t0) / K, world)
     e2e_value = N * world / e2e_step_s
     h2d = N * 4 * 4
     d2h = N * venv.obs_dim * 4 + N * 4 + N + N          # obs, reward, flag byte, targets-reached byte
-    e2e_launches = N_REGIONS * e2e_steps * (2 if N >= 16384 else 1)
+    e2e_launches = K * (2 if N >= 16384 else 1)
+    if args.dump_outputs:
+        env_outputs.update(e2e_obs=obs.copy(), e2e_reward=rew.copy(), e2e_flags=flags.copy())
     venv.close()
     # what bounds e2e: the step's results cross PCIe (the kernel writes them into pinned host memory as it runs); the link's
     # device->host rate is measured here with plain pinned copies of 64 MiB (copy engine, nothing else on the link)
@@ -580,10 +605,13 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     if not args.no_ppo and args.workload == "physics_only":
         ppo = {}
         try:
-            ppo["waypoints_v3_B"] = ppo_measure("waypoints_v3", 4096, 128, 4096 * 128 // 4, 20, rank, local_rank, world, iters=3)
+            ppo["waypoints_v3_B"] = ppo_measure("waypoints_v3", 4096, 128, 4096 * 128 // 4, 20, rank, local_rank, world, iters=3,
+                                                outputs=outputs, name="waypoints_v3_B")
             ppo["waypoints_v3_A"] = ppo_measure("waypoints_v3", 4096, 2048, 128, 20, rank, local_rank, world, iters=1, warm=1,
-                                                epochs_run=None if args.ppo_a_full else args.ppo_a_epochs)
-            ppo["waypoint_objlock"] = ppo_measure("waypoint_objlock", 65536, 64, 65536 * 64 // 4, 20, rank, local_rank, world, iters=2)
+                                                epochs_run=None if args.ppo_a_full else args.ppo_a_epochs,
+                                                outputs=outputs, name="waypoints_v3_A")
+            ppo["waypoint_objlock"] = ppo_measure("waypoint_objlock", 65536, 64, 65536 * 64 // 4, 20, rank, local_rank, world, iters=2,
+                                                  outputs=outputs, name="waypoint_objlock")
         except Exception as e:
             ppo["error"] = f"{type(e).__name__}: {e}"
             if world > 1:
@@ -631,15 +659,14 @@ def run_ours(args, rank: int, local_rank: int, world: int):
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": step_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": bench_config(args),
-            "timed": {"regions": N_REGIONS, "replays_per_region": R, "timed_launches": K * R, "region_ms": region_ms,
-                      "statistic": "median region / (K*R), MAX over ranks", "best_region_ms_per_step": best_ms,
+            "timed": {"regions": 1, "timed_launches": K, "region_ms": region_ms, "statistic": "region / K, MAX over ranks",
                       "physics_substeps_per_sec": value * cfg.inner_per_step * cfg.substeps_per_inner,
                       "l2": f"rotating {replicas} env batches ({replicas * state_bytes / 2**20:.0f} MiB > 2x L2)",
                       "launch": "host loop" if args.no_graph else
                                 f"CUDA graph of {replicas} launches chained by programmatic dependent launch edges (each launch steps "
                                 f"another env batch; the next one places its blocks while this one drains; FWSIM_PDL=0 = plain edges)"},
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "us_per_step": e2e_step_s * 1e6, "steps_per_region": e2e_steps, "regions": N_REGIONS, "roofline": pcie},
+                    "us_per_step": e2e_step_s * 1e6, "steps_per_region": K, "regions": 1, "roofline": pcie},
             "gpu_launches": int(launches + e2e_launches),
             "clocks": clocks,
             "roofline": roof,
@@ -650,6 +677,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
             v, sample = oracle_rate(args.workload, host_cores(), args.cpu_seconds)
             line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": host_cores(), "kind": "port",
                                     "sample": sample + f"; {cpu_model()}"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, env_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -665,9 +694,13 @@ def run_ppo(args, rank: int, local_rank: int, world: int):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     N, T = args.ppo_envs, args.ppo_n_steps
     bs = args.ppo_batch_size if args.ppo_batch_size > 0 else N * T // args.ppo_minibatches
-    K = max(1, min(args.steps, 5))
-    r = ppo_measure(args.ppo_preset, N, T, bs, args.ppo_epochs, rank, local_rank, world, iters=K, warm=1)
+    K = args.steps
+    outputs = {} if args.dump_outputs else None
+    r = ppo_measure(args.ppo_preset, N, T, bs, args.ppo_epochs, rank, local_rank, world, iters=K, warm=1, outputs=outputs,
+                    name=args.ppo_preset)
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {}, outputs)
         line = {"metric": "ppo_env_steps_per_sec", "value": r["sps"], "unit": "env-steps/s", "n_gpus": world,
                 "steps": K, "warmup": 2, "ms_per_step": r["iter_ms"], "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "f32", "data": "synthetic",
