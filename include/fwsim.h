@@ -102,7 +102,8 @@ typedef struct FwConfig {
                      * 4 duck-only lock/strike (FixedwingObjLockEnv: attitude + target_vector + 9*history (+4 deltas) obs) */
     int32_t num_targets, sparse_reward, angle_repr, max_steps, context_len;
     int32_t early_return_on_crash, complete_truncates;
-    int32_t wind_mode, wind_randomize, wind_rand_phase, wind_start_substep;
+    int32_t wind_mode, wind_randomize, wind_rand_phase, wind_start_substep;   /* wind_mode: 0 off, 1 constant, 2 gust_sine,
+                                                                              * 3 gridded field (fw_set_wind_field) */
     int32_t num_obstacles, cam_interval_substeps, lock_hold_steps, switch_min_seen, cam_res;
     int32_t force_generic_kernel;   /* 1 = never pick the kernels specialised for the standard aircraft layout (testing) */
     int32_t cam_mode;               /* 0 tracking chase camera (looks at the aircraft from cam_offset), 1 fixed camera at
@@ -129,7 +130,8 @@ typedef struct FwStateHost {
     int32_t* physics_steps; /* [N] */
     uint32_t* episode;   /* [N] */
     float* new_dist;     /* [N] WaypointHandler.new_distance */
-    float* wind;         /* [N,7] base xyz, gust amp xyz, phase */
+    float* wind;         /* [N,7] base xyz, gust amp xyz, phase.  wind_mode 3 (gridded field): the episode's spatial shift xyz
+                          * (metres; the field is sampled at position - shift), 0, 0, 0, time offset (seconds) */
     /* ObjLock tasks (2 and 4) only (ignored otherwise) */
     float* duck;         /* [N,3] duck position */
     float* obst;         /* [N,FW_MAX_OBST,3] cylinders x, y, height (first n_obst rows valid) */
@@ -142,6 +144,26 @@ typedef struct FwStateHost {
 
 typedef struct FwSim* fw_handle;
 
+/* Gridded wind field (FwConfig.wind_mode = 3): a regular lattice of world-frame (ENU) wind vectors, nx * ny * nz points from
+ * `origin` with `spacing` metres along world x, y, z, and nt time slices t_step seconds apart.  The step kernels evaluate it at
+ * every lifting surface's link CoM in the world (pos + R r_surf[s]) on every physics substep: trilinear in space with
+ * coordinates clamped to the box (a one-point axis is constant), linear in time and periodic with period nt * t_step (nt = 1 is
+ * a static field).  Time and gating are those of the uniform modes: physics step ps sees t = (ps - 1) dt + the episode's time
+ * offset, from wind_start_substep on.  With FwConfig.wind_randomize every reset draws a spatial shift ~ U(shift_lo, shift_hi)
+ * (the field is sampled at position - shift) and, when randomize_time is set, a time offset ~ U(0, nt * t_step); both come
+ * from the Philox stream of the other modes' wind draws (index 0), so they do not depend on how envs are sharded.
+ * Replaces: Aviary.register_wind_field_function(f) with f(time_s, positions[n,3]) -> [n,3], sampled on the lattice. */
+typedef struct FwWindField {
+    const float* values;     /* HOST [nt][nz][ny][nx][3] float32, m/s; copied by fw_set_wind_field */
+    int32_t nx, ny, nz, nt;  /* each >= 1; nx * ny * nz * nt < 2^31 */
+    double origin[3];        /* world position of lattice point (0, 0, 0), metres */
+    double spacing[3];       /* > 0, metres */
+    double t_step;           /* > 0, seconds between slices (any positive value when nt = 1) */
+    double shift_lo[3], shift_hi[3];   /* per-episode spatial shift range (wind_randomize), metres */
+    int32_t randomize_time;  /* 1: per-episode time offset ~ U(0, nt * t_step) (wind_randomize) */
+    int32_t _pad;
+} FwWindField;
+
 int fw_abi_version(void);
 const char* fw_last_error(void);
 int fw_config_size(void);
@@ -151,6 +173,12 @@ int fw_config_size(void);
  * rank r owns [r*N, (r+1)*N); the RNG is keyed by the global id so results do not depend on the split). */
 int fw_create(const FwConfig* cfg, int32_t n_envs, int32_t device, uint64_t seed, uint32_t env_id0, fw_handle* out);
 int fw_destroy(fw_handle h);
+/* Install the gridded wind field of a wind_mode 3 handle (see FwWindField).  fw_create with wind_mode 3 allocates the batch but
+ * defers its first reset to this call; step, reset and rollout entry points return FW_ESTATE until it has run.  Synchronous and
+ * one-shot: the values are validated (finite), uploaded to handle-owned device memory and the batch is reset; a second call
+ * returns FW_ESTATE, a handle of another wind mode FW_EINVAL.  The field stays fixed for the handle's lifetime (fw_destroy frees
+ * it), so every launch and CUDA graph sees the same field. */
+int fw_set_wind_field(fw_handle h, const FwWindField* field);
 int fw_num_envs(fw_handle h);
 int fw_obs_dim(fw_handle h);
 /* action width: 4 ([roll, pitch, yaw, thrust], Fixedwing mode 0) or 6 for task 3, the low-level env

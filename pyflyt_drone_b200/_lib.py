@@ -21,6 +21,15 @@ class FwStateHostC(C.Structure):
     ]
 
 
+class FwWindFieldC(C.Structure):
+    """include/fwsim.h FwWindField (the host-side description of a gridded wind field, wind_mode 3)."""
+    _fields_ = [
+        ("values", C.c_void_p), ("nx", C.c_int32), ("ny", C.c_int32), ("nz", C.c_int32), ("nt", C.c_int32),
+        ("origin", C.c_double * 3), ("spacing", C.c_double * 3), ("t_step", C.c_double),
+        ("shift_lo", C.c_double * 3), ("shift_hi", C.c_double * 3), ("randomize_time", C.c_int32), ("_pad", C.c_int32),
+    ]
+
+
 class FwError(RuntimeError):
     pass
 
@@ -35,6 +44,7 @@ SYMBOLS = [
     ("fw_config_size", C.c_int, []),
     ("fw_create", C.c_int, [C.POINTER(FwConfigC), C.c_int32, C.c_int32, C.c_uint64, C.c_uint32, C.POINTER(_P)]),
     ("fw_destroy", C.c_int, [_P]),
+    ("fw_set_wind_field", C.c_int, [_P, C.POINTER(FwWindFieldC)]),
     ("fw_num_envs", C.c_int, [_P]),
     ("fw_obs_dim", C.c_int, [_P]),
     ("fw_act_dim", C.c_int, [_P]),

@@ -267,9 +267,15 @@ def _wind_fields(wind: dict | None, hook: str) -> dict:
     if not wind or not bool(wind.get("enabled", False)):
         return dict(wind_mode=0)
     mode = str(wind.get("mode", "constant")).lower()
-    if mode not in ("constant", "gust_sine"):
+    if mode not in ("constant", "gust_sine", "field"):
         raise ValueError(f"Unsupported wind mode: {mode}")
     rnd = bool(wind.get("randomize_on_reset", False))
+    if mode == "field":
+        # gridded field (pyflyt_drone_b200/wind.py): the WindField itself travels beside the config, to FixedwingVecEnv
+        from .wind import WindField
+        if not isinstance(wind.get("field"), WindField):
+            raise ValueError("wind mode 'field' needs wind_config['field'] = a pyflyt_drone_b200.wind.WindField")
+        return dict(wind_mode=3, wind_randomize=int(rnd), wind_start_substep=0 if hook == "env" else 20)
 
     def vec(key):
         return [float(x) for x in np.asarray(wind.get(key, (0.0, 0.0, 0.0)), dtype=np.float64).reshape(3)]

@@ -64,7 +64,15 @@ struct FwSim {
     // the only hazard is device-lane work still in flight when a host-lane call starts: the flag makes that call wait
     // for the device first.  Pure-host and pure-device users never pay for it.
     bool dev_lane_dirty;
+    // gridded wind field (wind_mode 3): device lattice, and whether the batch still waits for it (fw_set_wind_field)
+    float4* wf_mem;
+    bool field_pending;
 };
+
+// step / reset / rollout entry points on a wind_mode 3 handle whose field has not been installed yet
+static int need_field(const FwSim* h) {
+    return h->field_pending ? fail(FW_ESTATE, "wind_mode 3: install the wind field with fw_set_wind_field first") : FW_OK;
+}
 
 // host-lane entry: wait for device-lane launches that may still be running on the caller's streams
 static int host_lane_enter(FwSim* h) {
@@ -109,6 +117,7 @@ static int derive(const FwConfig& c, int n, uint64_t seed, uint32_t env_id0, FwD
     memset(&d, 0, sizeof(d));
     const double PI = 3.14159265358979323846, DEG = PI / 180.0;
     if (!(c.dt > 0) || !(c.mass > 0)) return fail(FW_EINVAL, "dt and mass must be positive");
+    if (c.wind_mode < 0 || c.wind_mode > 3) return fail(FW_EINVAL, "wind_mode %d unknown (0 off, 1 constant, 2 gust_sine, 3 gridded field)", c.wind_mode);
     if (c.task < 0 || c.task > 4) return fail(FW_EINVAL, "task %d unknown (0 physics, 1 waypoints, 2 waypoint+objlock, 3 low-level, 4 duck-only objlock)", c.task);
     const bool cam_task = c.task == 2 || c.task == 4;
     if (cam_task && (c.num_obstacles < 0 || c.num_obstacles > FW_MAX_OBST)) return fail(FW_EINVAL, "num_obstacles out of range");
@@ -277,7 +286,7 @@ static int derive(const FwConfig& c, int n, uint64_t seed, uint32_t env_id0, FwD
     d.area_reward_scale = (float)c.area_reward_scale; d.lock_lost_penalty = (float)c.lock_lost_penalty;
     d.approach_clip = (float)c.approach_clip;
     d.warm_cached = 0;
-    d.packed = c.packed_pairs != 0 ? 1 : 0;
+    d.packed = (c.packed_pairs != 0 && c.wind_mode != 3) ? 1 : 0;    // the packed path has no gridded field
     d.seed_lo = (uint32_t)(seed & 0xffffffffu); d.seed_hi = (uint32_t)(seed >> 32); d.env_id0 = env_id0;
     d.n = n;
     d.i_begin = 0; d.i_end = n;
@@ -369,6 +378,7 @@ static size_t carve_planes(const FwConfig& cfg, const FwDev& dev, size_t N, char
 }
 
 static int fw_create_impl(const FwConfig* cfg, int32_t n_envs, int32_t device, uint64_t seed, uint32_t env_id0, FwSim* h);
+static int initial_episodes(FwSim* h);
 
 extern "C" int fw_create(const FwConfig* cfg, int32_t n_envs, int32_t device, uint64_t seed, uint32_t env_id0, fw_handle* out) {
     if (!cfg || !out) return fail(FW_EINVAL, "null argument");
@@ -400,7 +410,6 @@ static int fw_create_impl(const FwConfig* cfg, int32_t n_envs, int32_t device, u
     if (rc != FW_OK) return rc;
     h->obs_dim = h->dev.obs_dim;
     const size_t N = (size_t)n_envs;
-    const bool cam_task = cfg->task == 2 || cfg->task == 4;
     h->plane_bytes = carve_planes(*cfg, h->dev, N, nullptr, h->pl);
     ce = cudaMalloc((void**)&h->plane_mem, h->plane_bytes);
     if (ce != cudaSuccess) return fail(FW_ENOMEM, "cudaMalloc(%zu): %s", h->plane_bytes, cudaGetErrorString(ce));
@@ -412,8 +421,21 @@ static int fw_create_impl(const FwConfig* cfg, int32_t n_envs, int32_t device, u
     CU(cudaStreamCreateWithFlags(&h->io_stream, cudaStreamNonBlocking));
     h->io_streams[0] = h->io_stream;
     CU(cudaStreamCreateWithFlags(&h->io_streams[1], cudaStreamNonBlocking));
+    if (h->dev.wind_mode == 3) {          // the first reset needs the field: fw_set_wind_field runs the set-up
+        h->field_pending = true;
+        return FW_OK;
+    }
+    return initial_episodes(h);
+}
 
-
+// The warm-up cache decision, the first reset of every env and the spare episodes of the camera tasks: the tail of fw_create,
+// or of fw_set_wind_field for a wind_mode 3 handle.
+static int initial_episodes(FwSim* h) {
+    cudaError_t ce;
+    const FwConfig* cfg = &h->cfg;
+    const int32_t n_envs = h->n;
+    const size_t N = (size_t)n_envs;
+    const bool cam_task = cfg->task == 2 || cfg->task == 4;
     // cache the deterministic warm-up result when no wind acts during it
     if (!cam_task && (h->dev.wind_mode == 0 || h->dev.wind_start_substep >= h->dev.warmup_substeps)) {
         float* d_warm = nullptr;
@@ -501,6 +523,7 @@ extern "C" int fw_destroy(fw_handle h) {
                 break;
             }
     if (h->plane_mem) cudaFree(h->plane_mem);
+    if (h->wf_mem) cudaFree(h->wf_mem);
     if (h->d_act) cudaFree(h->d_act);
     if (h->d_obs) cudaFree(h->d_obs);
     if (h->d_rew) cudaFree(h->d_rew);
@@ -525,6 +548,60 @@ extern "C" int fw_destroy(fw_handle h) {
     return FW_OK;
 }
 
+extern "C" int fw_set_wind_field(fw_handle h, const FwWindField* f) {
+    // argument checks first, without touching the device
+    if (!f) return fail(FW_EINVAL, "null wind field");
+    if (!f->values) return fail(FW_EINVAL, "wind field: values is null");
+    if (f->nx < 1 || f->ny < 1 || f->nz < 1 || f->nt < 1) return fail(FW_EINVAL, "wind field: every dimension must be >= 1");
+    const int64_t pts = (int64_t)f->nx * f->ny * f->nz;
+    if (pts * f->nt >= ((int64_t)1 << 31)) return fail(FW_EINVAL, "wind field: nx * ny * nz * nt must be < 2^31");
+    for (int k = 0; k < 3; ++k) {
+        if (!(f->spacing[k] > 0) || !std::isfinite(f->spacing[k])) return fail(FW_EINVAL, "wind field: spacing must be finite and > 0");
+        if (!std::isfinite(f->origin[k])) return fail(FW_EINVAL, "wind field: origin must be finite");
+        if (!std::isfinite(f->shift_lo[k]) || !std::isfinite(f->shift_hi[k]) || f->shift_lo[k] > f->shift_hi[k])
+            return fail(FW_EINVAL, "wind field: shift range must be finite with shift_lo <= shift_hi");
+    }
+    if (!(f->t_step > 0) || !std::isfinite(f->t_step)) return fail(FW_EINVAL, "wind field: t_step must be finite and > 0");
+    const size_t nval = (size_t)(pts * f->nt) * 3;
+    for (size_t k = 0; k < nval; ++k)
+        if (!std::isfinite(f->values[k])) return fail(FW_EINVAL, "wind field: value %zu is not finite", k);
+    if (!h) return fail(FW_EINVAL, "null handle");
+    if (h->dev.wind_mode != 3) return fail(FW_EINVAL, "fw_set_wind_field needs a handle created with wind_mode 3 (has %d)", h->dev.wind_mode);
+    if (!h->field_pending) return fail(FW_ESTATE, "the wind field of this handle is already set (one field per handle)");
+    CU(cudaSetDevice(h->device));
+    // float4 lattice points: one 16-byte load per corner
+    const size_t npts = (size_t)(pts * f->nt);
+    std::vector<float4> host(npts);
+    for (size_t k = 0; k < npts; ++k) host[k] = make_float4(f->values[3 * k], f->values[3 * k + 1], f->values[3 * k + 2], 0.0f);
+    cudaError_t ce = cudaMalloc((void**)&h->wf_mem, npts * sizeof(float4));
+    if (ce != cudaSuccess) { h->wf_mem = nullptr; return fail(FW_ENOMEM, "cudaMalloc(%zu) for the wind field: %s", npts * sizeof(float4), cudaGetErrorString(ce)); }
+    ce = cudaMemcpyAsync(h->wf_mem, host.data(), npts * sizeof(float4), cudaMemcpyHostToDevice, h->io_stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(h->io_stream);
+    if (ce != cudaSuccess) {                  // the handle stays pending: a later call may try again
+        cudaFree(h->wf_mem);
+        h->wf_mem = nullptr;
+        return fail(FW_ECUDA, "uploading the wind field: %s", cudaGetErrorString(ce));
+    }
+    FwDev& d = h->dev;
+    d.wf = h->wf_mem;
+    d.wf_n[0] = f->nx; d.wf_n[1] = f->ny; d.wf_n[2] = f->nz; d.wf_n[3] = f->nt;
+    d.wf_pts = (int)pts;
+    for (int k = 0; k < 3; ++k) {
+        d.wf_origin[k] = (float)f->origin[k];
+        d.wf_inv_sp[k] = (float)(1.0 / f->spacing[k]);
+        d.wf_max[k] = (float)((k == 0 ? f->nx : (k == 1 ? f->ny : f->nz)) - 1);
+        d.wf_shift_lo[k] = (float)f->shift_lo[k]; d.wf_shift_hi[k] = (float)f->shift_hi[k];
+    }
+    d.wf_sps = (float)(h->cfg.dt / f->t_step);
+    d.wf_inv_tstep = (float)(1.0 / f->t_step);
+    d.wf_nt = (float)f->nt;
+    d.wf_inv_nt = (float)(1.0 / f->nt);
+    d.wf_period = (float)(f->nt * f->t_step);
+    d.wf_rand_time = f->randomize_time != 0;
+    h->field_pending = false;
+    return initial_episodes(h);
+}
+
 extern "C" int fw_num_envs(fw_handle h) { return h ? h->n : fail(FW_EINVAL, "null handle"); }
 extern "C" int fw_obs_dim(fw_handle h) { return h ? h->obs_dim : fail(FW_EINVAL, "null handle"); }
 extern "C" int fw_act_dim(fw_handle h) { return h ? h->dev.act_dim : fail(FW_EINVAL, "null handle"); }
@@ -532,6 +609,7 @@ extern "C" int64_t fw_launch_count(fw_handle h) { return h ? h->launches : 0; }
 
 extern "C" int fw_reset(fw_handle h, const uint8_t* mask_dev, float* obs_dev, void* stream) {
     if (!h) return fail(FW_EINVAL, "null handle");
+    if (need_field(h) != FW_OK) return FW_ESTATE;
     CU(cudaSetDevice(h->device));
     // the first whole-batch reset after fw_create only emits the observation of the episode-0 state
     const bool emit_only = h->fresh && mask_dev == nullptr;
@@ -547,6 +625,7 @@ extern "C" int fw_step(fw_handle h, const float* act_dev, float* obs_dev, float*
     if (!h) return fail(FW_EINVAL, "null handle");
     if (!act_dev) return fail(FW_EINVAL, "act_dev is null");
     if ((reinterpret_cast<uintptr_t>(act_dev) & 15u) != 0) return fail(FW_EINVAL, "act_dev must be 16-byte aligned");
+    if (need_field(h) != FW_OK) return FW_ESTATE;
     CU(cudaSetDevice(h->device));
     int rc = launch_step(h, h->dev, h->pl, act_dev, obs_dev, rew_dev, flags_dev, term_obs_dev, false, 1, (cudaStream_t)stream);
     if (rc != FW_OK) return rc;
@@ -558,6 +637,7 @@ extern "C" int fw_step(fw_handle h, const float* act_dev, float* obs_dev, float*
 extern "C" int fw_step_random(fw_handle h, int32_t n_steps, float* rew_dev, uint8_t* flags_dev, void* stream) {
     if (!h) return fail(FW_EINVAL, "null handle");
     if (n_steps < 0) return fail(FW_EINVAL, "n_steps < 0");
+    if (need_field(h) != FW_OK) return FW_ESTATE;
     CU(cudaSetDevice(h->device));
     h->fresh = false;
     h->dev_lane_dirty = true;
@@ -575,6 +655,7 @@ extern "C" int fw_rollout_random(const fw_handle* hs, int32_t n_handles, int32_t
     for (int k = 0; k < n_handles; ++k) {
         if (!hs[k]) return fail(FW_EINVAL, "null handle in list");
         if (hs[k]->device != hs[0]->device) return fail(FW_EINVAL, "handles of one rollout must share a device");
+        if (need_field(hs[k]) != FW_OK) return FW_ESTATE;
         hs[k]->fresh = false;
         hs[k]->dev_lane_dirty = true;
     }
@@ -629,6 +710,7 @@ extern "C" int fw_step_host(fw_handle h, const float* act_host, float* obs_host,
                             float* term_obs_host) {
     if (!h) return fail(FW_EINVAL, "null handle");
     if (!act_host) return fail(FW_EINVAL, "act_host is null");
+    if (need_field(h) != FW_OK) return FW_ESTATE;
     CU(cudaSetDevice(h->device));
     int rc = ensure_host_io(h);
     if (rc != FW_OK) return rc;
@@ -782,6 +864,7 @@ extern "C" int fw_observe_host(fw_handle h, float* obs_host) { return reset_host
 
 static int reset_host_impl(fw_handle h, float* obs_host, bool observe_only) {
     if (!h) return fail(FW_EINVAL, "null handle");
+    if (need_field(h) != FW_OK) return FW_ESTATE;
     CU(cudaSetDevice(h->device));
     int rc = ensure_host_io(h);
     if (rc != FW_OK) return rc;

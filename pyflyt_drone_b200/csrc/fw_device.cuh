@@ -137,6 +137,28 @@ struct FwDev {
     // env range [i_begin, i_end) a step launch covers (whole batch by default; the host lane launches chunks so that
     // the device-to-host copy of one chunk overlaps the kernel of the next)
     int i_begin, i_end;
+    // gridded wind field (wind_mode 3, fw_set_wind_field): world-frame wind as float4 lattice points [nt][nz][ny][nx] in HBM,
+    // owned by the handle and fixed before the first launch.  Per env, w0 holds the episode's spatial shift (xyz, metres; the
+    // field is sampled at position - shift) and time offset (w, seconds).
+    const float4* wf;
+    int wf_n[4];                          // nx, ny, nz, nt
+    int wf_pts;                           // nx * ny * nz: points per time slice
+    float wf_origin[3], wf_inv_sp[3];     // lattice origin, 1 / spacing
+    float wf_max[3];                      // n - 1 per axis: the clamp of the lattice coordinate
+    float wf_sps, wf_inv_tstep, wf_nt, wf_inv_nt;   // dt / t_step (slices per substep), 1 / t_step, nt, 1 / nt
+    float wf_period;                      // nt * t_step: the time offset is drawn from [0, period)
+    float wf_shift_lo[3], wf_shift_hi[3];
+    int wf_rand_time;
+};
+
+// time pair of the gridded field for one substep, shared by all surfaces: slices a, b and the weight of b.  on = false before
+// the wind starts (stamp < 0 or < wind_start_substep): the surfaces then see calm air.
+struct FwFieldT {
+    const float4* a;
+    const float4* b;
+    float wb;
+    float sx, sy, sz;     // the episode's spatial shift
+    bool on;
 };
 
 // SoA state in HBM: float4 planes (16-byte coalesced accesses, one plane element per env)
@@ -337,6 +359,87 @@ __device__ __forceinline__ void fw_surface(const FwDev& p, const SF& sf, float a
     tq = Q * CMc;
 }
 
+// ------------------------------------------------------------------ gridded wind field (wind_mode 3)
+// Time: linear between slices, periodic with period nt * t_step; the stamp is the one fw_wind uses (physics step ps - 1).
+__device__ __forceinline__ void fw_field_time(const FwDev& p, int ps, const float4& w0, FwFieldT& t) {
+    const int stamp = ps - 1;
+    t.on = stamp >= 0 && stamp >= p.wind_start_substep;
+    t.sx = w0.x; t.sy = w0.y; t.sz = w0.z;
+    float u = fmaf((float)stamp, p.wf_sps, w0.w * p.wf_inv_tstep);     // slices since t = 0
+    u -= p.wf_nt * floorf(u * p.wf_inv_nt);
+    const int nt = p.wf_n[3];
+    const int i0 = min(max((int)u, 0), nt - 1);
+    const int i1 = i0 + 1 < nt ? i0 + 1 : 0;
+    t.wb = fminf(fmaxf(u - (float)i0, 0.0f), 1.0f);
+    t.a = p.wf + (size_t)i0 * p.wf_pts;
+    t.b = p.wf + (size_t)i1 * p.wf_pts;
+}
+
+// lattice coordinate along one axis: clamped to the box, cell index i0 and the step to its neighbour (0 on the last point
+// or on a one-point axis: i1 = min(i0 + 1, n - 1))
+__device__ __forceinline__ void fw_field_axis(float x, float org, float inv_sp, float gmax, int n, int& i0, int& di, float& f) {
+    const float g = fminf(fmaxf((x - org) * inv_sp, 0.0f), gmax);
+    i0 = min((int)g, n - 1);
+    di = i0 + 1 < n ? 1 : 0;
+    f = g - (float)i0;
+}
+
+__device__ __forceinline__ float3 fw_field_trilinear(const float4* __restrict__ s, int base, int dx, int dy, int dz, float fx,
+                                                     float fy, float fz) {
+    const float4 c000 = __ldg(s + base), c100 = __ldg(s + base + dx);
+    const float4 c010 = __ldg(s + base + dy), c110 = __ldg(s + base + dy + dx);
+    const float4 c001 = __ldg(s + base + dz), c101 = __ldg(s + base + dz + dx);
+    const float4 c011 = __ldg(s + base + dz + dy), c111 = __ldg(s + base + dz + dy + dx);
+    float3 r;
+    {
+        const float x00 = fmaf(fx, c100.x - c000.x, c000.x), x10 = fmaf(fx, c110.x - c010.x, c010.x);
+        const float x01 = fmaf(fx, c101.x - c001.x, c001.x), x11 = fmaf(fx, c111.x - c011.x, c011.x);
+        const float y0 = fmaf(fy, x10 - x00, x00), y1 = fmaf(fy, x11 - x01, x01);
+        r.x = fmaf(fz, y1 - y0, y0);
+    }
+    {
+        const float x00 = fmaf(fx, c100.y - c000.y, c000.y), x10 = fmaf(fx, c110.y - c010.y, c010.y);
+        const float x01 = fmaf(fx, c101.y - c001.y, c001.y), x11 = fmaf(fx, c111.y - c011.y, c011.y);
+        const float y0 = fmaf(fy, x10 - x00, x00), y1 = fmaf(fy, x11 - x01, x01);
+        r.y = fmaf(fz, y1 - y0, y0);
+    }
+    {
+        const float x00 = fmaf(fx, c100.z - c000.z, c000.z), x10 = fmaf(fx, c110.z - c010.z, c010.z);
+        const float x01 = fmaf(fx, c101.z - c001.z, c001.z), x11 = fmaf(fx, c111.z - c011.z, c011.z);
+        const float y0 = fmaf(fy, x10 - x00, x00), y1 = fmaf(fy, x11 - x01, x01);
+        r.z = fmaf(fz, y1 - y0, y0);
+    }
+    return r;
+}
+
+// world-frame wind of the field at world point (x, y, z) for the time pair t: trilinear in space (clamped to the box) on both
+// slices, linear in time -- 8 corners x 2 slices of 16-byte read-only loads
+__device__ __forceinline__ float3 fw_wind_field(const FwDev& p, const FwFieldT& t, float x, float y, float z) {
+    int ix, iy, iz, dx, dy, dz;
+    float fx, fy, fz;
+    fw_field_axis(x - t.sx, p.wf_origin[0], p.wf_inv_sp[0], p.wf_max[0], p.wf_n[0], ix, dx, fx);
+    fw_field_axis(y - t.sy, p.wf_origin[1], p.wf_inv_sp[1], p.wf_max[1], p.wf_n[1], iy, dy, fy);
+    fw_field_axis(z - t.sz, p.wf_origin[2], p.wf_inv_sp[2], p.wf_max[2], p.wf_n[2], iz, dz, fz);
+    const int nx = p.wf_n[0], nxy = nx * p.wf_n[1];
+    const int base = iz * nxy + iy * nx + ix;
+    const float3 a = fw_field_trilinear(t.a, base, dx, dy * nx, dz * nxy, fx, fy, fz);
+    const float3 b = fw_field_trilinear(t.b, base, dx, dy * nx, dz * nxy, fx, fy, fz);
+    return make_float3(fmaf(t.wb, b.x - a.x, a.x), fmaf(t.wb, b.y - a.y, a.y), fmaf(t.wb, b.z - a.z, a.z));
+}
+
+// local airflow (body frame) of the surface with body-frame link CoM r minus the field's wind at that link CoM
+__device__ __forceinline__ void fw_field_subtract(const FwDev& p, const FwFieldT& t, const EnvState& e, const float* m,
+                                                  const float r[3], float& sx, float& sy, float& sz) {
+    if (!t.on) return;
+    const float x = e.px + m[0] * r[0] + m[1] * r[1] + m[2] * r[2];
+    const float y = e.py + m[3] * r[0] + m[4] * r[1] + m[5] * r[2];
+    const float z = e.pz + m[6] * r[0] + m[7] * r[1] + m[8] * r[2];
+    const float3 w = fw_wind_field(p, t, x, y, z);
+    sx -= m[0] * w.x + m[3] * w.y + m[6] * w.z;
+    sy -= m[1] * w.x + m[4] * w.y + m[7] * w.z;
+    sz -= m[2] * w.x + m[5] * w.y + m[8] * w.z;
+}
+
 // ------------------------------------------------------------------ one 240 Hz substep
 // cmd: latched actuator commands [5 surfaces + motor]; wind: world-frame wind seen by the surfaces
 // (already selected for this substep's time stamp); nz: N(0,1) draw for the motor noise.
@@ -345,9 +448,11 @@ __device__ __forceinline__ void fw_surface(const FwDev& p, const SF& sf, float a
 // unit is +x; lift unit +z for surfaces 0,1,2,4 and +y for surface 3 (vertical tail); thrust along +x; the aircraft
 // is symmetric about its xz plane, so the inverse spatial inertia splits into a lateral {wx, wz, vy} and a
 // longitudinal {wy, vx, vz} 3x3 block.  The arithmetic is the generic path's with the structural zeros skipped.
-template <bool STD = false>
+// FIELD = gridded wind (wind_mode 3): wn* are ignored (pass 0); every surface subtracts R^T w_s from its own local airflow,
+// w_s = the field at its link CoM in the world, pos + R r_s, for the time pair ft.
+template <bool STD = false, bool FIELD = false>
 __device__ __forceinline__ void fw_substep(const FwDev& p, EnvState& e, const float cmd[6], float wnx, float wny,
-                                           float wnz, float nz, bool& contact) {
+                                           float wnz, float nz, bool& contact, const FwFieldT& ft = FwFieldT()) {
     const float dt = p.dt;
     Mat3 R = fw_quat_mat(e.qx, e.qy, e.qz, e.qw);
     const float* m = R.m;
@@ -369,9 +474,10 @@ __device__ __forceinline__ void fw_substep(const FwDev& p, EnvState& e, const fl
             float sx = fmaf(wby, sf.r[2], fmaf(-wbz, sf.r[1], vbx));
             float sy = fmaf(wbz, sf.r[0], fmaf(-wbx, sf.r[2], vby));
             float sz = fmaf(wbx, sf.r[1], fmaf(-wby, sf.r[0], vbz));
+            if (FIELD) fw_field_subtract(p, ft, e, m, sf.r, sx, sy, sz);
             float fn, fp, tq;
             // force = lift*fn + fwd*fp at the link CoM; torque about O = fn (r x lift) + fp (r x fwd) + tq (lift x fwd)
-            if (s != 3) {               // lift +z, fwd +x: ra = (ry, -rx, 0), rb = (0, rz, -ry), lift x fwd = +y
+            if (s != 3) {              // lift +z, fwd +x: ra = (ry, -rx, 0), rb = (0, rz, -ry), lift x fwd = +y
                 fw_surface<true, false>(p, sf, e.act[s], sx, sy, sz, fn, fp, tq);
                 Fx += fp; Fz += fn;
                 Tx += sf.ra[0] * fn;
@@ -391,6 +497,7 @@ __device__ __forceinline__ void fw_substep(const FwDev& p, EnvState& e, const fl
         float sx = fmaf(wby, sf.r[2], fmaf(-wbz, sf.r[1], vbx));
         float sy = fmaf(wbz, sf.r[0], fmaf(-wbx, sf.r[2], vby));
         float sz = fmaf(wbx, sf.r[1], fmaf(-wby, sf.r[0], vbz));
+        if (FIELD) fw_field_subtract(p, ft, e, m, sf.r, sx, sy, sz);
         float fn, fp, tq;
         {
             fw_surface(p, sf, e.act[s], sx, sy, sz, fn, fp, tq);
@@ -647,9 +754,33 @@ __device__ __forceinline__ void fw_write_obs_lowlevel(const FwPlanes& pl, const 
 // end_reset: warmup_substeps substeps at zero setpoint.  Kept out of line: it is the rare path (only when a wind
 // field acts during the warm-up, otherwise resets copy the cached result) and inlining it would duplicate
 // the whole substep body and double the kernel's instruction-cache footprint.
+// One substep under the wind of the env's mode: the uniform wind of fw_wind, or (FIELD) the gridded field per surface.
+template <bool STD, bool FIELD>
+__device__ __forceinline__ void fw_substep_wind(const FwDev& p, EnvState& e, const float cmd[6], const float4& w0,
+                                                const float4& w1, float nz, bool& contact) {
+    if (FIELD) {
+        FwFieldT ft;
+        fw_field_time(p, e.physics_steps, w0, ft);
+        fw_substep<STD, true>(p, e, cmd, 0.0f, 0.0f, 0.0f, nz, contact, ft);
+    } else {
+        float wx, wy, wz;
+        fw_wind(p, e.physics_steps, w0, w1, wx, wy, wz);
+        fw_substep<STD>(p, e, cmd, wx, wy, wz, nz, contact);
+    }
+}
+
+template <bool FIELD = false>
 static __device__ __noinline__ void fw_warmup_loop(const FwDev& p, EnvState& e, float4 w0, float4 w1, int nsub) {
     float cmd[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     bool contact = false;
+    if (FIELD) {
+        if (p.std_geom) {
+            for (int k = 0; k < nsub; ++k) fw_substep_wind<true, true>(p, e, cmd, w0, w1, 0.0f, contact);
+            return;
+        }
+        for (int k = 0; k < nsub; ++k) fw_substep_wind<false, true>(p, e, cmd, w0, w1, 0.0f, contact);
+        return;
+    }
     if (p.std_geom) {                // same choice of physics path as the step kernels (uniform branch)
         for (int k = 0; k < nsub; ++k) {
             float wx, wy, wz;
@@ -666,14 +797,29 @@ static __device__ __noinline__ void fw_warmup_loop(const FwDev& p, EnvState& e, 
 }
 
 // ---- reset pieces (begin_reset / WaypointHandler.reset / end_reset), composed per task by the kernels
+// FIELD: w0 = (spatial shift xyz ~ U(shift_lo, shift_hi), time offset ~ U(0, nt t_step) when randomize_time), w1 = 0; both
+// zero without wind_randomize.  Same Philox stream and counter as the uniform modes' draws.
+template <bool FIELD = false>
 __device__ __forceinline__ void fw_reset_begin(const FwDev& p, const FwPlanes& pl, EnvState& e, int i, uint32_t gid,
                                                uint32_t episode, float4& w0, float4& w1) {
     e.episode = episode;
     e.step_count = 0;
     e.tidx = 0;
-    w0 = make_float4(p.wind_base[0], p.wind_base[1], p.wind_base[2], p.gust_phase);
-    w1 = make_float4(p.gust_amp[0], p.gust_amp[1], p.gust_amp[2], 0.0f);
-    if (p.wind_mode != 0) {
+    if (FIELD) {
+        w0 = make_float4(0.f, 0.f, 0.f, 0.f);
+        w1 = w0;
+        if (p.wind_randomize) {
+            const uint4 r0 = fw_philox(p.seed_lo, p.seed_hi, gid, episode, 0u, FWD_STREAM_WIND);
+            w0.x = p.wf_shift_lo[0] + fw_u01(r0.x) * (p.wf_shift_hi[0] - p.wf_shift_lo[0]);
+            w0.y = p.wf_shift_lo[1] + fw_u01(r0.y) * (p.wf_shift_hi[1] - p.wf_shift_lo[1]);
+            w0.z = p.wf_shift_lo[2] + fw_u01(r0.z) * (p.wf_shift_hi[2] - p.wf_shift_lo[2]);
+            if (p.wf_rand_time) w0.w = fw_u01(r0.w) * p.wf_period;
+        }
+        pl.w0[i] = w0; pl.w1[i] = w1;
+    }
+    w0 = FIELD ? w0 : make_float4(p.wind_base[0], p.wind_base[1], p.wind_base[2], p.gust_phase);
+    w1 = FIELD ? w1 : make_float4(p.gust_amp[0], p.gust_amp[1], p.gust_amp[2], 0.0f);
+    if (!FIELD && p.wind_mode != 0) {
         if (p.wind_randomize) {
             uint4 r0 = fw_philox(p.seed_lo, p.seed_hi, gid, episode, 0u, FWD_STREAM_WIND);
             uint4 r1 = fw_philox(p.seed_lo, p.seed_hi, gid, episode, 1u, FWD_STREAM_WIND);
@@ -726,6 +872,7 @@ __device__ __forceinline__ void fw_sample_targets(const FwDev& p, const FwPlanes
 }
 
 // nsub warm-up substeps at zero setpoint (end_reset); copies the cached result when it is valid
+template <bool FIELD = false>
 __device__ __forceinline__ void fw_warm(const FwDev& p, EnvState& e, const float4& w0, const float4& w1, int nsub,
                                         bool allow_cache) {
     if (allow_cache && p.warm_cached && nsub == p.warmup_substeps) {
@@ -739,7 +886,7 @@ __device__ __forceinline__ void fw_warm(const FwDev& p, EnvState& e, const float
         e.physics_steps = p.warmup_substeps;
     } else if (nsub > 0) {
         EnvState tmp = e;          // only this copy is address-taken (local memory); `e` stays in registers
-        fw_warmup_loop(p, tmp, w0, w1, nsub);
+        fw_warmup_loop<FIELD>(p, tmp, w0, w1, nsub);
         e = tmp;
     }
 }
@@ -755,12 +902,13 @@ __device__ __forceinline__ void fw_reset_finish(const FwDev& p, const FwPlanes& 
 }
 
 // begin_reset/end_reset for the physics-only and Waypoints tasks
+template <bool FIELD = false>
 __device__ __forceinline__ void fw_reset_env(const FwDev& p, const FwPlanes& pl, EnvState& e, int i, uint32_t gid,
                                              uint32_t episode) {
     float4 w0, w1;
-    fw_reset_begin(p, pl, e, i, gid, episode, w0, w1);
+    fw_reset_begin<FIELD>(p, pl, e, i, gid, episode, w0, w1);
     if (p.task != 0) fw_sample_targets(p, pl, i, gid, episode);
-    fw_warm(p, e, w0, w1, p.warmup_substeps, true);
+    fw_warm<FIELD>(p, e, w0, w1, p.warmup_substeps, true);
     fw_reset_finish(p, pl, e, i);
 }
 

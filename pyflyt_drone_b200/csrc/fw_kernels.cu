@@ -76,7 +76,7 @@ __device__ __forceinline__ void fw_flush_obs(float* __restrict__ dst_base, const
 
 // One agent step of env i held in registers (FixedwingBaseEnv.step + SubprocVecEnv reset-on-done).
 // Returns the reward; flag bits in `bits`; the observation (if TASK != 0) is left in `row`.
-template <int TASK, bool STD>
+template <int TASK, bool STD, bool FIELD = false>
 __device__ __forceinline__ float fw_env_step(const FwDev& p, const FwPlanes& pl, EnvState& e, int i,
                                              uint32_t gid, float a0, float a1, float a2, float a3, const float4& w0_in,
                                              const float4& w1_in, float& ep_ret, float* row, float* term_obs_row,
@@ -110,9 +110,7 @@ __device__ __forceinline__ float fw_env_step(const FwDev& p, const FwPlanes& pl,
                 const int q = ps & 3;
                 nz = q == 0 ? n0 : (q == 1 ? n1 : (q == 2 ? n2 : n3));
             }
-            float wx, wy, wz;
-            fw_wind(p, ps, w0, w1, wx, wy, wz);
-            fw_substep<STD>(p, e, cmd, wx, wy, wz, nz, contact);
+            fw_substep_wind<STD, FIELD>(p, e, cmd, w0, w1, nz, contact);
         }
         // compute_state: WaypointHandler.distance_to_targets (old <- new, new <- |delta_0|)
         float old_dist = e.new_dist;
@@ -161,7 +159,7 @@ __device__ __forceinline__ float fw_env_step(const FwDev& p, const FwPlanes& pl,
         if (oob) atomicAdd(&pl.stats[5], 1.0);
         if (complete) atomicAdd(&pl.stats[6], 1.0);
         // SubprocVecEnv worker: obs = env.reset()
-        fw_reset_env(p, pl, e, i, gid, e.episode + 1u);
+        fw_reset_env<FIELD>(p, pl, e, i, gid, e.episode + 1u);
         if (p.wind_mode != 0) { w0 = pl.w0[i]; w1 = pl.w1[i]; }
         if (TASK != 0 && row != nullptr) fw_write_obs(p, pl, e, i, 0, 0.f, 0.f, 0.f, 0.f, row);
         if (fault && TASK != 0 && term_obs_row != nullptr)     // a finite stand-in: the first observation of the new episode
@@ -175,7 +173,7 @@ __device__ __forceinline__ float fw_env_step(const FwDev& p, const FwPlanes& pl,
 // FixedwingLowLevelEnv.step (fixedwing_lowlevel_env.py:97-141): six-channel surface/thrust command (Fixedwing mode -1),
 // ONE Aviary.step (2 physics substeps) per env step, psi/h/V tracking reward, altitude-band termination, truncation at
 // `max_steps` (>=); SubprocVecEnv reset-on-done.  No warm-up substeps and no ground-contact / dome test in this env.
-template <bool STD>
+template <bool STD, bool FIELD = false>
 __device__ __forceinline__ float fw_env_step_lowlevel(const FwDev& p, const FwPlanes& pl, EnvState& e, int i, uint32_t gid,
                                                       const float a[6], const float4& w0_in, const float4& w1_in, float& ep_ret,
                                                       float* row, float* term_obs_row, uint32_t& bits) {
@@ -196,9 +194,7 @@ __device__ __forceinline__ float fw_env_step_lowlevel(const FwDev& p, const FwPl
             const int q = ps & 3;
             nz = q == 0 ? nn[0] : (q == 1 ? nn[1] : (q == 2 ? nn[2] : nn[3]));
         }
-        float wx, wy, wz;
-        fw_wind(p, ps, w0, w1, wx, wy, wz);
-        fw_substep<STD>(p, e, cmd, wx, wy, wz, nz, contact);
+        fw_substep_wind<STD, FIELD>(p, e, cmd, w0, w1, nz, contact);
     }
     float yaw, speed, tref[3];
     fw_write_obs_lowlevel(pl, e, i, p.n, a, row, yaw, speed, tref);
@@ -221,7 +217,7 @@ __device__ __forceinline__ float fw_env_step_lowlevel(const FwDev& p, const FwPl
         atomicAdd(&pl.stats[1], (double)ep_ret);
         atomicAdd(&pl.stats[2], (double)e.step_count);
         if (oob) atomicAdd(&pl.stats[5], 1.0);
-        fw_reset_env(p, pl, e, i, gid, e.episode + 1u);
+        fw_reset_env<FIELD>(p, pl, e, i, gid, e.episode + 1u);
         if (row != nullptr) {
             const float z6[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             fw_write_obs_lowlevel(pl, e, i, p.n, z6, row, yaw, speed, tref);
@@ -237,7 +233,7 @@ __device__ __forceinline__ float fw_env_step_lowlevel(const FwDev& p, const FwPl
 // K1.  RANDOM_ACT: actions U(-1,1)^4 from Philox keyed (seed, global env id, episode, step_count); `spl` agent
 // steps per launch with the state held in registers between them (the random-action sweep never needs the
 // intermediate observations, so nothing but the final state goes back to HBM).
-template <int TASK, bool RANDOM_ACT, bool STD>
+template <int TASK, bool RANDOM_ACT, bool STD, bool FIELD = false>
 __global__ void __launch_bounds__(FW_BLOCK, FW_MIN_BLOCKS)
 fw_step_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4* __restrict__ act,
                float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ flg,
@@ -283,7 +279,7 @@ fw_step_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4*
                     a6[0] = u0.x; a6[1] = u0.y; a6[2] = u1.x; a6[3] = u1.y; a6[4] = u2.x; a6[5] = u2.y;
                 }
                 if (p.wind_mode != 0 && st > 0) { w0 = pl.w0[i]; w1 = pl.w1[i]; }
-                reward = fw_env_step_lowlevel<STD>(p, pl, e, i, gid, a6, w0, w1, ep_ret, st == nst - 1 ? orow : nullptr,
+                reward = fw_env_step_lowlevel<STD, FIELD>(p, pl, e, i, gid, a6, w0, w1, ep_ret, st == nst - 1 ? orow : nullptr,
                                                    (!RANDOM_ACT && term_obs != nullptr && orow != nullptr) ? term_obs + (size_t)i * D : nullptr,
                                                    bits);
             }
@@ -293,12 +289,12 @@ fw_step_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4*
                 float a0 = 2.0f * fw_u01(r.x) - 1.0f, a1 = 2.0f * fw_u01(r.y) - 1.0f;
                 float a2 = 2.0f * fw_u01(r.z) - 1.0f, a3 = 2.0f * fw_u01(r.w) - 1.0f;
                 if (p.wind_mode != 0 && st > 0) { w0 = pl.w0[i]; w1 = pl.w1[i]; }
-                reward = fw_env_step<TASK, STD>(p, pl, e, i, gid, a0, a1, a2, a3, w0, w1, ep_ret,
+                reward = fw_env_step<TASK, STD, FIELD>(p, pl, e, i, gid, a0, a1, a2, a3, w0, w1, ep_ret,
                                            st == spl - 1 ? row : nullptr, nullptr, bits, tidx_info);
             }
         } else {
             float4 a = act[i];
-            reward = fw_env_step<TASK, STD>(p, pl, e, i, gid, a.x, a.y, a.z, a.w, w0, w1, ep_ret, row,
+            reward = fw_env_step<TASK, STD, FIELD>(p, pl, e, i, gid, a.x, a.y, a.z, a.w, w0, w1, ep_ret, row,
                                        (TASK != 0 && term_obs != nullptr && row != nullptr) ? term_obs + (size_t)i * D : nullptr,
                                        bits, tidx_info);
         }
@@ -625,6 +621,7 @@ fw_step2_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4
     }
 }
 
+template <bool FIELD = false>
 __global__ void __launch_bounds__(FW_BLOCK)
 fw_reset_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const uint8_t* __restrict__ mask,
                 float* __restrict__ obs, int bulk_ok, int emit_only) {
@@ -639,7 +636,7 @@ fw_reset_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const uint8_
         fw_load(pl, i, e);
         const bool sel = !emit_only && (mask == nullptr || mask[i] != 0);
         if (sel) {
-            fw_reset_env(p, pl, e, i, p.env_id0 + (uint32_t)i, e.episode + 1u);
+            fw_reset_env<FIELD>(p, pl, e, i, p.env_id0 + (uint32_t)i, e.episode + 1u);
             pl.ep_ret[i] = 0.0f;
             fw_store(pl, i, e);
         }
@@ -662,13 +659,13 @@ fw_reset_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const uint8_
 
 // reset of the lanes with `doing` set: begin_reset, waypoints, duck/obstacles, warm-up with the camera frame PyFlyt
 // captures at physics step 12 of it, then the compute_state of end_reset (fixedwing_waypoint_objlock_env.py:170-195)
-template <int TASK>
+template <int TASK, bool FIELD = false>
 __device__ __forceinline__ void ol_reset_lanes(const FwDev& p, const FwPlanes& pl, bool doing, EnvState& e, OlState& ol,
                                                float* so, float* depth_row, float* hs, int i, uint32_t gid, uint32_t episode,
                                                int tid) {
     float4 w0 = make_float4(0.f, 0.f, 0.f, 0.f), w1 = w0;
     if (doing) {
-        fw_reset_begin(p, pl, e, i, gid, episode, w0, w1);
+        fw_reset_begin<FIELD>(p, pl, e, i, gid, episode, w0, w1);
         if (TASK == 2) {
             fw_sample_targets(p, pl, i, gid, episode);
             ol_reset(p, pl, ol, i, gid, episode, so, tid, FW_BLOCK);
@@ -681,7 +678,7 @@ __device__ __forceinline__ void ol_reset_lanes(const FwDev& p, const FwPlanes& p
     while (dn < p.warmup_substeps) {                       // trip count depends on the config only: warp-uniform
         int next = p.warmup_substeps;
         if (p.cam_interval > 0) next = min(next, (dn / p.cam_interval + 1) * p.cam_interval);
-        if (doing) fw_warm(p, e, w0, w1, next - dn, false);
+        if (doing) fw_warm<FIELD>(p, e, w0, w1, next - dn, false);
         dn = next;
         const bool need = doing && p.cam_interval > 0 && dn % p.cam_interval == 0 && dn % p.substeps_per_inner == 0;
         ol_capture_warp(p, need, e, ol, so, tid, FW_BLOCK, depth_row);
@@ -794,7 +791,7 @@ __device__ __forceinline__ void ol_write_obs(const FwDev& p, const FwPlanes& pl,
 // without a valid spare (first episodes after an injected state, two finishes in quick succession, FWSIM_SPARE=0) run the
 // reset inline.  (Inlined: out-of-line versions -- `e` / `ol` passed through local copies, or the refill as a role of this
 // kernel's leading blocks -- measured 3-15 % slower: the step kernel is sensitive to its stack frame, profiles/r2_objlock.md.)
-template <int TASK>
+template <int TASK, bool FIELD = false>
 __device__ __forceinline__ void ol_finish_episode(const FwDev& p, const FwPlanes& pl, bool done, uint32_t info, EnvState& e,
                                                       OlState& ol, float4& w0, float4& w1, float& ep_ret, float* so,
                                                       float* depth_row, float* hs, int i, uint32_t gid, float* row,
@@ -822,7 +819,7 @@ __device__ __forceinline__ void ol_finish_episode(const FwDev& p, const FwPlanes
         atomicAdd(&pl.stats[inline_reset ? 10 : 9], 1.0);      // fw_spare_stats: resets served inline / from a spare
     }
     if (__any_sync(0xffffffffu, inline_reset))
-        ol_reset_lanes<TASK>(p, pl, inline_reset, e, ol, so, depth_row, hs, i, gid, e.episode + 1u, tid);
+        ol_reset_lanes<TASK, FIELD>(p, pl, inline_reset, e, ol, so, depth_row, hs, i, gid, e.episode + 1u, tid);
     if (done) {
         if (p.wind_mode != 0 && inline_reset) { w0 = pl.w0[i]; w1 = pl.w1[i]; }
         if (row != nullptr) ol_write_obs<TASK>(p, pl, e, ol, hs, i, 0, 0.f, 0.f, 0.f, 0.f, row, tid);
@@ -833,7 +830,7 @@ __device__ __forceinline__ void ol_finish_episode(const FwDev& p, const FwPlanes
 }
 
 // one agent step for the whole warp; `active` = lane owns an env
-template <int TASK, bool STD>
+template <int TASK, bool STD, bool FIELD = false>
 __device__ __forceinline__ float fw_env_step_objlock(const FwDev& p, const FwPlanes& pl, bool active, EnvState& e, OlState& ol,
                                                      float* so, float* depth_row, float* hs, int i, uint32_t gid, float a0, float a1,
                                                      float a2, float a3, float4& w0, float4& w1, float& ep_ret, float* row,
@@ -870,10 +867,17 @@ __device__ __forceinline__ float fw_env_step_objlock(const FwDev& p, const FwPla
                     const int q = ps & 3;
                     nz = q == 0 ? n0 : (q == 1 ? n1 : (q == 2 ? n2 : n3));
                 }
-                float wx, wy, wz;
-                fw_wind(p, ps, w0, w1, wx, wy, wz);
-                contact = contact || ol_contact(p, e, ol, so, tid, FW_BLOCK, cand, duck_near);    // pose
-                fw_substep<STD>(p, e, cmd, wx, wy, wz, nz, contact);
+                if (FIELD) {
+                    FwFieldT ft;
+                    fw_field_time(p, ps, w0, ft);
+                    contact = contact || ol_contact(p, e, ol, so, tid, FW_BLOCK, cand, duck_near);    // pose
+                    fw_substep<STD, true>(p, e, cmd, 0.0f, 0.0f, 0.0f, nz, contact, ft);
+                } else {
+                    float wx, wy, wz;
+                    fw_wind(p, ps, w0, w1, wx, wy, wz);
+                    contact = contact || ol_contact(p, e, ol, so, tid, FW_BLOCK, cand, duck_near);    // pose
+                    fw_substep<STD>(p, e, cmd, wx, wy, wz, nz, contact);
+                }
             }
         }
         // drone.update_last(): camera frame every cam_interval physics steps
@@ -942,7 +946,7 @@ __device__ __forceinline__ float fw_env_step_objlock(const FwDev& p, const FwPla
     if (active) ep_ret += reward;
     if (__any_sync(0xffffffffu, done)) {
         const uint32_t info = (fault ? 1u : 0u) | (col ? 2u : 0u) | (oob ? 4u : 0u) | (complete ? 8u : 0u) | (strike ? 16u : 0u);
-        ol_finish_episode<TASK>(p, pl, done, info, e, ol, w0, w1, ep_ret, so, depth_row, hs, i, gid, row, term_obs_row);
+        ol_finish_episode<TASK, FIELD>(p, pl, done, info, e, ol, w0, w1, ep_ret, so, depth_row, hs, i, gid, row, term_obs_row);
     }
     bits = (term ? 1u : 0u) | (trunc ? 2u : 0u) | (col ? 4u : 0u) | (oob ? 8u : 0u) | (complete ? 16u : 0u) | (strike ? 32u : 0u) |
            (fault ? 64u : 0u);
@@ -960,7 +964,7 @@ __device__ __forceinline__ void ol_smem_carve(const FwDev& p, float* stage, floa
 
 // launch bound 7 blocks/SM x 64 threads (register cap 146; ptxas settles at 128 with ~70 bytes of spills, so 8 blocks fit):
 // 148 x 448 = 66,304 >= 65,536 envs, a single wave either way
-template <bool RANDOM_ACT, int TASK, bool STD>
+template <bool RANDOM_ACT, int TASK, bool STD, bool FIELD = false>
 __global__ void __launch_bounds__(FW_BLOCK, 7)
 fw_step_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4* __restrict__ act,
                        float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ flg,
@@ -1004,7 +1008,7 @@ fw_step_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const
                 a0 = a.x; a1 = a.y; a2 = a.z; a3 = a.w;
             }
         }
-        reward = fw_env_step_objlock<TASK, STD>(p, pl, active, e, ol, so, depth_row, hs, i, gid, a0, a1, a2, a3, w0, w1, ep_ret,
+        reward = fw_env_step_objlock<TASK, STD, FIELD>(p, pl, active, e, ol, so, depth_row, hs, i, gid, a0, a1, a2, a3, w0, w1, ep_ret,
                                      (st == nsteps - 1) ? row : nullptr,
                                      (!RANDOM_ACT && term_obs != nullptr && row != nullptr && active) ? term_obs + (size_t)i * D : nullptr,
                                      bits, tidx_info);
@@ -1026,7 +1030,7 @@ fw_step_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const
     }
 }
 
-template <int TASK>
+template <int TASK, bool FIELD = false>
 __global__ void __launch_bounds__(FW_BLOCK)
 fw_reset_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const uint8_t* __restrict__ mask,
                         float* __restrict__ obs, int bulk_ok, int emit_only) {
@@ -1046,7 +1050,7 @@ fw_reset_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, cons
         if (TASK == 4) ol_hist_load(p, pl, i, hs, threadIdx.x, FW_BLOCK);
     }
     const bool sel = active && !emit_only && (mask == nullptr || mask[i] != 0);
-    ol_reset_lanes<TASK>(p, pl, sel, e, ol, so, depth_row, hs, i, p.env_id0 + (uint32_t)i, e.episode + 1u, threadIdx.x);
+    ol_reset_lanes<TASK, FIELD>(p, pl, sel, e, ol, so, depth_row, hs, i, p.env_id0 + (uint32_t)i, e.episode + 1u, threadIdx.x);
     if (sel) {
         pl.ep_ret[i] = 0.0f;
         fw_store(pl, i, e);
@@ -1067,7 +1071,7 @@ fw_reset_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, cons
 // clears the list's counter for the step launch that appends to it next.
 // whole_batch > 0: episode (live episode + 1) of every env 0..whole_batch-1, full warps (fw_create, right after the first reset).
 #define FW_REFILL_GRID 64
-template <int TASK>
+template <int TASK, bool FIELD = false>
 __global__ void __launch_bounds__(FW_BLOCK, 7)
 fw_refill_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const int2* __restrict__ list,
                          int* __restrict__ count, int* __restrict__ blocks_done, int cap, int whole_batch) {
@@ -1087,7 +1091,7 @@ fw_refill_objlock_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, con
         const int i = ent.x;
         EnvState e = {};
         OlState ol = {};
-        ol_reset_lanes<TASK>(p, sv, doing, e, ol, so, depth_row, hs, i, p.env_id0 + (uint32_t)i, (uint32_t)ent.y, threadIdx.x);
+        ol_reset_lanes<TASK, FIELD>(p, sv, doing, e, ol, so, depth_row, hs, i, p.env_id0 + (uint32_t)i, (uint32_t)ent.y, threadIdx.x);
         if (doing) {
             sv.s0[i] = make_float4(e.px, e.py, e.pz, e.thr);
             sv.s1[i] = make_float4(e.qx, e.qy, e.qz, e.qw);
@@ -1156,10 +1160,32 @@ static bool packed_enabled(const FwDev& p) {
     return p.packed != 0;
 }
 
+// the gridded-wind (FIELD) instantiations of the one-env kernels, selected by wind_mode 3
+static fw_step_fn step_fn_field(const FwDev& p, bool random_act) {
+    const int task = p.task;
+    const bool sg = p.std_geom != 0;
+    const bool r = random_act;
+    switch (task) {
+    case 0: return sg ? (r ? fw_step_kernel<0, true, true, true> : fw_step_kernel<0, false, true, true>)
+                      : (r ? fw_step_kernel<0, true, false, true> : fw_step_kernel<0, false, false, true>);
+    case 1: return sg ? (r ? fw_step_kernel<1, true, true, true> : fw_step_kernel<1, false, true, true>)
+                      : (r ? fw_step_kernel<1, true, false, true> : fw_step_kernel<1, false, false, true>);
+    case 3: return sg ? (r ? fw_step_kernel<3, true, true, true> : fw_step_kernel<3, false, true, true>)
+                      : (r ? fw_step_kernel<3, true, false, true> : fw_step_kernel<3, false, false, true>);
+    case 2: return sg ? (r ? fw_step_objlock_kernel<true, 2, true, true> : fw_step_objlock_kernel<false, 2, true, true>)
+                      : (r ? fw_step_objlock_kernel<true, 2, false, true> : fw_step_objlock_kernel<false, 2, false, true>);
+    case 4: return sg ? (r ? fw_step_objlock_kernel<true, 4, true, true> : fw_step_objlock_kernel<false, 4, true, true>)
+                      : (r ? fw_step_objlock_kernel<true, 4, false, true> : fw_step_objlock_kernel<false, 4, false, true>);
+    default: return nullptr;
+    }
+}
+
 static StepLaunch step_launch(const FwDev& p, bool random_act) {
     const int task = p.task;
     const bool std_geom = p.std_geom != 0;
     fw_step_fn fn = nullptr;
+    // gridded wind: one env per thread (the packed path does not sample fields)
+    if (p.wind_mode == 3) return StepLaunch{step_fn_field(p, random_act), FW_BLOCK, FW_BLOCK, stage_bytes(p)};
     // two envs per thread on the packed fp32x2 path: standard layout, no quaternion step limiter (fw_pack.cuh)
     if (std_geom && !p.quat_limiter && packed_enabled(p) && (task == 0 || task == 1 || task == 3)) {
         if (task == 0) fn = random_act ? fw_step2_kernel<0, true> : fw_step2_kernel<0, false>;
@@ -1236,6 +1262,12 @@ cudaError_t fwk_graph_add_random_step(cudaGraph_t g, cudaGraphNode_t* deps, int 
     return cudaGraphAddDependencies_v2(g, deps, out, &ed, 1);
 }
 
+typedef void (*fw_refill_fn)(const FwDev, const FwPlanes, const int2*, int*, int*, int, int);
+static fw_refill_fn refill_fn(const FwDev& p) {
+    if (p.wind_mode == 3) return p.task == 2 ? fw_refill_objlock_kernel<2, true> : fw_refill_objlock_kernel<4, true>;
+    return p.task == 2 ? fw_refill_objlock_kernel<2> : fw_refill_objlock_kernel<4>;
+}
+
 static int refill_grid(int work, bool whole_batch) {
     const int per_block = (FW_BLOCK / 32) * (whole_batch ? 32 : OL_REFILL_PER_WARP);
     const int grid = (work + per_block - 1) / per_block;
@@ -1247,7 +1279,7 @@ static int refill_grid(int work, bool whole_batch) {
 cudaError_t fwk_launch_refill(const FwDev& p, const FwPlanes& pl, const int2* list, int* count, int* blocks_done, int cap,
                               int whole_batch, cudaStream_t st) {
     if (p.task != 2 && p.task != 4) return cudaErrorNotSupported;
-    auto fn = p.task == 2 ? fw_refill_objlock_kernel<2> : fw_refill_objlock_kernel<4>;
+    auto fn = refill_fn(p);
     if (!smem_opt_in((const void*)fn, stage_bytes(p))) return cudaErrorInvalidValue;
     fn<<<refill_grid(whole_batch > 0 ? whole_batch : cap, whole_batch > 0), FW_BLOCK, stage_bytes(p), st>>>(p, pl, list, count, blocks_done,
                                                                                                           cap, whole_batch);
@@ -1256,7 +1288,7 @@ cudaError_t fwk_launch_refill(const FwDev& p, const FwPlanes& pl, const int2* li
 
 cudaError_t fwk_graph_add_refill(cudaGraph_t g, cudaGraphNode_t* deps, int ndeps, const FwDev& p, const FwPlanes& pl,
                                  const int2* list, int* count, int* blocks_done, int cap, cudaGraphNode_t* out) {
-    auto fn = p.task == 2 ? fw_refill_objlock_kernel<2> : fw_refill_objlock_kernel<4>;
+    auto fn = refill_fn(p);
     if (!smem_opt_in((const void*)fn, stage_bytes(p))) return cudaErrorInvalidValue;
     FwDev pc = p; FwPlanes plc = pl;
     const int2* l = list; int* c = count; int* bd = blocks_done; int cap_ = cap, wb = 0;
@@ -1283,11 +1315,16 @@ cudaError_t fwk_graph_add_refill(cudaGraph_t g, cudaGraphNode_t* deps, int ndeps
 cudaError_t fwk_launch_reset(const FwDev& p, const FwPlanes& pl, const uint8_t* mask, float* obs, bool emit_only,
                              cudaStream_t st) {
     const int bulk_ok = (obs != nullptr) && ((reinterpret_cast<uintptr_t>(obs) & 15u) == 0);
+    const bool field = p.wind_mode == 3;
     if (p.task == 2 || p.task == 4) {
-        auto fn = p.task == 2 ? fw_reset_objlock_kernel<2> : fw_reset_objlock_kernel<4>;
+        auto fn = field ? (p.task == 2 ? fw_reset_objlock_kernel<2, true> : fw_reset_objlock_kernel<4, true>)
+                        : (p.task == 2 ? fw_reset_objlock_kernel<2> : fw_reset_objlock_kernel<4>);
         if (!smem_opt_in((const void*)fn, stage_bytes(p))) return cudaErrorInvalidValue;
         fn<<<grid_for(p.n), FW_BLOCK, stage_bytes(p), st>>>(p, pl, mask, obs, bulk_ok, emit_only ? 1 : 0);
-    } else fw_reset_kernel<<<grid_for(p.n), FW_BLOCK, stage_bytes(p), st>>>(p, pl, mask, obs, bulk_ok, emit_only ? 1 : 0);
+    } else {
+        auto fn = field ? fw_reset_kernel<true> : fw_reset_kernel<false>;
+        fn<<<grid_for(p.n), FW_BLOCK, stage_bytes(p), st>>>(p, pl, mask, obs, bulk_ok, emit_only ? 1 : 0);
+    }
     return cudaGetLastError();
 }
 

@@ -23,6 +23,13 @@ from .config import (EnvConfig, FLAG_COLLISION, FLAG_COMPLETE, FLAG_OOB, FLAG_ST
 from .vec_env import FixedwingVecEnv
 
 
+def _field_of(wind_config: dict | None):
+    """The WindField of a wind_config dict in mode "field" (None otherwise); _wind_fields validates the dict."""
+    if wind_config and wind_config.get("enabled", False) and str(wind_config.get("mode", "")).lower() == "field":
+        return wind_config["field"]
+    return None
+
+
 def _quat_to_mat(q: np.ndarray) -> np.ndarray:
     x, y, z, w = (float(v) for v in q)
     s = 2.0 / (x * x + y * y + z * z + w * w)
@@ -62,11 +69,22 @@ class _AviaryView:
     def __init__(self, owner: "FixedwingWaypointsEnv"):
         self._o = owner
 
-    def register_wind_field_function(self, wind_field) -> None:
-        raise NotImplementedError(
-            "Python wind closures cannot run inside the CUDA step; pass the same wind_config dict the reference feeds "
-            "to _register_wind_field (envs/utils.py:141-205) to FixedwingWaypointsEnv(wind_config=...) or call "
-            "env.set_wind_config(dict) -- constant and gust_sine fields with per-reset randomisation are built in.")
+    def register_wind_field_function(self, wind_field, *, origin=None, spacing=None, shape=None, n_slices: int = 1,
+                                     t_step: float | None = None) -> None:
+        """PyFlyt's hook for a custom wind ``f(time_s, positions[n, 3]) -> [n, 3]``.  A Python closure cannot run inside
+        the CUDA step: with the lattice keywords the function is sampled once (``WindField.from_function``) and the
+        gridded field is flown from the next ``reset()`` on, interpolated at every lifting surface."""
+        if origin is None or spacing is None or shape is None:
+            raise NotImplementedError(
+                "Python wind closures cannot run inside the CUDA step: pass the sampling lattice, "
+                "register_wind_field_function(f, origin=(x, y, z), spacing=metres, shape=(nx, ny, nz)[, n_slices=, "
+                "t_step=]), and f is sampled once into a gridded field (pyflyt_drone_b200.wind.WindField); or pass the "
+                "wind_config dict the reference feeds to _register_wind_field (envs/utils.py:141-205) to the env or to "
+                "env.set_wind_config(dict).")
+        from .wind import WindField
+        field = WindField.from_function(wind_field, origin=origin, spacing=spacing, shape=shape, n_slices=n_slices,
+                                        t_step=t_step)
+        self._o.set_wind_config({"enabled": True, "mode": "field", "field": field})
 
     def state(self, index: int = 0) -> np.ndarray:
         return self._o._raw_state()
@@ -124,7 +142,8 @@ class FixedwingWaypointsEnv:
         if task == "waypoints" and wind_config is not None:
             self.cfg = self.cfg.replace(**_wind_fields(wind_config, "env"))
         self._device, self._seed0 = device, int(seed)
-        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=self._seed0)
+        self._wind_field = _field_of(wind_config)
+        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=self._seed0, wind_field=self._wind_field)
         att = (12 if self.cfg.angle_repr == 0 else 13) + 4 + 6
         self._att = att
         self.attitude_space = spaces.Box(low=-np.inf, high=np.inf, shape=(att - 10,), dtype=np.float64)
@@ -198,8 +217,9 @@ class FixedwingWaypointsEnv:
     def set_wind_config(self, wind_config: dict | None) -> None:
         """What WindOnResetWrapper does for the reference: takes effect from the next reset()."""
         self.cfg = self.cfg.replace(**_wind_fields(wind_config, "wrapper"))
+        self._wind_field = _field_of(wind_config)
         self._vec.close()
-        self._vec = FixedwingVecEnv(1, config=self.cfg, device=self._device, seed=self._seed0)
+        self._vec = FixedwingVecEnv(1, config=self.cfg, device=self._device, seed=self._seed0, wind_field=self._wind_field)
         self._needs_reset = True
         self._auto_reset_done = False
 
@@ -273,7 +293,7 @@ class FixedwingLowLevelEnv:
         if render_mode is not None:
             raise ValueError("rendering is out of scope for the batched simulator")
         self.cfg: EnvConfig = make_config("lowlevel", wind=wind_config)
-        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=int(seed))
+        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=int(seed), wind_field=_field_of(wind_config))
         self.observation_space = spaces.Box(low=-np.inf, high=np.inf, shape=(21,), dtype=np.float64)
         self.action_space = spaces.Box(low=-1.0, high=1.0, shape=(6,), dtype=np.float64)
         self.prev_action = np.zeros(6)
@@ -380,7 +400,7 @@ class FixedwingObjLockEnv:
         self.cfg: EnvConfig = make_config("objlock_duck", wind=wind_config if wind_config is not None else {"enabled": False},
                                           **over)
         self._device, self._seed0 = device, int(seed)
-        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=self._seed0)
+        self._vec = FixedwingVecEnv(1, config=self.cfg, device=device, seed=self._seed0, wind_field=_field_of(wind_config))
         att = (12 if self.cfg.angle_repr == 0 else 13) + 4 + 6
         self._att = att
         self.combined_space = spaces.Box(low=-np.inf, high=np.inf, shape=(att,), dtype=np.float64)

@@ -670,7 +670,7 @@ class PPO:
         if own:
             n = max(1, min(self.n_envs, int(n_eval_episodes)))
             env = FixedwingVecEnv(n, config=self.env.cfg, device=self.env.device_index, seed=self.seed + 7919,
-                                  env_id0=self.env.env_id0 + (1 << 24))
+                                  env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None))
         obs = env.reset_tensor()
         n = env.num_envs
         quota = torch.tensor(self.episode_quotas(n_eval_episodes, n), dtype=torch.int64, device=self.device)

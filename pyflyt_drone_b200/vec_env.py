@@ -24,6 +24,7 @@ from .compat import spaces
 from .compat.vec_env import VecEnv
 from .config import (EnvConfig, FLAG_COLLISION, FLAG_COMPLETE, FLAG_FAULT, FLAG_OOB, FLAG_STRIKE, FLAG_TERM, FLAG_TRUNC,
                      make_config)
+from .wind import WindField
 
 _STATE_FIELDS = {
     "pos": (np.float32, 3), "quat": (np.float32, 4), "vel": (np.float32, 3), "omega": (np.float32, 3),
@@ -49,10 +50,19 @@ class FixedwingVecEnv(VecEnv):
     metadata = {"render_modes": []}
 
     def __init__(self, num_envs: int, preset: str = "waypoints_v3", config: EnvConfig | None = None,
-                 device: int = 0, seed: int = 0, env_id0: int = 0, info_mode: str = "auto", **overrides):
+                 device: int = 0, seed: int = 0, env_id0: int = 0, info_mode: str = "auto", wind_field: WindField | None = None,
+                 **overrides):
         self.cfg = config if config is not None else make_config(preset, **overrides)
         if config is not None and overrides:
             self.cfg = self.cfg.replace(**overrides)
+        # gridded wind (wind_mode 3): the config keeps its wind_start_substep / wind_randomize; the field is installed by _open()
+        if wind_field is not None:
+            if not isinstance(wind_field, WindField):
+                raise TypeError("wind_field must be a pyflyt_drone_b200.wind.WindField")
+            self.cfg = self.cfg.replace(wind_mode=3)
+        elif self.cfg.wind_mode == 3:
+            raise ValueError("wind_mode 3 (gridded field) needs wind_field=WindField(...)")
+        self.wind_field = wind_field
         self.num_envs = int(num_envs)
         self.device_index = int(device)
         self._seed = int(seed)
@@ -76,6 +86,14 @@ class FixedwingVecEnv(VecEnv):
         self._h = C.c_void_p()
         _lib.check(self.lib.fw_create(C.byref(self._c_cfg), self.num_envs, self.device_index, self._seed,
                                       self.env_id0, C.byref(self._h)))
+        if self.wind_field is not None:
+            desc = self.wind_field.to_c()
+            rc = self.lib.fw_set_wind_field(self._h, C.byref(desc))
+            if rc != 0:
+                msg = self.lib.fw_last_error()
+                self.lib.fw_destroy(self._h)
+                self._h = C.c_void_p()
+                raise _lib.FwError(f"libfwsim error {rc}: {msg.decode() if msg else '?'}")
         self.obs_dim = int(self.lib.fw_obs_dim(self._h))
         self.act_dim = int(self.lib.fw_act_dim(self._h))     # 4, or 6 for the low-level task
         D = max(self.obs_dim, 1)
