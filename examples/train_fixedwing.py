@@ -52,6 +52,8 @@ def main():
     ap.add_argument("--batch_size", type=int, default=None)
     ap.add_argument("--total_timesteps", type=int, default=None)
     ap.add_argument("--pretrained_model", type=str, default=None)
+    ap.add_argument("--eval_freq", type=int, default=10_000, help="timesteps between evaluations (20 episodes each)")
+    ap.add_argument("--save_freq", type=int, default=50_000, help="timesteps between checkpoints")
     args = ap.parse_args()
     cfg = dict(TRAIN_CONFIG[args.task])
     for k in ("num_envs", "n_steps", "batch_size", "total_timesteps"):
@@ -65,6 +67,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
 
+    from pyflyt_drone_b200.callbacks import CheckpointCallback, EvalCallback
     from pyflyt_drone_b200.ppo import PPO
     from pyflyt_drone_b200.vec_env import FixedwingVecEnv
 
@@ -83,11 +86,18 @@ def main():
                 verbose=1 if rank == 0 else 0)
     if args.pretrained_model:
         model.load(args.pretrained_model)
+    # the reference's WaypointEvalCallback(eval_freq=10000 // num_envs, n_eval_episodes=20, best_model_save_path=model_dir)
+    # and CheckpointCallback(save_freq=50000 // num_envs); here both frequencies count timesteps (rank 0 evaluates and writes)
+    eval_cb = EvalCallback(eval_freq=args.eval_freq, n_eval_episodes=20, best_model_save_path=cfg["model_dir"],
+                           log_path=os.path.join(cfg["model_dir"], "eval_logs"), verbose=1)
+    ckpt_cb = CheckpointCallback(save_freq=args.save_freq, save_path=os.path.join(cfg["model_dir"], "checkpoints"),
+                                 name_prefix="ppo_fixedwing")
     try:
-        model.learn(total_timesteps=cfg["total_timesteps"])
+        model.learn(total_timesteps=cfg["total_timesteps"], callback=lambda l, g: eval_cb(l, g) and ckpt_cb(l, g))
     except KeyboardInterrupt:
         print("Training interrupted by user.")
     finally:
+        eval_cb.close()
         if rank == 0:
             os.makedirs(cfg["model_dir"], exist_ok=True)
             model.save(os.path.join(cfg["model_dir"], "final_model.pt"))
@@ -95,9 +105,10 @@ def main():
             paths = model.export_sb3(os.path.join(cfg["model_dir"], "sb3_export"))      # policy.pth + vecnorm.npz for SB3
             print("exported", paths)
             # the reference's eval flow (eval/eval_waypoints.py): frozen statistics, raw returns, deterministic actions
-            mean_r, std_r, mean_len, targets = model.evaluate_policy(n_eval_episodes=100)
-            print(f"evaluation over 100 episodes: reward {mean_r:.2f} +/- {std_r:.2f}, length {mean_len:.1f}, "
-                  f"targets reached per episode {targets:.2f}")
+            res = model.evaluate(n_eval_episodes=100)
+            print(f"evaluation over 100 episodes: reward {res.mean_reward:.2f} +/- {res.std_reward:.2f}, length "
+                  f"{res.mean_length:.1f}, targets reached per episode {res.mean_targets_reached:.2f}, "
+                  f"success rate {res.success_rate:.2f}")
         env.close()
         if world > 1:
             dist.destroy_process_group()

@@ -83,6 +83,24 @@ int ppo_timeout_bootstrap_a(const float* params, int32_t d, int32_t a, const flo
 /* counter[0] += inc on the device (one node of the rollout graph). */
 int ppo_counter_add(uint32_t* counter, uint32_t inc, void* stream);
 
+/* Per-episode bookkeeping of stable_baselines3 evaluate_policy on the device, one thread per env, one launch per agent
+ * step (after the step that produced rew / flags).  The eval step index is step + *step_dev (the ppo_policy_forward
+ * convention, so a captured chunk of steps replays with ppo_counter_add advancing step_dev); steps at or after
+ * step_limit record and accumulate nothing.
+ *   rew [n], flags [n]      the step's rewards and flag bytes
+ *   targets_reached [n]     the pre-reset num_targets_reached plane (fw_targets_reached); NULL = task without targets
+ *   ret [n] (double), len [n], count [n]   running return (ret += (double)rew), length, episodes recorded so far
+ *   quota [n], offset [n]   episodes env i records (SB3: (n_eval_episodes + i) // n) and its first slot in the table
+ *   remaining               envs with count < quota; decremented (atomically) when an env fills its quota
+ * An env whose episode ends (flags & 3) while count < quota writes slot offset + count of the episode table:
+ * ep_return (return), ep_length (length), ep_targets (targets reached, 0 without a plane), ep_flags (the terminal step's
+ * flag byte), ep_step (eval step index of the episode's last step).  Every ended episode then zeroes ret and len.  The
+ * slot depends only on the env and its episode number: the table is bit-reproducible. */
+int ppo_eval_ledger(const float* rew, const uint8_t* flags, const uint8_t* targets_reached, int32_t n, double* ret,
+                    int32_t* len, int32_t* count, const int32_t* quota, const int32_t* offset, uint32_t step,
+                    const uint32_t* step_dev, int32_t step_limit, int32_t* remaining, double* ep_return, int32_t* ep_length,
+                    uint8_t* ep_targets, uint8_t* ep_flags, int32_t* ep_step, void* stream);
+
 /* Value tower only (last_values of a rollout). */
 int ppo_value_forward(const float* params, int32_t d, const float* obs_raw, const double* obs_stats, float clip_obs,
                       int32_t n, float* value, void* stream);

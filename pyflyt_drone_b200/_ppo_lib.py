@@ -18,6 +18,8 @@ PPO_SYMBOLS = [
     ("ppo_policy_forward_tc", C.c_int, [_P, C.c_int32, _P, _P, _F, C.c_int32, C.c_uint64, C.c_uint32, C.c_uint32, _P,
                                         C.c_int32, _P, _P, _P, _P, _P, _P]),
     ("ppo_counter_add", C.c_int, [_P, C.c_uint32, _P]),
+    ("ppo_eval_ledger", C.c_int, [_P, _P, _P, C.c_int32, _P, _P, _P, _P, _P, C.c_uint32, _P, C.c_int32, _P, _P, _P, _P, _P, _P,
+                                  _P]),
     ("ppo_moments_finalize", C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),
     ("ppo_random_permutation", C.c_int, [_P, C.c_int64, C.c_uint64, C.c_uint64, _P]),
     ("ppo_random_permutation_window", C.c_int, [_P, C.c_int64, C.c_uint64, _P, C.c_int64, _P]),

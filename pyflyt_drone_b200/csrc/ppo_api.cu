@@ -220,6 +220,20 @@ extern "C" int ppo_counter_add(uint32_t* counter, uint32_t inc, void* stream) {
     return FW_OK;
 }
 
+extern "C" int ppo_eval_ledger(const float* rew, const uint8_t* flags, const uint8_t* targets_reached, int32_t n, double* ret,
+                               int32_t* len, int32_t* count, const int32_t* quota, const int32_t* offset, uint32_t step,
+                               const uint32_t* step_dev, int32_t step_limit, int32_t* remaining, double* ep_return,
+                               int32_t* ep_length, uint8_t* ep_targets, uint8_t* ep_flags, int32_t* ep_step, void* stream) {
+    if (!rew || !flags || !ret || !len || !count || !quota || !offset || !step_dev || !remaining || !ep_return || !ep_length ||
+        !ep_targets || !ep_flags || !ep_step)
+        return pfail(FW_EINVAL, "null argument");
+    if (n <= 0) return pfail(FW_EINVAL, "n must be positive");
+    if (step_limit < 0) return pfail(FW_EINVAL, "step_limit must not be negative");
+    PCU(ppok_eval_ledger(rew, flags, targets_reached, n, ret, len, count, quota, offset, step, step_dev, step_limit, remaining,
+                         ep_return, ep_length, ep_targets, ep_flags, ep_step, (cudaStream_t)stream));
+    return FW_OK;
+}
+
 // workspace layout (floats): [0,8) arrival counter of the reduce+Adam kernel (unsigned, starts zeroed) + pad | [8,16) adv stats
 // of a single-minibatch call | [16, 16 + 160*P) per-CTA gradient partials | 160*8 per-CTA loss statistics | PPO_MAX_WINDOW
 // scratch slices of PPO_ADV_SCRATCH floats (doubles: arrival counter + 592 block partials; the counters start zeroed and

@@ -565,3 +565,48 @@ cudaError_t ppok_counter_add(uint32_t* ctr, uint32_t inc, cudaStream_t st) {
     ppo_counter_add_kernel<<<1, 32, 0, st>>>(ctr, inc);
     return cudaGetLastError();
 }
+
+// ------------------------------------------------------------------ evaluation ledger (evaluate_policy's bookkeeping)
+// One thread per env.  The return is summed in double in step order, as the host loop of PPO.evaluate_policy does
+// (ret += rew.double()), so recorded returns are bit-identical to it.  The table slot of an episode is fixed by its env and
+// episode number; the only atomic is the count of envs still below quota, which the host polls once per chunk of steps.
+__global__ void __launch_bounds__(256)
+ppo_eval_ledger_kernel(const float* __restrict__ rew, const uint8_t* __restrict__ flags, const uint8_t* __restrict__ tidx, int n,
+                       double* __restrict__ ret, int* __restrict__ len, int* __restrict__ count, const int* __restrict__ quota,
+                       const int* __restrict__ offset, uint32_t step, const uint32_t* __restrict__ step_dev, int step_limit,
+                       int* __restrict__ remaining, double* __restrict__ ep_ret, int* __restrict__ ep_len,
+                       uint8_t* __restrict__ ep_tr, uint8_t* __restrict__ ep_flags, int* __restrict__ ep_step) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t s = step + step_dev[0];
+    if (s >= (uint32_t)step_limit) return;
+    double r = ret[i] + (double)rew[i];
+    int l = len[i] + 1;
+    const uint8_t f = flags[i];
+    if (f & 3u) {
+        const int c = count[i], q = quota[i];
+        if (c < q) {
+            const size_t slot = (size_t)offset[i] + (size_t)c;
+            ep_ret[slot] = r;
+            ep_len[slot] = l;
+            ep_tr[slot] = tidx != nullptr ? tidx[i] : (uint8_t)0;
+            ep_flags[slot] = f;
+            ep_step[slot] = (int)s;
+            count[i] = c + 1;
+            if (c + 1 == q) atomicSub(remaining, 1);
+        }
+        r = 0.0;
+        l = 0;
+    }
+    ret[i] = r;
+    len[i] = l;
+}
+
+cudaError_t ppok_eval_ledger(const float* rew, const uint8_t* flags, const uint8_t* tidx, int n, double* ret, int* len, int* count,
+                             const int* quota, const int* offset, uint32_t step, const uint32_t* step_dev, int step_limit,
+                             int* remaining, double* ep_ret, int* ep_len, uint8_t* ep_tr, uint8_t* ep_flags, int* ep_step,
+                             cudaStream_t st) {
+    ppo_eval_ledger_kernel<<<(n + 255) / 256, 256, 0, st>>>(rew, flags, tidx, n, ret, len, count, quota, offset, step, step_dev,
+                                                            step_limit, remaining, ep_ret, ep_len, ep_tr, ep_flags, ep_step);
+    return cudaGetLastError();
+}

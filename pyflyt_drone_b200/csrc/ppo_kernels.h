@@ -14,6 +14,10 @@ cudaError_t ppok_forward(const float* params, int d, const float* obs_raw, const
                          cudaStream_t st, const uint8_t* boot_flags = nullptr, float boot_gamma = 0.0f,
                          float* boot_rew = nullptr, int a = PPO_A);
 cudaError_t ppok_counter_add(uint32_t* ctr, uint32_t inc, cudaStream_t st);
+cudaError_t ppok_eval_ledger(const float* rew, const uint8_t* flags, const uint8_t* tidx, int n, double* ret, int* len, int* count,
+                             const int* quota, const int* offset, uint32_t step, const uint32_t* step_dev, int step_limit,
+                             int* remaining, double* ep_ret, int* ep_len, uint8_t* ep_tr, uint8_t* ep_flags, int* ep_step,
+                             cudaStream_t st);
 cudaError_t ppok_permutation(long long* out, long long n, uint64_t seed, uint64_t epoch, cudaStream_t st);
 cudaError_t ppok_permutation_window(long long* out, long long n, uint64_t seed, uint32_t* ctr, long long window_len, cudaStream_t st);
 cudaError_t ppok_moments(const float* x, int n, int d, double* stats, double* scratch, double* accum, cudaStream_t st);

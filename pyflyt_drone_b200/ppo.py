@@ -216,6 +216,109 @@ class RolloutStats:
     update_s: float = 0.0
 
 
+@dataclass
+class EvalResult:
+    """The episodes ``PPO.evaluate`` selected and the reference's evaluation metrics over them.
+
+    Per-episode arrays, in the order stable_baselines3's ``evaluate_policy`` appends episodes (finish step, then env index):
+    ``returns`` (float64, raw rewards summed in step order), ``lengths``, ``targets_reached`` (``info["num_targets_reached"]``
+    before the auto-reset; 0 on tasks without targets), ``flags`` (the flag byte of the episode's last step),
+    ``env_index`` and ``finish_step`` (evaluation step index of the last step).
+
+    The means are those of ``PPO.evaluate_policy``, computed the same way on the same device, so they agree bit for bit:
+    ``mean_reward``, ``std_reward`` (population), ``mean_length``, ``mean_targets_reached`` (0.0 without targets).  With no
+    finished episode every mean and rate is NaN.
+
+    The rates are the reference's ``eval/*`` metrics (SURVEY §5 "metrics / logging": what ``WaypointEvalCallback`` and the
+    ObjLock script's callback read from the info dict of each finished episode), as fractions of the episodes:
+      ``wp_reach_rate[i - 1]``  ``eval/wp{i}_reach_rate``: ``num_targets_reached >= i``, i = 1..num_targets (empty without
+                                targets)
+      ``success_rate``          ``eval/success_rate``: ``duck_strike`` on the ObjLock tasks (the duck-only env's
+                                ``is_success``), ``env_complete`` (every waypoint reached) on the others
+      ``duck_strike_rate``      ``eval/duck_strike_rate``: ``duck_strike``
+      ``collision_rate``, ``out_of_bounds_rate``  ``collision`` / ``out_of_bounds`` of the last step
+      ``truncation_rate``       ``TimeLimit.truncated``: time limit reached without termination
+    """
+    returns: np.ndarray
+    lengths: np.ndarray
+    targets_reached: np.ndarray
+    flags: np.ndarray
+    env_index: np.ndarray
+    finish_step: np.ndarray
+    task: int
+    num_targets: int
+    mean_reward: float
+    std_reward: float
+    mean_length: float
+    mean_targets_reached: float
+    wp_reach_rate: np.ndarray
+    success_rate: float
+    duck_strike_rate: float
+    collision_rate: float
+    out_of_bounds_rate: float
+    truncation_rate: float
+
+    @property
+    def has_targets(self) -> bool:
+        return self.task in (1, 2)
+
+    @property
+    def n_episodes(self) -> int:
+        return int(self.returns.shape[0])
+
+    @property
+    def successes(self) -> np.ndarray:
+        """Per-episode success (the definition of ``success_rate``)."""
+        from .config import FLAG_COMPLETE, FLAG_STRIKE
+        bit = FLAG_STRIKE if self.task in (2, 4) else FLAG_COMPLETE
+        return (self.flags & bit) != 0
+
+    @classmethod
+    def from_episodes(cls, returns, lengths, targets_reached, flags, env_index, finish_step, task: int, num_targets: int,
+                      device: str | torch.device = "cpu") -> "EvalResult":
+        """Orders the episodes by (finish step, env index) and computes the metrics; the means are reduced by torch on
+        ``device`` (the device ``evaluate_policy`` reduces on, for bitwise agreement with it)."""
+        from .config import FLAG_COLLISION, FLAG_OOB, FLAG_STRIKE, FLAG_TERM, FLAG_TRUNC
+        finish_step, env_index = np.asarray(finish_step, np.int32), np.asarray(env_index, np.int32)
+        order = np.lexsort((env_index, finish_step))
+        returns = np.asarray(returns, np.float64)[order]
+        lengths = np.asarray(lengths, np.int32)[order]
+        targets_reached = np.asarray(targets_reached, np.uint8)[order]
+        flags = np.asarray(flags, np.uint8)[order]
+        has_targets = task in (1, 2)
+        if not has_targets:
+            targets_reached = np.zeros_like(targets_reached)
+        nt = int(num_targets) if has_targets else 0
+        out = dict(returns=returns, lengths=lengths, targets_reached=targets_reached, flags=flags, env_index=env_index[order],
+                   finish_step=finish_step[order], task=int(task), num_targets=nt)
+        if returns.shape[0] == 0:
+            nan = float("nan")
+            return cls(**out, mean_reward=nan, std_reward=nan, mean_length=nan, mean_targets_reached=nan,
+                       wp_reach_rate=np.full(nt, nan), success_rate=nan, duck_strike_rate=nan, collision_rate=nan,
+                       out_of_bounds_rate=nan, truncation_rate=nan)
+        r = torch.from_numpy(returns).to(device)
+        rate = lambda m: float(np.count_nonzero(m)) / returns.shape[0]  # noqa: E731
+        res = cls(**out, mean_reward=float(r.mean()), std_reward=float(r.std(unbiased=False)),
+                  mean_length=float(torch.from_numpy(lengths).to(device).double().mean()),
+                  mean_targets_reached=float(torch.from_numpy(targets_reached).to(device).double().mean()) if has_targets else 0.0,
+                  wp_reach_rate=np.array([rate(targets_reached >= i) for i in range(1, nt + 1)], np.float64),
+                  success_rate=0.0, duck_strike_rate=rate(flags & FLAG_STRIKE), collision_rate=rate(flags & FLAG_COLLISION),
+                  out_of_bounds_rate=rate(flags & FLAG_OOB),
+                  truncation_rate=rate(((flags & FLAG_TRUNC) != 0) & ((flags & FLAG_TERM) == 0)))
+        res.success_rate = rate(res.successes)
+        return res
+
+    def metrics(self) -> dict[str, float]:
+        """The metrics under the names the reference's training scripts log (SURVEY §5 "metrics / logging")."""
+        m = {"eval/mean_reward": self.mean_reward, "eval/mean_ep_length": self.mean_length,
+             "eval/success_rate": self.success_rate}
+        for i, v in enumerate(self.wp_reach_rate, 1):
+            m[f"eval/wp{i}_reach_rate"] = float(v)
+        if self.task in (2, 4):
+            m["eval/duck_strike_rate"] = self.duck_strike_rate
+        return m
+
+
 class PPO:
     """Keyword-compatible with the reference's ``PPO("MlpPolicy", env, ...)`` call
     (train/train_Fixedwing_Waypoints_v3.py:293-310); ``env`` is a FixedwingVecEnv."""
@@ -289,6 +392,7 @@ class PPO:
         self._perm_ctr = torch.zeros(2, dtype=torch.int32, device=self.device)
         self._perm_epoch = 0
         self._obs = None               # raw observation tensor (view of the env's persistent buffer)
+        self._eval_state = None        # PPO.evaluate's buffers and captured chunk for its last eval env
         self._gen = torch.Generator(device=self.device).manual_seed(seed)
         self.stats = RolloutStats()
         self.world = 1
@@ -704,6 +808,112 @@ class PPO:
         ln = torch.cat(done_len).double()
         targets = float(torch.cat(done_tr).mean()) if done_tr else 0.0
         return float(r.mean()), float(r.std(unbiased=False)), float(ln.mean()), targets
+
+    # agent steps per evaluation chunk: the host reads the count of unfinished envs once per chunk.  Even, because the camera
+    # tasks alternate a refill parity on every step and a replayed chunk must end on the parity it was captured with.
+    EVAL_CHUNK = 32
+
+    def make_eval_env(self, n_eval_episodes: int) -> FixedwingVecEnv:
+        """The batch ``evaluate`` builds when given no env: the training env's configuration (and wind field) on a fresh batch
+        of at most ``n_eval_episodes`` envs, seed ``seed + 7919``, env ids from ``env_id0 + 2**24`` -- ``evaluate_policy``'s."""
+        n = max(1, min(self.n_envs, int(n_eval_episodes)))
+        return FixedwingVecEnv(n, config=self.env.cfg, device=self.env.device_index, seed=self.seed + 7919,
+                               env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None))
+
+    def evaluate(self, env=None, n_eval_episodes: int = 100, deterministic: bool = True,
+                 max_steps: int | None = None) -> EvalResult:
+        """``evaluate_policy`` with the bookkeeping on the device and the per-episode table it does not return.
+
+        Same arguments, defaults, own-env rule (``make_eval_env``), per-env quotas and episodes: every step runs the CUDA-core
+        forward of ``predict`` (frozen VecNormalize statistics, no moment accumulation), ``fw_step``, the copy of the pre-reset
+        targets-reached plane and ``ppo_eval_ledger``, which records each env's first ``quota`` finished episodes into a table
+        slot fixed by env and episode number.  Steps run in chunks of ``EVAL_CHUNK``; with ``use_cuda_graph`` a chunk is
+        captured once per eval env and replayed, and the host reads the count of envs below quota between chunks -- one sync
+        per chunk instead of one per step.  ``max_steps`` is exact: steps at or after it record nothing.
+
+        The episodes, and the four means (``EvalResult.mean_*``), are bit-identical to ``evaluate_policy``'s.  The env's state
+        afterwards is not: ``evaluate`` may step a caller-supplied env up to ``EVAL_CHUNK - 1`` steps past the step on which
+        the last needed episode ended, where ``evaluate_policy`` stops on that step.
+
+        ``deterministic=False`` samples the Gaussian policy with Philox noise keyed by the model seed and counted by the
+        evaluation's own step index (restarting at 0 on every call): the training counter and ``predict``'s call counter are
+        neither read nor advanced, so evaluating never changes what training draws."""
+        own = env is None
+        if own:
+            env = self.make_eval_env(n_eval_episodes)
+        try:
+            return self._evaluate(env, int(n_eval_episodes), bool(deterministic), max_steps)
+        finally:
+            if own:
+                self._eval_state = None            # the captured chunk names the env's buffers: it goes first
+                env.close()
+
+    def _evaluate(self, env, n_eval_episodes: int, deterministic: bool, max_steps: int | None) -> EvalResult:
+        n, K = env.num_envs, self.EVAL_CHUNK
+        quotas = np.asarray(self.episode_quotas(n_eval_episodes, n), np.int64)
+        limit = max_steps if max_steps is not None else int(quotas.max()) * (int(env.cfg.max_steps) + 2) + 8
+        limit = min(max(int(limit), 0), 2 ** 31 - 1)
+        key = (n_eval_episodes, deterministic, limit)
+        s = self._eval_state
+        if s is None or s["env"] is not env or s["key"] != key:
+            self._eval_state = None
+            dev = self.device
+            i32, f64 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.float64, device=dev)
+            E = max(int(quotas.sum()), 1)
+            s = dict(env=env, key=key, graph=None, quota=torch.tensor(quotas, **i32),
+                     offset=torch.tensor(np.cumsum(quotas) - quotas, **i32), ret=torch.zeros(n, **f64),
+                     len=torch.zeros(n, **i32), count=torch.zeros(n, **i32), step=torch.zeros(1, **i32),
+                     remaining=torch.zeros(1, **i32), act=torch.zeros((n, self.a), dtype=torch.float32, device=dev),
+                     val=torch.zeros(n, dtype=torch.float32, device=dev), ep_ret=torch.zeros(E, **f64),
+                     ep_len=torch.zeros(E, **i32), ep_tr=torch.zeros(E, dtype=torch.uint8, device=dev),
+                     ep_flags=torch.zeros(E, dtype=torch.uint8, device=dev), ep_step=torch.zeros(E, **i32))
+            self._eval_state = s
+        s["obs"] = env.reset_tensor()
+        for k in ("ret", "len", "count", "step"):
+            s[k].zero_()
+        active = int((quotas > 0).sum())
+        s["remaining"].fill_(active)
+        done = 0
+        while done < limit and active > 0:
+            if self.use_graph and s["graph"] is not None:
+                s["graph"].replay()
+            else:
+                self._eval_chunk(s, env, deterministic, limit)
+            done += K
+            if int(s["remaining"].item()) == 0:
+                break
+            if self.use_graph and s["graph"] is None:
+                # the chunk that just ran eagerly was the warm-up; capture does not execute the launches it records
+                torch.cuda.synchronize()
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    self._eval_chunk(s, env, deterministic, limit)
+                s["graph"] = g
+        count = s["count"].cpu().numpy().astype(np.int64)
+        slot = np.repeat(np.cumsum(quotas) - quotas, count) + (np.arange(int(count.sum())) - np.repeat(np.cumsum(count) - count, count))
+        take = lambda name: s[name].cpu().numpy()[slot]  # noqa: E731
+        return EvalResult.from_episodes(take("ep_ret"), take("ep_len"), take("ep_tr"), take("ep_flags"),
+                                        np.repeat(np.arange(n), count), take("ep_step"), env.cfg.task, env.cfg.num_targets,
+                                        device=self.device)
+
+    def _eval_chunk(self, s: dict, env, deterministic: bool, limit: int) -> None:
+        """EVAL_CHUNK agent steps of an evaluation: forward, env step, targets-reached copy, ledger; then the step index
+        advances by the chunk.  Every pointer is persistent, so the same launches serve as a replayed graph."""
+        n, lib = env.num_envs, self.lib
+        tidx = None
+        seed = (self.seed ^ 0x1B873593) & (2 ** 63 - 1)        # a key of its own: neither the training's nor predict's
+        for k in range(self.EVAL_CHUNK):
+            _lib.check(lib.ppo_policy_forward_a(_p(self.policy.theta), self.d, self.a, _p(s["obs"]), self._stats_ptr(),
+                                                self.vecnorm.clip_obs, n, seed, env.env_id0 & 0xFFFFFFFF, k, _p(s["step"]),
+                                                int(deterministic), None, _p(s["act"]), None, None, _p(s["val"]), _stream()))
+            _, rew, flags = env.step_tensor(s["act"])
+            if env.cfg.task in (1, 2):
+                tidx = env.targets_reached_tensor()
+            _lib.check(lib.ppo_eval_ledger(_p(rew), _p(flags), _p(tidx), n, _p(s["ret"]), _p(s["len"]), _p(s["count"]),
+                                           _p(s["quota"]), _p(s["offset"]), k, _p(s["step"]), limit, _p(s["remaining"]),
+                                           _p(s["ep_ret"]), _p(s["ep_len"]), _p(s["ep_tr"]), _p(s["ep_flags"]), _p(s["ep_step"]),
+                                           _stream()))
+        _lib.check(lib.ppo_counter_add(_p(s["step"]), self.EVAL_CHUNK, _stream()))
 
     def save(self, path: str) -> None:
         torch.save({"policy": self.policy.state_dict(), "optimizer": self.optimizer.state_dict(),
