@@ -505,8 +505,10 @@ ppo_grad_tc_kernel(const float* params, int d, const float* __restrict__ obs, co
         if (tid == 0) {
             double ta = 0.0, tb = 0.0;
             for (int k = 0; k < UT_THREADS / 32; ++k) { ta += sd[2 * k]; tb += sd[2 * k + 1]; }
-            const double n = (double)batch, mean = ta / n;
-            double var = batch > 1 ? (tb - n * mean * mean) / (n - 1.0) : 0.0;
+            // a one-sample minibatch is not normalised (stable_baselines3: normalize_advantage and len(advantages) > 1):
+            // mean 0, std 1 make (adv - mean) / (std + 1e-8f) exactly adv
+            const double n = (double)batch, mean = batch > 1 ? ta / n : 0.0;
+            double var = batch > 1 ? (tb - n * mean * mean) / (n - 1.0) : 1.0;
             if (var < 0.0) var = 0.0;
             small[UtSmem::FUSED] = (float)mean; small[UtSmem::FUSED + 1] = (float)sqrt(var);
         }
@@ -1111,8 +1113,9 @@ ppo_adv_stats_kernel(const float* __restrict__ adv, const long long* __restrict_
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) { ta += __shfl_xor_sync(0xffffffffu, ta, o); tb += __shfl_xor_sync(0xffffffffu, tb, o); }
     if (threadIdx.x != 0) return;
-    double n = (double)batch, mean = ta / n;
-    double var = batch > 1 ? (tb - n * mean * mean) / (n - 1.0) : 0.0;       // torch.std(): unbiased
+    // torch.std(): unbiased; a one-sample minibatch is not normalised (mean 0, std 1: see ppo_grad_tc_kernel)
+    double n = (double)batch, mean = batch > 1 ? ta / n : 0.0;
+    double var = batch > 1 ? (tb - n * mean * mean) / (n - 1.0) : 1.0;
     if (var < 0.0) var = 0.0;
     out[0] = (float)mean; out[1] = (float)sqrt(var);
     scratch[0] = 0.0;

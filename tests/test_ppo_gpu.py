@@ -378,7 +378,8 @@ def test_graph_replayed_update_equals_the_eager_update():
     env.close()
 
 
-@pytest.mark.parametrize("preset,batch", [("waypoints_v3", 128), ("waypoints_v3", 200), ("lowlevel", 128), ("objlock_duck", 128)])
+@pytest.mark.parametrize("preset,batch", [("waypoints_v3", 128), ("waypoints_v3", 200), ("lowlevel", 128), ("objlock_duck", 128),
+                                          ("waypoints_v3", 1)])
 def test_single_cta_optimizer_steps_equal_the_launch_per_kernel_update(preset, batch):
     """ppo_minibatch_steps_a (a window of optimizer steps in one single-CTA launch: advantage statistics, gradient, clip,
     Adam per step) against the same steps as separate launches (ppo_minibatch_grad_a + ppo_adam_step): same gradient kernel
@@ -421,7 +422,7 @@ def test_single_cta_optimizer_steps_equal_the_launch_per_kernel_update(preset, b
     env.close()
 
 
-@pytest.mark.parametrize("preset,batch", [("waypoints_v3", 1000), ("lowlevel", 512), ("objlock_duck", 700)])
+@pytest.mark.parametrize("preset,batch", [("waypoints_v3", 1000), ("lowlevel", 512), ("objlock_duck", 700), ("waypoints_v3", 1)])
 def test_window_update_is_bit_identical_to_separate_launches(preset, batch):
     """ppo_window_update_a (one advantage-statistics launch per window, clip + Adam by the last block of the gradient
     reduction) against ppo_minibatch_grad_a + ppo_adam_step per minibatch: same kernels' arithmetic, so parameters, Adam
@@ -542,6 +543,37 @@ def test_kernel_update_learns_like_the_torch_update():
     rel = float((dk - dt).norm() / dt.norm())
     assert cos > 0.99 and rel < 0.12, (cos, rel)
     assert float((dk - dt).abs().max()) < 0.25 * float(moved) + 2e-5
+
+
+@pytest.mark.parametrize("n_envs,n_steps,batch", [(4, 4, 1), (1, 129, 128)])
+def test_one_sample_minibatches_update_like_the_torch_update(n_envs, n_steps, batch):
+    """stable_baselines3 does not normalise the advantage of a one-sample minibatch.  batch_size 1 runs the single-CTA
+    optimizer steps (ppo_minibatch_steps_a); 129 samples in minibatches of 128 end with a ragged one-sample step
+    (ppo_minibatch_grad_a + ppo_adam_step).  From the same rollout, parameters and fresh Adam state, one epoch of the kernel
+    update must land where the torch update does, within the bounds of test_kernel_update_learns_like_the_torch_update."""
+    from pyflyt_drone_b200.ppo import PPO
+    from pyflyt_drone_b200.vec_env import FixedwingVecEnv
+    env = FixedwingVecEnv(n_envs, preset="waypoints_v3", seed=9)
+    m = PPO("MlpPolicy", env, n_steps=n_steps, batch_size=batch, n_epochs=1, seed=9, ent_coef=0.001, use_cuda_graph=False)
+    m.collect_rollouts()
+    theta0, epoch0 = m.policy.theta.detach().clone(), m._perm_epoch
+    out = {}
+    for mode in ("kernel", "torch"):          # both start from zero Adam moments and draw the same permutation
+        with torch.no_grad():
+            m.policy.theta.copy_(theta0)
+        m._perm_epoch = epoch0
+        m.update = mode
+        m.train()
+        torch.cuda.synchronize()
+        out[mode] = m.policy.theta.detach() - theta0
+    dk, dt = out["kernel"], out["torch"]
+    moved = dt.abs().max()
+    assert float(moved) > 1e-4
+    cos = float(torch.dot(dk, dt) / (dk.norm() * dt.norm()))
+    rel = float((dk - dt).norm() / dt.norm())
+    assert cos > 0.99 and rel < 0.12, (cos, rel)
+    assert float((dk - dt).abs().max()) < 0.25 * float(moved) + 2e-5
+    env.close()
 
 
 class FlatInit:
