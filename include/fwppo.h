@@ -208,6 +208,70 @@ int ppo_window_update_p2p_a(float* params, int32_t d, int32_t a, const float* ob
                             float* workspace, float* grad, float* stats, int32_t world, int32_t rank, void* const* peer_buffers,
                             uint32_t* sequence, void* stream);
 
+/* ---- Populations: `members` independent PPO models in one launch per kernel ----
+ * Member m owns rows [m * rows_per_member, (m + 1) * rows_per_member) of one env batch, its own parameter vector
+ * (params + m * ppo_param_count_a(d, a); the same stride for Adam moments and gradients), observation statistics
+ * (obs_stats + m * (2 d + 1)), return statistics (ret_stats + 3 m) and their scratch (moments: 2 d + 2 doubles, returns: 4 per
+ * member) and accumulators.  Each entry point computes, for every member, exactly what its standalone counterpart above computes
+ * over that member's rows with that member's values:
+ *   seeds [members]              the member's Philox key (forward) and permutation seed
+ *   hp [members * PPO_POP_HP]    the member's hyper-parameters at the PPO_POP_* indices (fp32)
+ *   env ids                      env_id0 + global row, i.e. the member's own ids start at env_id0 + m * rows_per_member
+ * Null pointers, members outside [1, PPO_POP_MAX_MEMBERS], rows_per_member < 1 or a batch of more than 2^31 - 1 rows return
+ * FW_EINVAL before anything is launched. */
+#define PPO_POP_MAX_MEMBERS 65535
+#define PPO_POP_HP 8
+#define PPO_POP_LR 0
+#define PPO_POP_CLIP_RANGE 1
+#define PPO_POP_ENT_COEF 2
+#define PPO_POP_VF_COEF 3
+#define PPO_POP_MAX_GRAD_NORM 4
+#define PPO_POP_GAMMA 5
+#define PPO_POP_GAE_LAMBDA 6
+/* ppo_policy_forward_a / ppo_policy_forward_tc_a for every member (the tensor-core form runs persistent CTAs per member over
+ * that member's 128-row tiles only) */
+int ppo_pop_policy_forward_a(int32_t members, int32_t rows_per_member, const uint64_t* seeds, const float* params, int32_t d,
+                             int32_t a, const float* obs_raw, const double* obs_stats, float clip_obs, uint32_t env_id0,
+                             uint32_t step, const uint32_t* step_dev, int32_t deterministic, float* obs_norm, float* act_env,
+                             float* act_raw, float* logp, float* value, void* stream);
+int ppo_pop_policy_forward_tc_a(int32_t members, int32_t rows_per_member, const uint64_t* seeds, const float* params, int32_t d,
+                                int32_t a, const float* obs_raw, const double* obs_stats, float clip_obs, uint32_t env_id0,
+                                uint32_t step, const uint32_t* step_dev, int32_t deterministic, float* obs_norm, float* act_env,
+                                float* act_raw, float* logp, float* value, void* stream);
+int ppo_pop_value_forward_a(int32_t members, int32_t rows_per_member, const float* params, int32_t d, int32_t a,
+                            const float* obs_raw, const double* obs_stats, float clip_obs, float* value, void* stream);
+/* gamma of each member from hp */
+int ppo_pop_timeout_bootstrap_a(int32_t members, int32_t rows_per_member, const float* hp, const float* params, int32_t d, int32_t a,
+                                const float* term_obs_raw, const double* obs_stats, float clip_obs, const uint8_t* flags,
+                                float* rew_inout, void* stream);
+int ppo_pop_moments_update(int32_t members, int32_t rows_per_member, const float* x, int32_t d, double* stats, double* scratch,
+                           double* accum, void* stream);
+int ppo_pop_reward_normalize(int32_t members, int32_t rows_per_member, const float* hp, const float* rew, const uint8_t* flags,
+                             float clip_rew, float* ret, double* ret_stats, double* scratch, double* accum, float* rew_norm,
+                             float* done_out, void* stream);
+/* GAE over [T, members * rows_per_member] with gamma and lambda of column / rows_per_member */
+int ppo_pop_gae(int32_t members, int32_t rows_per_member, const float* hp, const float* rewards, const float* values,
+                const float* dones, const float* last_values, int32_t T, float* advantages, float* returns, void* stream);
+/* out [members][n]: member m's ppo_random_permutation(n, seeds[m], epoch), each sample k written as the row
+ * (k / rows_per_member) * members * rows_per_member + m * rows_per_member + k % rows_per_member of the time-major population
+ * buffers (n = the member's sample count, T * rows_per_member) */
+int ppo_pop_random_permutation(int32_t members, int32_t rows_per_member, const uint64_t* seeds, int64_t* out, int64_t n,
+                               uint64_t epoch, void* stream);
+/* ppo_minibatch_steps_a for every member in one launch of `members` thread blocks: member m's index window is
+ * idx[m * idx_stride ..], its learning rate, clip range, entropy / value coefficients and max grad norm come from hp;
+ * step_counter and grad_norm_out hold one entry per member, stats 8 floats per member */
+int ppo_pop_minibatch_steps_a(int32_t members, const float* hp, float* params, int32_t d, int32_t a, const float* obs_norm,
+                              const float* act, const float* logp_old, const float* adv, const float* ret, const int64_t* idx,
+                              int64_t idx_stride, int32_t batch, int32_t steps, float* exp_avg, float* exp_avg_sq, float beta1,
+                              float beta2, float eps, int32_t* step_counter, float* grad_norm_out, float* grad, float* stats,
+                              void* stream);
+/* Training episode ledger, one thread per env, one launch per rollout step on the step's raw rewards and flags: ret [n] (double,
+ * summed in step order) and len [n] run per env; a finished episode (flags & 3) adds to acc [8][n] (env i's column) its count,
+ * return, length, targets reached (targets_reached may be NULL), collision, out-of-bounds, completed and strike flags -- the eight
+ * quantities of fw_episode_stats -- and restarts ret and len.  n = members * rows_per_member.  No atomics. */
+int ppo_pop_episode_ledger(int32_t members, int32_t rows_per_member, const float* rew, const uint8_t* flags,
+                           const uint8_t* targets_reached, double* ret, int32_t* len, double* acc, void* stream);
+
 /* torch.nn.utils.clip_grad_norm_(max_grad_norm) followed by torch.optim.Adam.step (no weight decay / amsgrad) on the
  * flat parameter vector; grad is pre-multiplied by grad_scale (1 / world_size after the NCCL sum).
  * step_counter: device int32 incremented by the call (bias correction). */

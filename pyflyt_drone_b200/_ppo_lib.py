@@ -46,6 +46,20 @@ PPO_SYMBOLS = [
     ("ppo_minibatch_grad", C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int32, _F, _F, _F, _P, _P, _P, _P]),
     ("ppo_adam_step", C.c_int, [_P, _P, _P, _P, C.c_int32, _F, _F, _F, _F, _F, _F, _P, _P, _P]),
     ("ppo_gae", C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _F, _F, _P, _P, _P]),
+    # populations (members, rows_per_member, ...)
+    ("ppo_pop_policy_forward_a", C.c_int, [C.c_int32, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _F, C.c_uint32, C.c_uint32,
+                                           _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    ("ppo_pop_policy_forward_tc_a", C.c_int, [C.c_int32, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _F, C.c_uint32, C.c_uint32,
+                                              _P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    ("ppo_pop_value_forward_a", C.c_int, [C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P, _F, _P, _P]),
+    ("ppo_pop_timeout_bootstrap_a", C.c_int, [C.c_int32, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _F, _P, _P, _P]),
+    ("ppo_pop_moments_update", C.c_int, [C.c_int32, C.c_int32, _P, C.c_int32, _P, _P, _P, _P]),
+    ("ppo_pop_reward_normalize", C.c_int, [C.c_int32, C.c_int32, _P, _P, _P, _F, _P, _P, _P, _P, _P, _P, _P]),
+    ("ppo_pop_gae", C.c_int, [C.c_int32, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, _P, _P, _P]),
+    ("ppo_pop_random_permutation", C.c_int, [C.c_int32, C.c_int32, _P, _P, C.c_int64, C.c_uint64, _P]),
+    ("ppo_pop_minibatch_steps_a", C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int32,
+                                            C.c_int32, _P, _P, _F, _F, _F, _P, _P, _P, _P, _P]),
+    ("ppo_pop_episode_ledger", C.c_int, [C.c_int32, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
 ]
 
 

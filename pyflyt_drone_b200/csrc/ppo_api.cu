@@ -461,3 +461,175 @@ extern "C" int ppo_adam_step(float* params, const float* grad, float* exp_avg, f
                   grad_norm_out, (cudaStream_t)stream));
     return FW_OK;
 }
+
+// ---- populations (include/fwppo.h "Populations"): argument checks, then one launch per kernel for every member
+static int check_pop(int32_t members, int32_t rows) {
+    if (members < 1 || members > PPO_POP_MAX_MEMBERS)
+        return pfail(FW_EINVAL, "members %d out of range [1,%d]", members, PPO_POP_MAX_MEMBERS);
+    if (rows < 1) return pfail(FW_EINVAL, "rows_per_member must be positive");
+    if ((long long)members * rows > 2147483647ll) return pfail(FW_EINVAL, "members * rows_per_member exceeds 2^31 - 1 rows");
+    return FW_OK;
+}
+static PpokPop make_pop(int32_t members, int32_t rows, const uint64_t* seeds, const float* hp, int32_t d, int32_t a) {
+    PpokPop p;
+    p.seeds = seeds; p.hp = hp; p.members = members; p.rows = rows;
+    p.param_stride = (d > 0 && (a == 4 || a == 6)) ? ppo_param_count_a(d, a) : 0;
+    return p;
+}
+
+static int pop_forward_impl(bool tc, int32_t members, int32_t rows, const uint64_t* seeds, const float* params, int32_t d, int32_t a,
+                            const float* obs_raw, const double* obs_stats, float clip_obs, uint32_t env_id0, uint32_t step,
+                            const uint32_t* step_dev, int32_t deterministic, float* obs_norm, float* act_env, float* act_raw,
+                            float* logp, float* value, void* stream) {
+    int rc = check_pop(members, rows);
+    if (rc) return rc;
+    if (!seeds || !params || !obs_raw || !act_env || !value) return pfail(FW_EINVAL, "null argument");
+    if ((rc = tc && a != 4 ? check_d_tc(d) : check_d(d)) != 0) return rc;
+    if ((rc = check_a(a)) != 0) return rc;
+    if ((reinterpret_cast<uintptr_t>(act_env) & 15u) || (act_raw && (reinterpret_cast<uintptr_t>(act_raw) & 15u)))
+        return pfail(FW_EINVAL, "action buffers must be 16-byte aligned");
+    const PpokPop pop = make_pop(members, rows, seeds, nullptr, d, a);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!tc)
+        PCU(ppok_pop_forward(pop, params, d, obs_raw, obs_stats, clip_obs, rows, env_id0, step, step_dev, deterministic, obs_norm,
+                             act_env, act_raw, logp, value, 1, st, nullptr, nullptr, a));
+    else if (a == 4 && d > PPO_TC_MAX_OBS)
+        PCU(ppo_a4d64::ppok_pop_forward_tc(pop, params, d, obs_raw, obs_stats, clip_obs, rows, env_id0, step, step_dev, deterministic,
+                                           obs_norm, act_env, act_raw, logp, value, st));
+    else if (a == 4)
+        PCU(ppo_a4::ppok_pop_forward_tc(pop, params, d, obs_raw, obs_stats, clip_obs, rows, env_id0, step, step_dev, deterministic,
+                                        obs_norm, act_env, act_raw, logp, value, st));
+    else
+        PCU(ppo_a6::ppok_pop_forward_tc(pop, params, d, obs_raw, obs_stats, clip_obs, rows, env_id0, step, step_dev, deterministic,
+                                        obs_norm, act_env, act_raw, logp, value, st));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_policy_forward_a(int32_t members, int32_t rows_per_member, const uint64_t* seeds, const float* params, int32_t d,
+                                        int32_t a, const float* obs_raw, const double* obs_stats, float clip_obs, uint32_t env_id0,
+                                        uint32_t step, const uint32_t* step_dev, int32_t deterministic, float* obs_norm, float* act_env,
+                                        float* act_raw, float* logp, float* value, void* stream) {
+    return pop_forward_impl(false, members, rows_per_member, seeds, params, d, a, obs_raw, obs_stats, clip_obs, env_id0, step, step_dev,
+                            deterministic, obs_norm, act_env, act_raw, logp, value, stream);
+}
+
+extern "C" int ppo_pop_policy_forward_tc_a(int32_t members, int32_t rows_per_member, const uint64_t* seeds, const float* params,
+                                           int32_t d, int32_t a, const float* obs_raw, const double* obs_stats, float clip_obs,
+                                           uint32_t env_id0, uint32_t step, const uint32_t* step_dev, int32_t deterministic,
+                                           float* obs_norm, float* act_env, float* act_raw, float* logp, float* value, void* stream) {
+    return pop_forward_impl(true, members, rows_per_member, seeds, params, d, a, obs_raw, obs_stats, clip_obs, env_id0, step, step_dev,
+                            deterministic, obs_norm, act_env, act_raw, logp, value, stream);
+}
+
+extern "C" int ppo_pop_value_forward_a(int32_t members, int32_t rows_per_member, const float* params, int32_t d, int32_t a,
+                                       const float* obs_raw, const double* obs_stats, float clip_obs, float* value, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!params || !obs_raw || !value) return pfail(FW_EINVAL, "null argument");
+    if ((rc = check_d(d)) != 0) return rc;
+    if ((rc = check_a(a)) != 0) return rc;
+    PCU(ppok_pop_forward(make_pop(members, rows_per_member, nullptr, nullptr, d, a), params, d, obs_raw, obs_stats, clip_obs,
+                         rows_per_member, 0, 0, nullptr, 1, nullptr, nullptr, nullptr, nullptr, value, 0, (cudaStream_t)stream, nullptr,
+                         nullptr, a));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_timeout_bootstrap_a(int32_t members, int32_t rows_per_member, const float* hp, const float* params, int32_t d,
+                                           int32_t a, const float* term_obs_raw, const double* obs_stats, float clip_obs,
+                                           const uint8_t* flags, float* rew_inout, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!hp || !params || !term_obs_raw || !flags || !rew_inout) return pfail(FW_EINVAL, "null argument");
+    if ((rc = check_d(d)) != 0) return rc;
+    if ((rc = check_a(a)) != 0) return rc;
+    PCU(ppok_pop_forward(make_pop(members, rows_per_member, nullptr, hp, d, a), params, d, term_obs_raw, obs_stats, clip_obs,
+                         rows_per_member, 0, 0, nullptr, 1, nullptr, nullptr, nullptr, nullptr, nullptr, 0, (cudaStream_t)stream, flags,
+                         rew_inout, a));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_moments_update(int32_t members, int32_t rows_per_member, const float* x, int32_t d, double* stats,
+                                      double* scratch, double* accum, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!x || !stats || !scratch) return pfail(FW_EINVAL, "null argument");
+    if ((rc = check_d(d)) != 0) return rc;
+    PCU(ppok_pop_moments(make_pop(members, rows_per_member, nullptr, nullptr, 0, 0), x, rows_per_member, d, stats, scratch, accum,
+                         (cudaStream_t)stream));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_reward_normalize(int32_t members, int32_t rows_per_member, const float* hp, const float* rew,
+                                        const uint8_t* flags, float clip_rew, float* ret, double* ret_stats, double* scratch,
+                                        double* accum, float* rew_norm, float* done_out, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!hp || !rew || !flags || !ret || !ret_stats || !scratch || !rew_norm) return pfail(FW_EINVAL, "null argument");
+    PCU(ppok_pop_reward_normalize(make_pop(members, rows_per_member, nullptr, hp, 0, 0), rew, flags, rows_per_member, clip_rew, ret,
+                                  ret_stats, scratch, accum, rew_norm, done_out, (cudaStream_t)stream));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_gae(int32_t members, int32_t rows_per_member, const float* hp, const float* rewards, const float* values,
+                           const float* dones, const float* last_values, int32_t T, float* advantages, float* returns, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!hp || !rewards || !values || !dones || !last_values || !advantages || !returns) return pfail(FW_EINVAL, "null argument");
+    if (T <= 0) return pfail(FW_EINVAL, "T must be positive");
+    PCU(ppok_pop_gae(make_pop(members, rows_per_member, nullptr, hp, 0, 0), rewards, values, dones, last_values, T, rows_per_member,
+                     advantages, returns, (cudaStream_t)stream));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_random_permutation(int32_t members, int32_t rows_per_member, const uint64_t* seeds, int64_t* out, int64_t n,
+                                          uint64_t epoch, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!seeds || !out) return pfail(FW_EINVAL, "null argument");
+    if (n < 0 || n % rows_per_member != 0) return pfail(FW_EINVAL, "n must be a non-negative multiple of rows_per_member");
+    if (n * (long long)members >= (1ll << 62)) return pfail(FW_EINVAL, "ppo_pop_random_permutation: n too large");
+    PpokPop pop = make_pop(members, rows_per_member, seeds, nullptr, 0, 0);
+    pop.epoch = epoch;
+    PCU(ppok_pop_permutation(pop, reinterpret_cast<long long*>(out), (long long)n, (cudaStream_t)stream));
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_minibatch_steps_a(int32_t members, const float* hp, float* params, int32_t d, int32_t a, const float* obs_norm,
+                                         const float* act, const float* logp_old, const float* adv, const float* ret, const int64_t* idx,
+                                         int64_t idx_stride, int32_t batch, int32_t steps, float* exp_avg, float* exp_avg_sq, float beta1,
+                                         float beta2, float eps, int32_t* step_counter, float* grad_norm_out, float* grad, float* stats,
+                                         void* stream) {
+    int rc = check_pop(members, 1);
+    if (rc) return rc;
+    if (!hp || !params || !obs_norm || !act || !logp_old || !adv || !ret || !idx || !exp_avg || !exp_avg_sq || !step_counter || !grad ||
+        !stats)
+        return pfail(FW_EINVAL, "null argument");
+    if (batch <= 0 || batch > PPO_FUSED_MAX_BATCH)
+        return pfail(FW_EINVAL, "batch %d out of range [1,%d] for the single-CTA optimizer steps", batch, PPO_FUSED_MAX_BATCH);
+    if (steps <= 0) return pfail(FW_EINVAL, "steps must be positive");
+    if (idx_stride < 0) return pfail(FW_EINVAL, "idx_stride must not be negative");
+    if ((rc = (a == 4) ? check_d(d) : check_d_tc(d)) != 0) return rc;
+    if ((rc = check_a(a)) != 0) return rc;
+    if (reinterpret_cast<uintptr_t>(act) & 15u) return pfail(FW_EINVAL, "action buffer must be 16-byte aligned");
+    if (ppo_param_count_a(d, a) > 16384) return pfail(FW_EINVAL, "parameter vector too long");
+    PpokPop pop = make_pop(members, 1, nullptr, hp, d, a);
+    pop.idx_stride = idx_stride;
+    const long long* ix = reinterpret_cast<const long long*>(idx);
+    cudaStream_t st = (cudaStream_t)stream;
+#define POP_STEPS_ARGS pop, params, d, obs_norm, act, logp_old, adv, ret, ix, batch, steps, exp_avg, exp_avg_sq, beta1, beta2, eps, \
+                       step_counter, grad_norm_out, grad, stats, st
+    if (a == 4 && d > PPO_TC_MAX_OBS) PCU(ppo_a4d64::ppok_pop_minibatch_steps(POP_STEPS_ARGS));
+    else if (a == 4) PCU(ppo_a4::ppok_pop_minibatch_steps(POP_STEPS_ARGS));
+    else PCU(ppo_a6::ppok_pop_minibatch_steps(POP_STEPS_ARGS));
+#undef POP_STEPS_ARGS
+    return FW_OK;
+}
+
+extern "C" int ppo_pop_episode_ledger(int32_t members, int32_t rows_per_member, const float* rew, const uint8_t* flags,
+                                      const uint8_t* targets_reached, double* ret, int32_t* len, double* acc, void* stream) {
+    int rc = check_pop(members, rows_per_member);
+    if (rc) return rc;
+    if (!rew || !flags || !ret || !len || !acc) return pfail(FW_EINVAL, "null argument");
+    PCU(ppok_pop_episode_ledger(rew, flags, targets_reached, members * rows_per_member, ret, len, acc, (cudaStream_t)stream));
+    return FW_OK;
+}

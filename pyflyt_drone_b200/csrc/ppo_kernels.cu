@@ -129,7 +129,9 @@ __device__ __forceinline__ void stage_stats(const double* __restrict__ stats, in
 
 // ------------------------------------------------------------------ K4: policy + value forward, one thread per env
 // AO = action width: 4 (roll, pitch, yaw, thrust) or 6 (the low-level env's surface / thrust channels)
-template <int AO, int DP>
+// POP: population launch, blockIdx.y = member (see PpokPop): every per-member pointer, the seed and the bootstrap's gamma
+// move to the member before the body runs over its `n` rows
+template <int AO, int DP, bool POP = false>
 __global__ void __launch_bounds__(PPO_FWD_THREADS)
 ppo_forward_kernel(const float* __restrict__ params, int d, const float* __restrict__ obs_raw,
                    const double* __restrict__ stats, float clip, int n, uint32_t seed_lo, uint32_t seed_hi,
@@ -137,8 +139,24 @@ ppo_forward_kernel(const float* __restrict__ params, int d, const float* __restr
                    float* __restrict__ obs_norm,
                    float* __restrict__ act_env, float* __restrict__ act_raw, float* __restrict__ logp,
                    float* __restrict__ value, int want_policy, const uint8_t* __restrict__ boot_flags, float boot_gamma,
-                   float* __restrict__ boot_rew) {
+                   float* __restrict__ boot_rew, PpokPop pop) {
     extern __shared__ __align__(16) float smem[];
+    if constexpr (POP) {
+        const int m = blockIdx.y;
+        const size_t r0 = (size_t)m * n;
+        params += (size_t)m * pop.param_stride;
+        obs_raw += r0 * d;
+        if (stats != nullptr) stats += (size_t)m * (2 * d + 1);
+        const uint64_t seed = pop.seeds != nullptr ? pop.seeds[m] : 0ull;      // value and bootstrap launches draw no noise
+        seed_lo = (uint32_t)(seed & 0xffffffffu); seed_hi = (uint32_t)(seed >> 32);
+        env_id0 += (uint32_t)r0;
+        if (obs_norm != nullptr) obs_norm += r0 * d;
+        if (act_env != nullptr) act_env += r0 * AO;
+        if (act_raw != nullptr) act_raw += r0 * AO;
+        if (logp != nullptr) logp += r0;
+        if (value != nullptr) value += r0;
+        if (boot_flags != nullptr) { boot_flags += r0; boot_rew += r0; boot_gamma = pop.hp[m * PPO_POP_HP + PPO_POP_GAMMA]; }
+    }
     // time-limit bootstrap mode: only blocks holding a truncated-but-not-terminated row do any work (truncations
     // arrive in bursts -- every env of a synchronised batch hits the step limit together -- and are absent otherwise)
     bool boot_need = false;
@@ -214,23 +232,24 @@ static size_t ppo_forward_smem_t() {
 }
 size_t ppo_forward_smem() { return ppo_forward_smem_t<A, 32>(); }
 
-template <int AO, int DP>
+template <int AO, int DP, bool POP = false>
 static cudaError_t ppok_forward_t(const float* params, int d, const float* obs_raw, const double* stats, float clip, int n,
                                   uint64_t seed, uint32_t env_id0, uint32_t step, const uint32_t* step_dev, int deterministic,
                                   float* obs_norm, float* act_env, float* act_raw, float* logp, float* value, int want_policy,
-                                  cudaStream_t st, const uint8_t* boot_flags, float boot_gamma, float* boot_rew) {
+                                  cudaStream_t st, const uint8_t* boot_flags, float boot_gamma, float* boot_rew,
+                                  const PpokPop& pop = PpokPop{}) {
     static bool attr_set = false;
     const size_t sm = ppo_forward_smem_t<AO, DP>();
     if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(ppo_forward_kernel<AO, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaError_t e = cudaFuncSetAttribute(ppo_forward_kernel<AO, DP, POP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         if (e != cudaSuccess) return e;
         attr_set = true;
     }
-    const int grid = (n + PPO_FWD_THREADS - 1) / PPO_FWD_THREADS;
-    ppo_forward_kernel<AO, DP><<<grid, PPO_FWD_THREADS, sm, st>>>(params, d, obs_raw, stats, clip, n, (uint32_t)(seed & 0xffffffffu),
-                                                              (uint32_t)(seed >> 32), env_id0, step, step_dev, deterministic,
-                                                              obs_norm, act_env, act_raw, logp, value, want_policy, boot_flags,
-                                                              boot_gamma, boot_rew);
+    const dim3 grid((n + PPO_FWD_THREADS - 1) / PPO_FWD_THREADS, POP ? pop.members : 1);
+    ppo_forward_kernel<AO, DP, POP><<<grid, PPO_FWD_THREADS, sm, st>>>(params, d, obs_raw, stats, clip, n, (uint32_t)(seed & 0xffffffffu),
+                                                                   (uint32_t)(seed >> 32), env_id0, step, step_dev, deterministic,
+                                                                   obs_norm, act_env, act_raw, logp, value, want_policy, boot_flags,
+                                                                   boot_gamma, boot_rew, pop);
     return cudaGetLastError();
 }
 
@@ -249,14 +268,38 @@ cudaError_t ppok_forward(const float* params, int d, const float* obs_raw, const
     return cudaErrorInvalidValue;
 }
 
+cudaError_t ppok_pop_forward(const PpokPop& pop, const float* params, int d, const float* obs_raw, const double* stats, float clip,
+                             int n, uint32_t env_id0, uint32_t step, const uint32_t* step_dev, int deterministic, float* obs_norm,
+                             float* act_env, float* act_raw, float* logp, float* value, int want_policy, cudaStream_t st,
+                             const uint8_t* boot_flags, float* boot_rew, int a) {
+    if (d > 64) return cudaErrorInvalidValue;
+#define FWD_DISPATCH(AO_, DP_)                                                                                               \
+    return ppok_forward_t<AO_, DP_, true>(params, d, obs_raw, stats, clip, n, 0, env_id0, step, step_dev, deterministic, obs_norm, \
+                                          act_env, act_raw, logp, value, want_policy, st, boot_flags, 0.0f, boot_rew, pop)
+    if (a == 4 && d <= 32) FWD_DISPATCH(4, 32);
+    if (a == 6 && d <= 32) FWD_DISPATCH(6, 32);
+    if (a == 4) FWD_DISPATCH(4, 64);
+#undef FWD_DISPATCH
+    return cudaErrorInvalidValue;
+}
+
 // ------------------------------------------------------------------ K7: running moments (RunningMeanStd.update)
 // scratch = double[2*d + 2]: column sums, column sums of squares, block-arrival counter (as double), spare.
 #define MOM_ROWS 128          // rows per block: 512 blocks at 65,536 envs, every load of a thread in flight at once
+// POP: blockIdx.y = member, n = rows per member; the member's rows, statistics, scratch and accumulator
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 ppo_moments_kernel(const float* __restrict__ x, int n, int d, double* __restrict__ stats, double* __restrict__ scratch,
                    double* __restrict__ accum, int rows_per_block) {
     __shared__ float s_sum[8][32], s_sq[8][32];
     __shared__ bool is_last;
+    if constexpr (POP) {
+        const int m = blockIdx.y;
+        x += (size_t)m * n * d;
+        stats += (size_t)m * (2 * d + 1);
+        scratch += (size_t)m * (2 * d + 2);
+        if (accum != nullptr) accum += (size_t)m * (2 * d + 1);
+    }
     // thread layout: 32 columns x 8 row-lanes; a warp reads 32 consecutive floats of one row when d == 32, and
     // d/32 of a 128-byte line otherwise (rows are contiguous, so the block still streams whole lines)
     const int lane_row = threadIdx.x >> 5;
@@ -371,13 +414,29 @@ cudaError_t ppok_moments(const float* x, int n, int d, double* stats, double* sc
     return cudaGetLastError();
 }
 
+cudaError_t ppok_pop_moments(const PpokPop& pop, const float* x, int n, int d, double* stats, double* scratch, double* accum,
+                             cudaStream_t st) {
+    const dim3 grid((n + MOM_ROWS - 1) / MOM_ROWS, pop.members);
+    ppo_moments_kernel<true><<<grid, 256, 0, st>>>(x, n, d, stats, scratch, accum, MOM_ROWS);
+    return cudaGetLastError();
+}
+
 // ------------------------------------------------------------------ VecNormalize reward path (two launches: the
 // normalisation needs the variance that includes this very batch of returns)
+// POP (both kernels): blockIdx.y = member, n = rows per member; the member's rows, return statistics, scratch (4 doubles per
+// member) and accumulator, and its gamma
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 ppo_ret_kernel(const float* __restrict__ rew, int n, float gamma, float* __restrict__ ret, double* __restrict__ ret_stats,
-               double* __restrict__ scratch, double* __restrict__ accum) {
+               double* __restrict__ scratch, double* __restrict__ accum, const float* __restrict__ pop_hp = nullptr) {
     __shared__ double s_a[8], s_b[8];
     __shared__ bool is_last;
+    if constexpr (POP) {
+        const int m = blockIdx.y;
+        rew += (size_t)m * n; ret += (size_t)m * n; ret_stats += 3 * m; scratch += 4 * m;
+        if (accum != nullptr) accum += 3 * m;
+        gamma = pop_hp[m * PPO_POP_HP + PPO_POP_GAMMA];
+    }
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     float v = 0.0f;
     if (i < n) { v = fmaf(ret[i], gamma, rew[i]); ret[i] = v; }
@@ -410,10 +469,16 @@ ppo_ret_kernel(const float* __restrict__ rew, int n, float gamma, float* __restr
     scratch[0] = 0.0; scratch[1] = 0.0; scratch[2] = 0.0;
 }
 
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 ppo_rew_finalize_kernel(const float* __restrict__ rew, const uint8_t* __restrict__ flags, int n, float clip,
                         float* __restrict__ ret, const double* __restrict__ ret_stats, float* __restrict__ rew_norm,
                         float* __restrict__ done_out) {
+    if constexpr (POP) {
+        const size_t r0 = (size_t)blockIdx.y * n;
+        rew += r0; flags += r0; ret += r0; ret_stats += 3 * blockIdx.y; rew_norm += r0;
+        if (done_out != nullptr) done_out += r0;
+    }
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float istd = (float)(1.0 / sqrt(ret_stats[1] + 1e-8));
@@ -431,6 +496,17 @@ cudaError_t ppok_reward_normalize(const float* rew, const uint8_t* flags, int n,
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     ppo_rew_finalize_kernel<<<grid, 256, 0, st>>>(rew, flags, n, clip, ret, ret_stats, rew_norm, done_out);
+    return cudaGetLastError();
+}
+
+cudaError_t ppok_pop_reward_normalize(const PpokPop& pop, const float* rew, const uint8_t* flags, int n, float clip, float* ret,
+                                      double* ret_stats, double* scratch, double* accum, float* rew_norm, float* done_out,
+                                      cudaStream_t st) {
+    const dim3 grid((n + 255) / 256, pop.members);
+    ppo_ret_kernel<true><<<grid, 256, 0, st>>>(rew, n, 0.0f, ret, ret_stats, scratch, accum, pop.hp);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    ppo_rew_finalize_kernel<true><<<grid, 256, 0, st>>>(rew, flags, n, clip, ret, ret_stats, rew_norm, done_out);
     return cudaGetLastError();
 }
 
@@ -453,10 +529,22 @@ __device__ __forceinline__ uint32_t ppo_mix32(uint32_t x, uint32_t k) {
     x ^= k; x *= 0x9E3779B1u; x ^= x >> 15; x *= 0x85EBCA77u; x ^= x >> 13; x *= 0xC2B2AE3Du; x ^= x >> 16;
     return x;
 }
+__host__ __device__ __forceinline__ void ppo_perm_keys(uint64_t seed, uint64_t epoch, uint32_t& k0, uint32_t& k1) {
+    k0 = (uint32_t)(seed ^ (epoch * 0x9E3779B97F4A7C15ull));
+    k1 = (uint32_t)((seed >> 32) ^ ((epoch * 0xC2B2AE3D27D4EB4Full) >> 32) ^ 0xA5A5A5A5u);
+}
+
+// POP: blockIdx.y = member; its permutation of [0, n) (n = its sample count) with its own seed, written to out[m * n ..] as
+// population rows (k / rows) * members * rows + m * rows + k % rows of the time-major [T, members * rows] rollout buffers
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
-ppo_permutation_kernel(long long* __restrict__ out, long long n, int hb, uint32_t k0, uint32_t k1) {
+ppo_permutation_kernel(long long* __restrict__ out, long long n, int hb, uint32_t k0, uint32_t k1, PpokPop pop) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if constexpr (POP) {
+        out += (size_t)blockIdx.y * n;
+        ppo_perm_keys(pop.seeds[blockIdx.y], pop.epoch, k0, k1);
+    }
     const uint32_t mask = (1u << hb) - 1u;
     unsigned long long x = (unsigned long long)i;
     do {                                     // cycle walking: re-encrypt until the value falls inside [0, n)
@@ -468,12 +556,11 @@ ppo_permutation_kernel(long long* __restrict__ out, long long n, int hb, uint32_
         }
         x = ((unsigned long long)L << hb) | R;
     } while (x >= (unsigned long long)n);
+    if constexpr (POP) {
+        const long long rows = pop.rows, k = (long long)x;
+        x = (unsigned long long)((k / rows) * pop.members * rows + (long long)blockIdx.y * rows + k % rows);
+    }
     out[i] = (long long)x;
-}
-
-__host__ __device__ __forceinline__ void ppo_perm_keys(uint64_t seed, uint64_t epoch, uint32_t& k0, uint32_t& k1) {
-    k0 = (uint32_t)(seed ^ (epoch * 0x9E3779B97F4A7C15ull));
-    k1 = (uint32_t)((seed >> 32) ^ ((epoch * 0xC2B2AE3D27D4EB4Full) >> 32) ^ 0xA5A5A5A5u);
 }
 
 __device__ __forceinline__ long long ppo_perm_at(long long i, long long n, int hb, uint32_t k0, uint32_t k1) {
@@ -519,7 +606,14 @@ cudaError_t ppok_permutation(long long* out, long long n, uint64_t seed, uint64_
     if (n <= 0) return cudaSuccess;
     uint32_t k0, k1;
     ppo_perm_keys(seed, epoch, k0, k1);
-    ppo_permutation_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(out, n, perm_half_bits(n), k0, k1);
+    ppo_permutation_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(out, n, perm_half_bits(n), k0, k1, PpokPop{});
+    return cudaGetLastError();
+}
+
+cudaError_t ppok_pop_permutation(const PpokPop& pop, long long* out, long long n, cudaStream_t st) {
+    if (n <= 0) return cudaSuccess;
+    const dim3 grid((unsigned)((n + 255) / 256), pop.members);
+    ppo_permutation_kernel<true><<<grid, 256, 0, st>>>(out, n, perm_half_bits(n), 0u, 0u, pop);
     return cudaGetLastError();
 }
 
@@ -533,12 +627,18 @@ cudaError_t ppok_permutation_window(long long* out, long long n, uint64_t seed, 
 }
 
 // ------------------------------------------------------------------ K5: GAE, one thread per env, coalesced over envs
+// POP: gamma and lambda of member i / pop.rows (n = every column of the population)
+template <bool POP = false>
 __global__ void __launch_bounds__(256)
 ppo_gae_kernel(const float* __restrict__ rewards, const float* __restrict__ values, const float* __restrict__ dones,
                const float* __restrict__ last_values, int T, int n, float gamma, float lam,
-               float* __restrict__ adv, float* __restrict__ ret) {
+               float* __restrict__ adv, float* __restrict__ ret, const float* __restrict__ pop_hp = nullptr, int pop_rows = 0) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if constexpr (POP) {
+        const float* h = pop_hp + (size_t)(i / pop_rows) * PPO_POP_HP;
+        gamma = h[PPO_POP_GAMMA]; lam = h[PPO_POP_GAE_LAMBDA];
+    }
     float next_value = last_values[i], gae = 0.0f;
     for (int t = T - 1; t >= 0; --t) {
         const size_t o = (size_t)t * n + i;
@@ -555,6 +655,14 @@ ppo_gae_kernel(const float* __restrict__ rewards, const float* __restrict__ valu
 cudaError_t ppok_gae(const float* rewards, const float* values, const float* dones, const float* last_values, int T, int n,
                      float gamma, float lam, float* adv, float* ret, cudaStream_t st) {
     ppo_gae_kernel<<<(n + 255) / 256, 256, 0, st>>>(rewards, values, dones, last_values, T, n, gamma, lam, adv, ret);
+    return cudaGetLastError();
+}
+
+cudaError_t ppok_pop_gae(const PpokPop& pop, const float* rewards, const float* values, const float* dones, const float* last_values,
+                         int T, int n, float* adv, float* ret, cudaStream_t st) {
+    const int cols = n * pop.members;
+    ppo_gae_kernel<true><<<(cols + 255) / 256, 256, 0, st>>>(rewards, values, dones, last_values, T, cols, 0.0f, 0.0f, adv, ret,
+                                                            pop.hp, n);
     return cudaGetLastError();
 }
 
@@ -608,5 +716,41 @@ cudaError_t ppok_eval_ledger(const float* rew, const uint8_t* flags, const uint8
                              cudaStream_t st) {
     ppo_eval_ledger_kernel<<<(n + 255) / 256, 256, 0, st>>>(rew, flags, tidx, n, ret, len, count, quota, offset, step, step_dev,
                                                             step_limit, remaining, ep_ret, ep_len, ep_tr, ep_flags, ep_step);
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ training episode ledger (population episode statistics)
+// One thread per env, one launch per rollout step, on the raw rewards and flags of the step.  Each env keeps its running return
+// (double, summed in step order) and length, and adds every finished episode to its own sums acc[k * n + i] for the eight
+// quantities of fw_episode_stats: episodes, return, length, targets reached, collisions, out-of-bounds, completed, strikes.  No
+// atomics: a member's statistics are reduced afterwards over its envs in env order.
+__global__ void __launch_bounds__(256)
+ppo_pop_episode_ledger_kernel(const float* __restrict__ rew, const uint8_t* __restrict__ flags, const uint8_t* __restrict__ tidx,
+                              int n, double* __restrict__ ret, int* __restrict__ len, double* __restrict__ acc) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    double r = ret[i] + (double)rew[i];
+    int l = len[i] + 1;
+    const uint8_t f = flags[i];
+    if (f & 3u) {
+        const size_t s = (size_t)n;
+        acc[i] += 1.0;
+        acc[s + i] += r;
+        acc[2 * s + i] += (double)l;
+        if (tidx != nullptr) acc[3 * s + i] += (double)tidx[i];
+        if (f & 4u) acc[4 * s + i] += 1.0;          // FLAG_COLLISION
+        if (f & 8u) acc[5 * s + i] += 1.0;          // FLAG_OOB
+        if (f & 16u) acc[6 * s + i] += 1.0;         // FLAG_COMPLETE
+        if (f & 32u) acc[7 * s + i] += 1.0;         // FLAG_STRIKE
+        r = 0.0;
+        l = 0;
+    }
+    ret[i] = r;
+    len[i] = l;
+}
+
+cudaError_t ppok_pop_episode_ledger(const float* rew, const uint8_t* flags, const uint8_t* tidx, int n, double* ret, int* len,
+                                    double* acc, cudaStream_t st) {
+    ppo_pop_episode_ledger_kernel<<<(n + 255) / 256, 256, 0, st>>>(rew, flags, tidx, n, ret, len, acc);
     return cudaGetLastError();
 }

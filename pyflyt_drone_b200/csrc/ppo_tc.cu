@@ -212,13 +212,31 @@ __device__ __forceinline__ void tc_load8(const float* __restrict__ obs_raw, floa
 
 // 512 threads = 4 warpgroups: TMEM lane (= env row of the tile) = tid & 127; warpgroup q = tid >> 7 owns hidden units
 // [32q, 32q+32) of the stacked pi|vf layers in both epilogues (q 0,1 = policy tower, 2,3 = value tower).
+// POP: population launch, grid (CTAs per member, members): blockIdx.y = member, whose weights, statistics, seed and rows the
+// CTA takes before it walks that member's tiles only (a member's tail tile is masked at its own n, as in a standalone launch)
+template <bool POP = false>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 ppo_forward_tc_kernel(const float* __restrict__ params, int d, const float* __restrict__ obs_raw,
                       const double* __restrict__ stats, float clip, int n, uint32_t seed_lo, uint32_t seed_hi,
                       uint32_t env_id0, uint32_t step, const uint32_t* __restrict__ step_dev, int deterministic,
                       float* __restrict__ obs_norm, float* __restrict__ act_env, float* __restrict__ act_raw,
-                      float* __restrict__ logp, float* __restrict__ value) {
+                      float* __restrict__ logp, float* __restrict__ value, PpokPop pop) {
     extern __shared__ __align__(1024) char smem[];
+    if constexpr (POP) {
+        const int m = blockIdx.y;
+        const size_t r0 = (size_t)m * n;
+        params += (size_t)m * pop.param_stride;
+        obs_raw += r0 * d;
+        if (stats != nullptr) stats += (size_t)m * (2 * d + 1);
+        const uint64_t seed = pop.seeds[m];
+        seed_lo = (uint32_t)(seed & 0xffffffffu); seed_hi = (uint32_t)(seed >> 32);
+        env_id0 += (uint32_t)r0;
+        if (obs_norm != nullptr) obs_norm += r0 * d;
+        act_env += r0 * A;
+        if (act_raw != nullptr) act_raw += r0 * A;
+        if (logp != nullptr) logp += r0;
+        value += r0;
+    }
     float* small = reinterpret_cast<float*>(smem + TcSmem::SMALL);
     const int tid = threadIdx.x, warp = tid >> 5;
     const int q = tid >> 7, lrow = tid & (TC_ROWS - 1);
@@ -428,25 +446,51 @@ ppo_forward_tc_kernel(const float* __restrict__ params, int d, const float* __re
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"((uint32_t)TC_TMEM_COLS) : "memory");
 }
 
+static int g_tc_sm_count = 0;
+static cudaError_t tc_setup() {
+    if (g_tc_sm_count != 0) return cudaSuccess;
+    int dev = 0, sms = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ppo_forward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::TOTAL);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ppo_forward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::TOTAL);
+    if (e != cudaSuccess) return e;
+    g_tc_sm_count = sms;
+    return cudaSuccess;
+}
+
 cudaError_t ppok_forward_tc(const float* params, int d, const float* obs_raw, const double* stats, float clip, int n,
                             uint64_t seed, uint32_t env_id0, uint32_t step, const uint32_t* step_dev, int deterministic,
                             float* obs_norm, float* act_env, float* act_raw, float* logp, float* value, cudaStream_t st) {
     if (d > DP) return cudaErrorInvalidValue;
-    static int sm_count = 0;
-    if (sm_count == 0) {
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e != cudaSuccess) return e;
-        e = cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(ppo_forward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::TOTAL);
-        if (e != cudaSuccess) { sm_count = 0; return e; }
-    }
+    cudaError_t e = tc_setup();
+    if (e != cudaSuccess) return e;
+    const int sm_count = g_tc_sm_count;
     const int ntiles = (n + TC_ROWS - 1) / TC_ROWS;
     const int grid = ntiles < sm_count ? ntiles : sm_count;          // persistent: one CTA per SM walks the tiles
     ppo_forward_tc_kernel<<<grid, TC_THREADS, TcSmem::TOTAL, st>>>(params, d, obs_raw, stats, clip, n, (uint32_t)(seed & 0xffffffffu),
                                                                (uint32_t)(seed >> 32), env_id0, step, step_dev, deterministic,
-                                                               obs_norm, act_env, act_raw, logp, value);
+                                                               obs_norm, act_env, act_raw, logp, value, PpokPop{});
+    return cudaGetLastError();
+}
+
+// n = rows per member.  Each member gets an equal share of the SMs (at least one CTA, at most one per tile); a CTA walks
+// only its member's tiles, so it stages one member's weights once, and every row sees the arithmetic of a standalone launch.
+cudaError_t ppok_pop_forward_tc(const PpokPop& pop, const float* params, int d, const float* obs_raw, const double* stats, float clip,
+                                int n, uint32_t env_id0, uint32_t step, const uint32_t* step_dev, int deterministic, float* obs_norm,
+                                float* act_env, float* act_raw, float* logp, float* value, cudaStream_t st) {
+    if (d > DP) return cudaErrorInvalidValue;
+    cudaError_t e = tc_setup();
+    if (e != cudaSuccess) return e;
+    const int ntiles = (n + TC_ROWS - 1) / TC_ROWS;
+    int per = g_tc_sm_count / pop.members;
+    if (per < 1) per = 1;
+    if (per > ntiles) per = ntiles;
+    ppo_forward_tc_kernel<true><<<dim3(per, pop.members), TC_THREADS, TcSmem::TOTAL, st>>>(
+        params, d, obs_raw, stats, clip, n, 0u, 0u, env_id0, step, step_dev, deterministic, obs_norm, act_env, act_raw, logp, value, pop);
     return cudaGetLastError();
 }
 

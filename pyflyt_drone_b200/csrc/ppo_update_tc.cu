@@ -412,13 +412,29 @@ __device__ __forceinline__ void ut_gather_async(char* smem, const float* __restr
 // activation columns [32q, 32q+32) of the stacked pi|vf layer (q 0,1 = policy tower, 2,3 = value tower) in every
 // epilogue, so the per-thread serial work is a quarter of a row and 16 warps hide each other's TMEM/SFU latency.
 // tanh' factors are kept in registers (packed bf16) from the forward epilogues instead of being recomputed.
-template <bool FUSED, bool P2P = false>
+//
+// POP (fused mode only): population launch of one CTA per member, blockIdx.y = member.  The CTA moves to its member's
+// parameters, Adam moments and step, gradient, statistics, grad-norm output and index window, and takes the member's learning
+// rate, clip range, entropy and value coefficients and max grad norm from its hyper-parameter record; the body is unchanged.
+template <bool FUSED, bool P2P = false, bool POP = false>
 __global__ void __launch_bounds__(UT_THREADS, 1)
 ppo_grad_tc_kernel(const float* params, int d, const float* __restrict__ obs, const float* __restrict__ act,
                    const float* __restrict__ logp_old, const float* __restrict__ adv, const float* __restrict__ ret,
                    const long long* __restrict__ idx_all, int batch, const float* __restrict__ adv_stats, PpoLossCfg cfg,
-                   float* out_partial, float* __restrict__ out_stats, int P, PpoFusedCfg fz) {
+                   float* out_partial, float* __restrict__ out_stats, int P, PpoFusedCfg fz, PpokPop pop) {
     extern __shared__ __align__(1024) char smem[];
+    if constexpr (POP) {
+        const int mb = blockIdx.y;
+        const size_t po = (size_t)mb * pop.param_stride;
+        const float* h = pop.hp + (size_t)mb * PPO_POP_HP;
+        params += po; fz.params += po; fz.m += po; fz.v += po; out_partial += po;
+        fz.step_ctr += mb;
+        if (fz.norm_out != nullptr) fz.norm_out += mb;
+        out_stats += (size_t)mb * 8;
+        idx_all += (size_t)mb * pop.idx_stride;
+        fz.lr = h[PPO_POP_LR]; fz.max_norm = h[PPO_POP_MAX_GRAD_NORM];
+        cfg.clip_range = h[PPO_POP_CLIP_RANGE]; cfg.ent_coef = h[PPO_POP_ENT_COEF]; cfg.vf_coef = h[PPO_POP_VF_COEF];
+    }
     float* small = reinterpret_cast<float*>(smem + UtSmem::SMALL);
     const int tid = threadIdx.x, warp = tid >> 5;
     const int q = tid >> 7;                  // warpgroup = column block
@@ -1323,7 +1339,7 @@ cudaError_t ppok_minibatch_grad(const float* params, int d, const float* obs, co
     PpoLossCfg cfg{clip_range, ent_coef, vf_coef, 1.0f / (float)batch, gs, 1.0f / gs};
     PpoFusedCfg fz{};
     ppo_grad_tc_kernel<false><<<grid, UT_THREADS, UtSmem::TOTAL, st>>>(params, d, obs, act, logp_old, adv, ret, idx, batch, adv_stats, cfg,
-                                                             partial, stats_partial, P, fz);
+                                                             partial, stats_partial, P, fz, PpokPop{});
     ppok_launch_grad_reduce(partial, stats_partial, grid, P, grad, stats, adam, st);
     return cudaGetLastError();
 }
@@ -1351,10 +1367,37 @@ cudaError_t ppok_minibatch_steps(float* params, int d, const float* obs, const f
     for (int j = 0; j < PEER_MAX_WORLD; ++j) fz.peer[j] = (world > 1 && j < world) ? static_cast<float*>(peers[j]) : nullptr;
     if (world > 1)
         ppo_grad_tc_kernel<true, true><<<1, UT_THREADS, UtSmem::TOTAL, st>>>(params, d, obs, act, logp_old, adv, ret, idx, batch, nullptr,
-                                                                          cfg, grad, stats, P, fz);
+                                                                          cfg, grad, stats, P, fz, PpokPop{});
     else
         ppo_grad_tc_kernel<true, false><<<1, UT_THREADS, UtSmem::TOTAL, st>>>(params, d, obs, act, logp_old, adv, ret, idx, batch, nullptr,
-                                                                           cfg, grad, stats, P, fz);
+                                                                           cfg, grad, stats, P, fz, PpokPop{});
+    return cudaGetLastError();
+}
+
+// Population form: one CTA per member (grid (1, members)), each running `steps` consecutive optimizer steps of its own
+// member over idx[m * pop.idx_stride ..]; the per-member loss and optimizer hyper-parameters come from pop.hp, the parameter
+// vectors, Adam moments and gradients are pop.param_stride floats apart, step_ctr / norm_out hold one entry and stats 8
+// floats per member.
+static bool g_ut_pop_attr_set = false;
+cudaError_t ppok_pop_minibatch_steps(const PpokPop& pop, float* params, int d, const float* obs, const float* act, const float* logp_old,
+                                     const float* adv, const float* ret, const long long* idx, int batch, int steps, float* m, float* v,
+                                     float beta1, float beta2, float eps, int* step_ctr, float* norm_out, float* grad, float* stats,
+                                     cudaStream_t st) {
+    if (d > DP || steps <= 0) return cudaErrorInvalidValue;
+    if (!g_ut_pop_attr_set) {
+        cudaError_t e = cudaFuncSetAttribute(ppo_grad_tc_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             UtSmem::TOTAL);
+        if (e != cudaSuccess) return e;
+        g_ut_pop_attr_set = true;
+    }
+    const int H_ = PPO_H, A_ = A;
+    const int P = (H_ * d + H_ + H_ * H_ + H_ + A_ * H_ + A_) + (H_ * d + H_ + H_ * H_ + H_ + H_ + 1) + A_;
+    float gs = 1.0f;
+    while (gs < (float)batch && gs < 1048576.0f) gs *= 2.0f;
+    PpoLossCfg cfg{0.0f, 0.0f, 0.0f, 1.0f / (float)batch, gs, 1.0f / gs};
+    PpoFusedCfg fz{steps, 0.0f, beta1, beta2, eps, 0.0f, params, m, v, step_ctr, norm_out, 1, 0, nullptr, {}};
+    ppo_grad_tc_kernel<true, false, true><<<dim3(1, pop.members), UT_THREADS, UtSmem::TOTAL, st>>>(
+        params, d, obs, act, logp_old, adv, ret, idx, batch, nullptr, cfg, grad, stats, P, fz, pop);
     return cudaGetLastError();
 }
 }  // namespace PPO_UT_NS
