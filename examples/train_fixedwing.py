@@ -3,7 +3,8 @@
 
 Counterpart of /root/reference/train/train_Fixedwing_Waypoints_v3.py (--task waypoints) and
 train_Fixedwing_Waypoints_ObjLock.py (--task objlock) / train_lowlevel_cmd.py (--task lowlevel) / train_objlock.py
-(--task duck, the duck-only lock-and-strike env): same hyper-parameter dictionary, same flow
+(--task duck, the duck-only lock-and-strike env) / train_highlevel_cmd.py (--task highlevel --tracker PATH, waypoints flown
+through a frozen --task lowlevel policy): same hyper-parameter dictionary, same flow
 (vectorised env -> observation/reward normalisation -> PPO("MlpPolicy", ...).learn -> save model + vecnorm),
 with SubprocVecEnv/VecNormalize/PPO replaced by their device-resident equivalents.
 
@@ -41,6 +42,13 @@ TRAIN_CONFIG = {
         "gamma": 0.99, "gae_lambda": 0.95, "clip_range": 0.2, "ent_coef": 0.001, "vf_coef": 0.5, "max_grad_norm": 0.5, "seed": 42,
         "model_dir": "models/obj_lock_only_ppo_b200", "preset": "objlock_duck",
     },
+    "highlevel": {   # train_highlevel_cmd.py: the waypoints episode commanded through a frozen tracker (--tracker)
+        "total_timesteps": 4_000_000, "num_envs": 32, "num_targets": 8, "goal_reach_distance": 4, "sparse_reward": True,
+        "learning_rate": 3e-4, "n_steps": 2048, "batch_size": 128, "n_epochs": 20, "gamma": 0.99, "gae_lambda": 0.95,
+        "clip_range": 0.2, "ent_coef": 0.001, "vf_coef": 0.5, "max_grad_norm": 0.5, "seed": 42,
+        "model_dir": "models/highlevel_ppo_b200", "flight_dome_size": 100.0, "max_duration_seconds": 120.0,
+        "context_length": 2, "preset": "highlevel",
+    },
 }
 
 
@@ -54,7 +62,11 @@ def main():
     ap.add_argument("--pretrained_model", type=str, default=None)
     ap.add_argument("--eval_freq", type=int, default=10_000, help="timesteps between evaluations (20 episodes each)")
     ap.add_argument("--save_freq", type=int, default=50_000, help="timesteps between checkpoints")
+    ap.add_argument("--tracker", type=str, default=None,
+                    help="--task highlevel: the low-level tracker (a PPO.save file of --task lowlevel, or an SB3 directory)")
     args = ap.parse_args()
+    if (args.task == "highlevel") != (args.tracker is not None):
+        ap.error("--tracker is required with --task highlevel, and only with it")
     cfg = dict(TRAIN_CONFIG[args.task])
     for k in ("num_envs", "n_steps", "batch_size", "total_timesteps"):
         if getattr(args, k) is not None:
@@ -69,6 +81,7 @@ def main():
 
     from pyflyt_drone_b200.callbacks import CheckpointCallback, EvalCallback
     from pyflyt_drone_b200.ppo import PPO
+    from pyflyt_drone_b200.tracker import Tracker
     from pyflyt_drone_b200.vec_env import FixedwingVecEnv
 
     if args.task in ("lowlevel", "duck"):       # the preset carries the whole env configuration of the script
@@ -79,7 +92,8 @@ def main():
                               env_id0=rank * cfg["num_envs"], num_targets=cfg["num_targets"],
                               goal_reach=float(cfg["goal_reach_distance"]), sparse_reward=int(cfg["sparse_reward"]),
                               dome=cfg["flight_dome_size"], max_steps=int(30 * cfg["max_duration_seconds"]),
-                              context_len=cfg["context_length"])
+                              context_len=cfg["context_length"],
+                              tracker=Tracker.load(args.tracker) if args.tracker else None)
     model = PPO("MlpPolicy", env, learning_rate=cfg["learning_rate"], n_steps=cfg["n_steps"], batch_size=cfg["batch_size"],
                 n_epochs=cfg["n_epochs"], gamma=cfg["gamma"], gae_lambda=cfg["gae_lambda"], clip_range=cfg["clip_range"],
                 ent_coef=cfg["ent_coef"], vf_coef=cfg["vf_coef"], max_grad_norm=cfg["max_grad_norm"], seed=cfg["seed"],

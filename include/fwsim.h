@@ -58,6 +58,7 @@ extern "C" {
 #define FW_TASK_OBJLOCK   2   /* FixedwingWaypointObjLockEnv + FlattenWaypointEnv */
 #define FW_TASK_LOWLEVEL  3   /* FixedwingLowLevelEnv (envs/fixedwing_envs/fixedwing_lowlevel_env.py) */
 #define FW_TASK_DUCK      4   /* FixedwingObjLockEnv + FlattenObjLockEnv (envs/fixedwing_objlock_env.py, flatten_objlock_env.py) */
+#define FW_TASK_HIGHLEVEL 5   /* the Waypoints episode of task 1 flown through a frozen low-level tracker (fw_set_tracker) */
 
 /* Everything the kernels need to know about the aircraft and the task.  Raw physical parameters only;
  * derived constants are computed inside fw_create. */
@@ -99,7 +100,8 @@ typedef struct FwConfig {
     int32_t freestream_3d, cd90_degrees;
     int32_t task;   /* 0 physics only, 1 Waypoints-v3, 2 Waypoint+ObjLock, 3 low-level tracking (FixedwingLowLevelEnv:
                      * 21-float obs, 6-channel action, one Aviary.step per env step, truncation at step_count >= max_steps),
-                     * 4 duck-only lock/strike (FixedwingObjLockEnv: attitude + target_vector + 9*history (+4 deltas) obs) */
+                     * 4 duck-only lock/strike (FixedwingObjLockEnv: attitude + target_vector + 9*history (+4 deltas) obs),
+                     * 5 high-level waypoints (task 1 through a frozen low-level tracker, fw_set_tracker) */
     int32_t num_targets, sparse_reward, angle_repr, max_steps, context_len;
     int32_t early_return_on_crash, complete_truncates;
     int32_t wind_mode, wind_randomize, wind_rand_phase, wind_start_substep;   /* wind_mode: 0 off, 1 constant, 2 gust_sine,
@@ -179,6 +181,42 @@ int fw_destroy(fw_handle h);
  * returns FW_ESTATE, a handle of another wind mode FW_EINVAL.  The field stays fixed for the handle's lifetime (fw_destroy frees
  * it), so every launch and CUDA graph sees the same field. */
 int fw_set_wind_field(fw_handle h, const FwWindField* field);
+
+/* High-level waypoints (FwConfig.task = 5): the hierarchical flow the reference starts in train/train_highlevel_cmd.py and
+ * examples/lowlevel.py.  Everything is task 1 (Waypoints: targets, reward, termination, flags, the 28/29-float observation
+ * with the agent's action in slots 12-15, reset and wind) except how the action reaches the aircraft.  The agent's action
+ * a in R^4 is a command
+ *     psi_ref = atan2(a1, a0)       (a direction vector: no wrap at +-pi; atan2(0, 0) = 0)
+ *     h_ref   = h_lo + (clamp(a2, -1, 1) + 1) / 2 * (h_hi - h_lo)
+ *     V_ref   = v_lo + (clamp(a3, -1, 1) + 1) / 2 * (v_hi - v_lo)
+ * and each of the inner_per_step inner iterations (120 Hz) is one decision of a frozen low-level tracker followed by one
+ * Aviary.step: the tracker sees task 3's 21-float observation with [psi_ref, h_ref, V_ref] as its target and its own
+ * previous action (per-env state, zero after a reset, carried across agent steps), normalised by its frozen VecNormalize
+ * statistics ((x - mean) / sqrt(var + 1e-8) clipped to +-clip_obs); its policy tower's mean, clipped to [-1, 1], is the
+ * six-channel mode -1 command (the arithmetic of ppo_policy_forward_a with deterministic = 1, bit for bit).
+ * The ranges default to task 3's reference distribution: h in [5, 20] m, V in [10, 20] m/s. */
+typedef struct FwTracker {
+    const float* params;      /* HOST: the flat parameter vector of include/fwppo.h for (obs 21, action 6),
+                               * ppo_param_count_a(21, 6) floats; only the policy tower is read */
+    const double* obs_mean;   /* HOST [21] VecNormalize obs_rms.mean, or NULL (un-normalised tracker) */
+    const double* obs_var;    /* HOST [21] obs_rms.var (>= 0), NULL exactly when obs_mean is */
+    double clip_obs;          /* > 0 */
+    double h_range[2];        /* altitude command range, metres, lo < hi */
+    double v_range[2];        /* airspeed command range, m/s, lo < hi */
+} FwTracker;
+
+/* Install the tracker of a task 5 handle.  fw_create with task 5 allocates the batch but defers its first reset to this call
+ * (after fw_set_wind_field as well, for a wind_mode 3 handle: whichever of the two comes last runs it); step, reset and
+ * observe entry points return FW_ESTATE until then.  Synchronous and one-shot: the descriptor is validated (finite values,
+ * var >= 0, lo < hi, clip_obs > 0) before the device is touched, then copied to handle-owned device memory; a second call
+ * returns FW_ESTATE, a handle of another task FW_EINVAL.  fw_rollout_random and fw_render return FW_EINVAL for task 5. */
+int fw_set_tracker(fw_handle h, const FwTracker* tracker);
+/* The tracker's previous action of every env, HOST [N, 6] (parity injection / inspection; synchronous). */
+int fw_get_tracker_state(fw_handle h, float* prev_host);
+int fw_set_tracker_state(fw_handle h, const float* prev_host);
+/* Opt-in: obs_dev = device [N, 21] floats (NULL clears it).  Every step enqueued while it is set writes the raw (un-normalised)
+ * tracker observation of each env's last tracker decision of that step; nothing is written while it is NULL. */
+int fw_set_tracker_obs_buffer(fw_handle h, float* obs_dev);
 int fw_num_envs(fw_handle h);
 int fw_obs_dim(fw_handle h);
 /* action width: 4 ([roll, pitch, yaw, thrust], Fixedwing mode 0) or 6 for task 3, the low-level env

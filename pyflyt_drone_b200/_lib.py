@@ -30,6 +30,14 @@ class FwWindFieldC(C.Structure):
     ]
 
 
+class FwTrackerC(C.Structure):
+    """include/fwsim.h FwTracker (the frozen low-level tracker of the high-level waypoint task, task 5)."""
+    _fields_ = [
+        ("params", C.c_void_p), ("obs_mean", C.c_void_p), ("obs_var", C.c_void_p), ("clip_obs", C.c_double),
+        ("h_range", C.c_double * 2), ("v_range", C.c_double * 2),
+    ]
+
+
 class FwError(RuntimeError):
     pass
 
@@ -45,6 +53,10 @@ SYMBOLS = [
     ("fw_create", C.c_int, [C.POINTER(FwConfigC), C.c_int32, C.c_int32, C.c_uint64, C.c_uint32, C.POINTER(_P)]),
     ("fw_destroy", C.c_int, [_P]),
     ("fw_set_wind_field", C.c_int, [_P, C.POINTER(FwWindFieldC)]),
+    ("fw_set_tracker", C.c_int, [_P, C.POINTER(FwTrackerC)]),
+    ("fw_get_tracker_state", C.c_int, [_P, _P]),
+    ("fw_set_tracker_state", C.c_int, [_P, _P]),
+    ("fw_set_tracker_obs_buffer", C.c_int, [_P, _P]),
     ("fw_num_envs", C.c_int, [_P]),
     ("fw_obs_dim", C.c_int, [_P]),
     ("fw_act_dim", C.c_int, [_P]),

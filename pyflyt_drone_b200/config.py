@@ -18,7 +18,7 @@ from . import aircraft
 
 NSURF, MAX_TARGETS, MAX_COL, MAX_OBST = 5, 16, 16, 32
 
-TASK_PHYSICS, TASK_WAYPOINTS, TASK_OBJLOCK, TASK_LOWLEVEL, TASK_DUCK = 0, 1, 2, 3, 4
+TASK_PHYSICS, TASK_WAYPOINTS, TASK_OBJLOCK, TASK_LOWLEVEL, TASK_DUCK, TASK_HIGHLEVEL = 0, 1, 2, 3, 4, 5
 MAX_HIST = 4
 
 FLAG_TERM, FLAG_TRUNC, FLAG_COLLISION, FLAG_OOB, FLAG_COMPLETE, FLAG_STRIKE, FLAG_FAULT = 1, 2, 4, 8, 16, 32, 64
@@ -372,8 +372,15 @@ def objlock_duck(wind: dict | None = None, **overrides) -> EnvConfig:
     return cfg.replace(**overrides) if overrides else cfg
 
 
+def highlevel(wind: dict | None = None, **overrides) -> EnvConfig:
+    """High-level waypoints (task 5): the waypoints_v3 episode, its action a command [psi, h, V] that a frozen low-level
+    tracker (pyflyt_drone_b200.tracker.Tracker, trained on the ``lowlevel`` preset) flies at 120 Hz -- the flow of the
+    reference's train/train_highlevel_cmd.py and examples/lowlevel.py.  FixedwingVecEnv needs ``tracker=``."""
+    return waypoints_v3(wind=wind, **{"task": TASK_HIGHLEVEL, **overrides})
+
+
 PRESETS = {"waypoints_v3": waypoints_v3, "waypoint_objlock": waypoint_objlock, "physics_only": physics_only,
-           "lowlevel": lowlevel, "objlock_duck": objlock_duck}
+           "lowlevel": lowlevel, "objlock_duck": objlock_duck, "highlevel": highlevel}
 
 
 def from_gym_kwargs(preset: str = "waypoints_v3", *, sparse_reward=None, num_targets=None, goal_reach_distance=None,

@@ -67,11 +67,18 @@ struct FwSim {
     // gridded wind field (wind_mode 3): device lattice, and whether the batch still waits for it (fw_set_wind_field)
     float4* wf_mem;
     bool field_pending;
+    // high-level waypoint task (task 5): the frozen tracker's device copies (one allocation: policy tower, statistics, the
+    // previous-action plane) and whether the batch still waits for it (fw_set_tracker)
+    char* trk_mem;
+    FwTrk trk;
+    bool tracker_pending;
 };
 
-// step / reset / rollout entry points on a wind_mode 3 handle whose field has not been installed yet
+// step / reset / rollout entry points on a handle whose wind field (wind_mode 3) or tracker (task 5) is not installed yet
 static int need_field(const FwSim* h) {
-    return h->field_pending ? fail(FW_ESTATE, "wind_mode 3: install the wind field with fw_set_wind_field first") : FW_OK;
+    if (h->field_pending) return fail(FW_ESTATE, "wind_mode 3: install the wind field with fw_set_wind_field first");
+    if (h->tracker_pending) return fail(FW_ESTATE, "task 5: install the low-level tracker with fw_set_tracker first");
+    return FW_OK;
 }
 
 // host-lane entry: wait for device-lane launches that may still be running on the caller's streams
@@ -118,7 +125,9 @@ static int derive(const FwConfig& c, int n, uint64_t seed, uint32_t env_id0, FwD
     const double PI = 3.14159265358979323846, DEG = PI / 180.0;
     if (!(c.dt > 0) || !(c.mass > 0)) return fail(FW_EINVAL, "dt and mass must be positive");
     if (c.wind_mode < 0 || c.wind_mode > 3) return fail(FW_EINVAL, "wind_mode %d unknown (0 off, 1 constant, 2 gust_sine, 3 gridded field)", c.wind_mode);
-    if (c.task < 0 || c.task > 4) return fail(FW_EINVAL, "task %d unknown (0 physics, 1 waypoints, 2 waypoint+objlock, 3 low-level, 4 duck-only objlock)", c.task);
+    if (c.task < 0 || c.task > 5)
+        return fail(FW_EINVAL, "task %d unknown (0 physics, 1 waypoints, 2 waypoint+objlock, 3 low-level, 4 duck-only objlock, "
+                    "5 high-level waypoints)", c.task);
     const bool cam_task = c.task == 2 || c.task == 4;
     if (cam_task && (c.num_obstacles < 0 || c.num_obstacles > FW_MAX_OBST)) return fail(FW_EINVAL, "num_obstacles out of range");
     if (cam_task && (c.cam_res < 3 || c.cam_res > 1024)) return fail(FW_EINVAL, "cam_res out of range");
@@ -421,15 +430,15 @@ static int fw_create_impl(const FwConfig* cfg, int32_t n_envs, int32_t device, u
     CU(cudaStreamCreateWithFlags(&h->io_stream, cudaStreamNonBlocking));
     h->io_streams[0] = h->io_stream;
     CU(cudaStreamCreateWithFlags(&h->io_streams[1], cudaStreamNonBlocking));
-    if (h->dev.wind_mode == 3) {          // the first reset needs the field: fw_set_wind_field runs the set-up
-        h->field_pending = true;
-        return FW_OK;
-    }
+    // the first reset needs the field and the tracker: the last of fw_set_wind_field / fw_set_tracker runs the set-up
+    h->field_pending = h->dev.wind_mode == 3;
+    h->tracker_pending = h->dev.task == 5;
+    if (h->field_pending || h->tracker_pending) return FW_OK;
     return initial_episodes(h);
 }
 
 // The warm-up cache decision, the first reset of every env and the spare episodes of the camera tasks: the tail of fw_create,
-// or of fw_set_wind_field for a wind_mode 3 handle.
+// or of whichever of fw_set_wind_field (wind_mode 3) and fw_set_tracker (task 5) completes the handle.
 static int initial_episodes(FwSim* h) {
     cudaError_t ce;
     const FwConfig* cfg = &h->cfg;
@@ -492,7 +501,7 @@ static int initial_episodes(FwSim* h) {
 static int launch_step(FwSim* h, const FwDev& dev, FwPlanes pl, const float* act, float* obs, float* rew, uint8_t* flg,
                        float* term_obs, bool random_act, int spl, cudaStream_t st) {
     if (!h->spare_on) {
-        CU(fwk_launch_step(dev, pl, act, obs, rew, flg, term_obs, random_act, spl, st));
+        CU(fwk_launch_step(dev, pl, act, obs, rew, flg, term_obs, random_act, spl, st, &h->trk));
         h->launches++;
         return FW_OK;
     }
@@ -524,6 +533,7 @@ extern "C" int fw_destroy(fw_handle h) {
             }
     if (h->plane_mem) cudaFree(h->plane_mem);
     if (h->wf_mem) cudaFree(h->wf_mem);
+    if (h->trk_mem) cudaFree(h->trk_mem);
     if (h->d_act) cudaFree(h->d_act);
     if (h->d_obs) cudaFree(h->d_obs);
     if (h->d_rew) cudaFree(h->d_rew);
@@ -599,7 +609,105 @@ extern "C" int fw_set_wind_field(fw_handle h, const FwWindField* f) {
     d.wf_period = (float)(f->nt * f->t_step);
     d.wf_rand_time = f->randomize_time != 0;
     h->field_pending = false;
-    return initial_episodes(h);
+    return h->tracker_pending ? FW_OK : initial_episodes(h);
+}
+
+// floats of the policy tower at the head of the flat (21, 6) parameter vector (include/fwppo.h)
+static const size_t TRK_TOWER = (size_t)64 * FW_TRK_OBS + 64 + 64 * 64 + 64 + FW_TRK_ACT * 64 + FW_TRK_ACT;
+
+static bool finite_range(const double r[2]) { return std::isfinite(r[0]) && std::isfinite(r[1]) && r[0] < r[1]; }
+
+extern "C" int fw_set_tracker(fw_handle h, const FwTracker* t) {
+    // argument checks first, without touching the device
+    if (!t) return fail(FW_EINVAL, "null tracker");
+    if (!t->params) return fail(FW_EINVAL, "tracker: params is null");
+    if ((t->obs_mean == nullptr) != (t->obs_var == nullptr))
+        return fail(FW_EINVAL, "tracker: obs_mean and obs_var are both set (normalised tracker) or both null");
+    for (size_t k = 0; k < TRK_TOWER; ++k)
+        if (!std::isfinite(t->params[k])) return fail(FW_EINVAL, "tracker: policy parameter %zu is not finite", k);
+    if (t->obs_mean)
+        for (int k = 0; k < FW_TRK_OBS; ++k) {
+            if (!std::isfinite(t->obs_mean[k])) return fail(FW_EINVAL, "tracker: obs_mean[%d] is not finite", k);
+            if (!std::isfinite(t->obs_var[k]) || t->obs_var[k] < 0) return fail(FW_EINVAL, "tracker: obs_var[%d] must be finite and >= 0", k);
+        }
+    if (!(t->clip_obs > 0) || !std::isfinite(t->clip_obs)) return fail(FW_EINVAL, "tracker: clip_obs must be finite and > 0");
+    if (!finite_range(t->h_range)) return fail(FW_EINVAL, "tracker: h_range must be finite with lo < hi");
+    if (!finite_range(t->v_range)) return fail(FW_EINVAL, "tracker: v_range must be finite with lo < hi");
+    if (!h) return fail(FW_EINVAL, "null handle");
+    if (h->dev.task != 5) return fail(FW_EINVAL, "fw_set_tracker needs a handle created with task 5 (has %d)", h->dev.task);
+    if (!h->tracker_pending) return fail(FW_ESTATE, "the tracker of this handle is already set (one tracker per handle)");
+    CU(cudaSetDevice(h->device));
+    // one allocation: tower | statistics (mean 21 | var 21, doubles) | previous-action plane [6][N], zeroed
+    const size_t N = (size_t)h->n;
+    const size_t off_stats = align_up(TRK_TOWER * sizeof(float), 256), off_prev = off_stats + align_up(2 * FW_TRK_OBS * sizeof(double), 256);
+    const size_t bytes = off_prev + (size_t)FW_TRK_ACT * N * sizeof(float);
+    std::vector<double> stats(2 * FW_TRK_OBS);
+    if (t->obs_mean)
+        for (int k = 0; k < FW_TRK_OBS; ++k) { stats[k] = t->obs_mean[k]; stats[FW_TRK_OBS + k] = t->obs_var[k]; }
+    cudaError_t ce = cudaMalloc((void**)&h->trk_mem, bytes);
+    if (ce != cudaSuccess) { h->trk_mem = nullptr; return fail(FW_ENOMEM, "cudaMalloc(%zu) for the tracker: %s", bytes, cudaGetErrorString(ce)); }
+    ce = cudaMemcpyAsync(h->trk_mem, t->params, TRK_TOWER * sizeof(float), cudaMemcpyHostToDevice, h->io_stream);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(h->trk_mem + off_stats, stats.data(), stats.size() * sizeof(double), cudaMemcpyHostToDevice, h->io_stream);
+    if (ce == cudaSuccess) ce = cudaMemsetAsync(h->trk_mem + off_prev, 0, (size_t)FW_TRK_ACT * N * sizeof(float), h->io_stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(h->io_stream);
+    if (ce != cudaSuccess) {                  // the handle stays pending: a later call may try again
+        cudaFree(h->trk_mem);
+        h->trk_mem = nullptr;
+        return fail(FW_ECUDA, "uploading the tracker: %s", cudaGetErrorString(ce));
+    }
+    FwTrk& k = h->trk;
+    k.params = reinterpret_cast<const float*>(h->trk_mem);
+    k.stats = t->obs_mean ? reinterpret_cast<const double*>(h->trk_mem + off_stats) : nullptr;
+    k.clip = (float)t->clip_obs;
+    k.h_lo = (float)t->h_range[0]; k.h_hi = (float)t->h_range[1];
+    k.v_lo = (float)t->v_range[0]; k.v_hi = (float)t->v_range[1];
+    k.prev = reinterpret_cast<float*>(h->trk_mem + off_prev);
+    h->tracker_pending = false;
+    return h->field_pending ? FW_OK : initial_episodes(h);
+}
+
+// the tracker entry points below need an installed tracker
+static int need_tracker(const FwSim* h) {
+    if (!h) return fail(FW_EINVAL, "null handle");
+    if (h->dev.task != 5) return fail(FW_EINVAL, "the tracker entry points need a task 5 handle (has %d)", h->dev.task);
+    if (h->tracker_pending) return fail(FW_ESTATE, "task 5: install the low-level tracker with fw_set_tracker first");
+    return FW_OK;
+}
+
+extern "C" int fw_get_tracker_state(fw_handle h, float* prev_host) {
+    if (!prev_host) return fail(FW_EINVAL, "null argument");
+    int rc = need_tracker(h);
+    if (rc != FW_OK) return rc;
+    CU(cudaSetDevice(h->device));
+    const size_t N = (size_t)h->n;
+    std::vector<float> soa((size_t)FW_TRK_ACT * N);
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpy(soa.data(), h->trk.prev, soa.size() * sizeof(float), cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < N; ++i)
+        for (int c = 0; c < FW_TRK_ACT; ++c) prev_host[i * FW_TRK_ACT + c] = soa[(size_t)c * N + i];
+    return FW_OK;
+}
+
+extern "C" int fw_set_tracker_state(fw_handle h, const float* prev_host) {
+    if (!prev_host) return fail(FW_EINVAL, "null argument");
+    int rc = need_tracker(h);
+    if (rc != FW_OK) return rc;
+    CU(cudaSetDevice(h->device));
+    const size_t N = (size_t)h->n;
+    std::vector<float> soa((size_t)FW_TRK_ACT * N);
+    for (size_t i = 0; i < N; ++i)
+        for (int c = 0; c < FW_TRK_ACT; ++c) soa[(size_t)c * N + i] = prev_host[i * FW_TRK_ACT + c];
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpy(h->trk.prev, soa.data(), soa.size() * sizeof(float), cudaMemcpyHostToDevice));
+    h->fresh = false;
+    return FW_OK;
+}
+
+extern "C" int fw_set_tracker_obs_buffer(fw_handle h, float* obs_dev) {
+    if (!h) return fail(FW_EINVAL, "null handle");
+    if (h->dev.task != 5) return fail(FW_EINVAL, "fw_set_tracker_obs_buffer needs a task 5 handle (has %d)", h->dev.task);
+    h->trk.obs_out = obs_dev;         // read by the step launches enqueued from now on (by value, at launch time)
+    return FW_OK;
 }
 
 extern "C" int fw_num_envs(fw_handle h) { return h ? h->n : fail(FW_EINVAL, "null handle"); }
@@ -615,6 +723,10 @@ extern "C" int fw_reset(fw_handle h, const uint8_t* mask_dev, float* obs_dev, vo
     const bool emit_only = h->fresh && mask_dev == nullptr;
     CU(fwk_launch_reset(h->dev, h->pl, mask_dev, obs_dev, emit_only, (cudaStream_t)stream));
     h->launches++;
+    if (h->dev.task == 5 && !emit_only) {       // a reset episode starts with the tracker's previous action at zero
+        CU(fwk_launch_tracker_clear(mask_dev, h->trk.prev, h->n, (cudaStream_t)stream));
+        h->launches++;
+    }
     h->fresh = false;
     h->dev_lane_dirty = true;
     return FW_OK;
@@ -655,6 +767,7 @@ extern "C" int fw_rollout_random(const fw_handle* hs, int32_t n_handles, int32_t
     for (int k = 0; k < n_handles; ++k) {
         if (!hs[k]) return fail(FW_EINVAL, "null handle in list");
         if (hs[k]->device != hs[0]->device) return fail(FW_EINVAL, "handles of one rollout must share a device");
+        if (hs[k]->dev.task == 5) return fail(FW_EINVAL, "fw_rollout_random does not run task 5 (high-level waypoints): use fw_step_random");
         if (need_field(hs[k]) != FW_OK) return FW_ESTATE;
         hs[k]->fresh = false;
         hs[k]->dev_lane_dirty = true;
@@ -766,7 +879,8 @@ extern "C" int fw_step_host(fw_handle h, const float* act_host, float* obs_host,
         FwPlanes plh = h->pl;
         plh.tidx_out = h->h_tidx;          // info["num_targets_reached"] goes straight to the host like the flags
         if (h->spare_on) { plh.refill_list = h->refill_list[par]; plh.refill_count = h->refill_ctl + par; }
-        CU(fwk_launch_step(pc, plh, act_dev_view ? act_dev_view : h->h_act, obs_dst, h->h_rew, h->h_flg, term_dst, false, 1, st));
+        CU(fwk_launch_step(pc, plh, act_dev_view ? act_dev_view : h->h_act, obs_dst, h->h_rew, h->h_flg, term_dst, false, 1, st,
+                           &h->trk));
         h->launches++;
         if (!zc_obs) {
             if (obs_host && D) CU(cudaMemcpyAsync(h->h_obs + n0 * D, h->d_obs + n0 * D, cn * D * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -831,6 +945,7 @@ extern "C" int fw_render(fw_handle h, int32_t env, int32_t width, int32_t height
     if (env < 0 || env >= h->n) return fail(FW_EINVAL, "env index %d out of range [0,%d)", env, h->n);
     if (width <= 0 || height <= 0 || width > 4096 || height > 4096) return fail(FW_EINVAL, "frame size must be in [1,4096]");
     if (!rgba_dev && !seg_dev && !depth_dev) return fail(FW_EINVAL, "no output buffer");
+    if (h->dev.task == 5) return fail(FW_EINVAL, "fw_render does not draw task 5 (high-level waypoints)");
     CU(cudaSetDevice(h->device));
     CU(fwk_render(h->dev, h->pl, env, width, height, rgba_dev, seg_dev, depth_dev, (cudaStream_t)stream));
     h->launches++;
@@ -875,6 +990,9 @@ static int reset_host_impl(fw_handle h, float* obs_host, bool observe_only) {
     cudaStream_t st = h->io_stream;
     CU(fwk_launch_reset(h->dev, h->pl, nullptr, D ? h->d_obs : nullptr, h->fresh || observe_only, st));
     h->launches++;
+    if (h->dev.task == 5 && !(h->fresh || observe_only)) {
+        CU(cudaMemsetAsync(h->trk.prev, 0, (size_t)FW_TRK_ACT * h->n * sizeof(float), st));
+    }
     if (!observe_only) h->fresh = false;
     if (obs_host && D) CU(cudaMemcpyAsync(h->h_obs, h->d_obs, N * D * sizeof(float), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));

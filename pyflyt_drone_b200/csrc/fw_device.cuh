@@ -724,10 +724,12 @@ __device__ __forceinline__ void fw_write_obs(const FwDev& p, const FwPlanes& pl,
 }
 
 // FixedwingLowLevelEnv._compute_obs (fixedwing_lowlevel_env.py:143-156): Aviary.state(0) flattened
-// [ang_vel_body, euler, lin_vel_body, lin_pos], the previous action (6) and the target [psi_ref, h_ref, V_ref];
-// also returns yaw and the body-frame speed the reward needs
-__device__ __forceinline__ void fw_write_obs_lowlevel(const FwPlanes& pl, const EnvState& e, int i, int n, const float a[6],
-                                                      float* o, float& yaw_out, float& speed_out, float tref[3]) {
+// [ang_vel_body, euler, lin_vel_body, lin_pos], the previous action (6) and the target [psi_ref, h_ref, V_ref], which
+// refs(tref) fills: task 3 reads its target plane (fw_write_obs_lowlevel), task 5 passes the high-level command.  Also
+// returns yaw and the body-frame speed the reward needs.
+template <class Refs>
+__device__ __forceinline__ void fw_write_obs_tracking(const EnvState& e, const float a[6], const Refs& refs, float* o,
+                                                      float& yaw_out, float& speed_out, float tref[3]) {
     Mat3 R = fw_quat_mat(e.qx, e.qy, e.qz, e.qw);
     const float* m = R.m;
     float roll, pitch, yaw;
@@ -735,7 +737,7 @@ __device__ __forceinline__ void fw_write_obs_lowlevel(const FwPlanes& pl, const 
     const float vbx = m[0] * e.vx + m[3] * e.vy + m[6] * e.vz;
     const float vby = m[1] * e.vx + m[4] * e.vy + m[7] * e.vz;
     const float vbz = m[2] * e.vx + m[5] * e.vy + m[8] * e.vz;
-    tref[0] = pl.targets[(size_t)0 * n + i]; tref[1] = pl.targets[(size_t)1 * n + i]; tref[2] = pl.targets[(size_t)2 * n + i];
+    refs(tref);
     yaw_out = yaw;
     speed_out = sqrtf(vbx * vbx + vby * vby + vbz * vbz);
     if (o == nullptr) return;
@@ -749,6 +751,13 @@ __device__ __forceinline__ void fw_write_obs_lowlevel(const FwPlanes& pl, const 
 #pragma unroll
     for (int c = 0; c < 6; ++c) o[k++] = a[c];
     o[k++] = tref[0]; o[k++] = tref[1]; o[k++] = tref[2];
+}
+
+__device__ __forceinline__ void fw_write_obs_lowlevel(const FwPlanes& pl, const EnvState& e, int i, int n, const float a[6],
+                                                      float* o, float& yaw_out, float& speed_out, float tref[3]) {
+    fw_write_obs_tracking(e, a, [&](float* t) {
+        t[0] = pl.targets[(size_t)0 * n + i]; t[1] = pl.targets[(size_t)1 * n + i]; t[2] = pl.targets[(size_t)2 * n + i];
+    }, o, yaw_out, speed_out, tref);
 }
 
 // end_reset: warmup_substeps substeps at zero setpoint.  Kept out of line: it is the rare path (only when a wind

@@ -21,6 +21,7 @@
 #include "fw_objlock.cuh"
 #include "fw_pack.cuh"
 #include "fw_kernels.h"
+#include "ppo_tower.cuh"
 
 #include <cstdlib>
 #include <cstring>
@@ -310,6 +311,209 @@ fw_step_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const float4*
             fw_flush_obs(obs, stage_warp, D, first_env, p.i_end, lane, bulk_ok != 0,
                          (!RANDOM_ACT && pl.obs_acc != nullptr) ? pl.obs_acc + (size_t)(blockIdx.x & (FW_OBS_ACC_SLOTS - 1)) * 2 * D : nullptr);
     }
+}
+
+// ================================================================== K1h: high-level waypoints (task 5)
+// The Waypoints episode flown through a frozen low-level tracker.  The agent's action is a command [psi, h, V]; every inner
+// iteration (120 Hz) the tracker policy turns the command and the current state into a six-channel surface / thrust
+// command (Fixedwing mode -1, the low-level env's rate and order), then one Aviary.step runs, then the Waypoints head.
+// The tower is the CUDA-core forward of ppo_tower.cuh: weights and normalisation constants staged in shared memory once
+// per CTA, the hidden vector in shared memory, one thread per env.
+#define FW_HL_BLOCK 128
+// 3 resident CTAs/SM: 3 x (27 KB tower + 128 x (64 hidden + obs_dim staging) floats) fits the 228 KB of an SM
+#ifndef FW_HL_MIN_BLOCKS
+#define FW_HL_MIN_BLOCKS 3
+#endif
+#define FW_TRK_DP 32          // tracker observation padded for float4 weight rows (ppo_forward_kernel's DP for 21 floats)
+
+// The command of high-level action a: psi = atan2(a1, a0), h and V mapped from [-1, 1] onto the tracker's ranges.
+__device__ __forceinline__ void fw_hl_command(const FwTrk& trk, float a0, float a1, float a2, float a3, float tref[3]) {
+    tref[0] = atan2f(a1, a0);
+    tref[1] = trk.h_lo + (fminf(fmaxf(a2, -1.f), 1.f) + 1.0f) * 0.5f * (trk.h_hi - trk.h_lo);
+    tref[2] = trk.v_lo + (fminf(fmaxf(a3, -1.f), 1.f) + 1.0f) * 0.5f * (trk.v_hi - trk.v_lo);
+}
+
+// fw_env_step<1> with the tracker between the agent's action and the physics.  prev: the tracker's previous action
+// (zeroed by the auto-reset); trow: this thread's scratch row of >= 21 floats holding the raw tracker observation of the
+// last decision when the function returns.
+template <bool STD, bool FIELD>
+__device__ __forceinline__ float fw_env_step_highlevel(const FwDev& p, const FwPlanes& pl, const FwTrk& trk, const float* s_pi,
+                                                       const float* s_mean, const float* s_istd, float* hbuf, float* trow,
+                                                       EnvState& e, int i, uint32_t gid, float a0, float a1, float a2, float a3,
+                                                       float (&prev)[FW_TRK_ACT], const float4& w0_in, const float4& w1_in,
+                                                       float& ep_ret, float* row, float* term_obs_row, uint32_t& bits,
+                                                       int& tidx_info) {
+    float4 w0 = w0_in, w1 = w1_in;
+    const bool fault_in = !fw_state_finite(e);
+    float reward = -0.1f;
+    bool term = false, trunc = false, col = false, oob = false, complete = false;
+    float tref[3];
+    fw_hl_command(trk, a0, a1, a2, a3, tref);
+    float n0 = 0.f, n1 = 0.f, n2 = 0.f, n3 = 0.f;
+    bool have_noise = false;
+    int obs_tidx = e.tidx;
+
+    for (int it = 0; it < p.inner_per_step; ++it) {
+        if (term || trunc) break;
+        // tracker decision: fw_write_obs_lowlevel's observation with the commanded refs, VecNormalize, policy mean, clip
+        float yaw, speed, tr[3];
+        fw_write_obs_tracking(e, prev, [&](float* t) { t[0] = tref[0]; t[1] = tref[1]; t[2] = tref[2]; }, trow, yaw, speed, tr);
+        float x[FW_TRK_DP];
+        load_obs<FW_TRK_DP>(trow, trk.stats != nullptr ? s_mean : nullptr, s_istd, trk.clip, FW_TRK_OBS, 0, x, nullptr);
+        float mu[FW_TRK_ACT];
+        tower_forward<FW_TRK_ACT, FW_TRK_DP>(s_pi, x, hbuf, mu);
+        float cmd[6];
+#pragma unroll
+        for (int c = 0; c < FW_TRK_ACT; ++c) { cmd[c] = ppo_clip_action(mu[c]); prev[c] = cmd[c]; }   // mode -1: cmd = action
+        bool contact = false;
+        for (int s = 0; s < p.substeps_per_inner; ++s) {
+            const int ps = e.physics_steps;
+            float nz = 0.0f;
+            if (p.noise_ratio > 0.0f) {
+                if (!have_noise || (ps & 3) == 0) {
+                    float nn[4];
+                    fw_normals4(p, gid, e.episode, (uint32_t)ps >> 2, nn);
+                    n0 = nn[0]; n1 = nn[1]; n2 = nn[2]; n3 = nn[3];
+                    have_noise = true;
+                }
+                const int q = ps & 3;
+                nz = q == 0 ? n0 : (q == 1 ? n1 : (q == 2 ? n2 : n3));
+            }
+            fw_substep_wind<STD, FIELD>(p, e, cmd, w0, w1, nz, contact);
+        }
+        // the Waypoints head of fw_env_step
+        float old_dist = e.new_dist;
+        obs_tidx = e.tidx;
+        if (e.tidx < p.num_targets) {
+            float dx = pl.targets[(size_t)(e.tidx * 3 + 0) * p.n + i] - e.px;
+            float dy = pl.targets[(size_t)(e.tidx * 3 + 1) * p.n + i] - e.py;
+            float dz = pl.targets[(size_t)(e.tidx * 3 + 2) * p.n + i] - e.pz;
+            e.new_dist = sqrtf(dx * dx + dy * dy + dz * dz);
+        }
+        if (e.step_count > p.max_steps) trunc = true;
+        if (contact) { reward = -100.0f; col = true; term = true; }
+        if (e.px * e.px + e.py * e.py + e.pz * e.pz > p.dome2) { reward = -100.0f; oob = true; term = true; }
+        if (e.tidx < p.num_targets && !(p.early_return_on_crash && (col || oob))) {
+            if (!p.sparse_reward) {
+                reward += fmaxf(3.0f * (old_dist - e.new_dist), 0.0f);
+                reward += 1.0f / e.new_dist;
+            }
+            if (e.new_dist < p.goal_reach) {
+                reward = 100.0f;
+                e.tidx += 1;
+                const bool all = e.tidx >= p.num_targets;
+                if (p.complete_truncates && all) trunc = true;
+            }
+        }
+    }
+    e.step_count += 1;
+    complete = e.tidx >= p.num_targets;
+    tidx_info = e.tidx;
+    const bool fault = fault_in || !fw_state_finite(e);
+    if (fault) { term = true; trunc = false; col = false; oob = false; reward = 0.0f; }
+    // the raw observation of the step's last tracker decision, before `row` (which may share trow's memory) is written
+    if (trk.obs_out != nullptr)
+        for (int k = 0; k < FW_TRK_OBS; ++k) trk.obs_out[(size_t)i * FW_TRK_OBS + k] = trow[k];
+
+    const bool done = term || trunc;
+    if (row != nullptr) fw_write_obs(p, pl, e, i, obs_tidx, a0, a1, a2, a3, row);
+    ep_ret += reward;
+    if (done) {
+        if (term_obs_row != nullptr && !fault)
+            for (int k = 0; k < p.obs_dim; ++k) term_obs_row[k] = row[k];
+        if (fault) atomicAdd(&pl.stats[8], 1.0);
+        atomicAdd(&pl.stats[0], 1.0);
+        atomicAdd(&pl.stats[1], (double)ep_ret);
+        atomicAdd(&pl.stats[2], (double)e.step_count);
+        atomicAdd(&pl.stats[3], (double)e.tidx);
+        if (col) atomicAdd(&pl.stats[4], 1.0);
+        if (oob) atomicAdd(&pl.stats[5], 1.0);
+        if (complete) atomicAdd(&pl.stats[6], 1.0);
+        fw_reset_env<FIELD>(p, pl, e, i, gid, e.episode + 1u);
+#pragma unroll
+        for (int c = 0; c < FW_TRK_ACT; ++c) prev[c] = 0.0f;
+        if (row != nullptr) fw_write_obs(p, pl, e, i, 0, 0.f, 0.f, 0.f, 0.f, row);
+        if (fault && term_obs_row != nullptr)
+            for (int k = 0; k < p.obs_dim; ++k) term_obs_row[k] = row[k];
+        ep_ret = 0.0f;
+    }
+    bits = (term ? 1u : 0u) | (trunc ? 2u : 0u) | (col ? 4u : 0u) | (oob ? 8u : 0u) | (complete ? 16u : 0u) | (fault ? 64u : 0u);
+    return reward;
+}
+
+// smem: [policy tower][mean 32][istd 32][hidden: 64 x FW_HL_BLOCK][observation staging: FW_HL_BLOCK x obs_dim].  A thread's
+// staging row doubles as its tracker-observation row until the step's own observation is written (obs_dim >= 22 > 21).
+static inline size_t hl_smem_bytes(const FwDev& p) {
+    return (size_t)(TowerOff<FW_TRK_ACT, FW_TRK_DP>::SIZE + 2 * FW_TRK_DP + PPO_H * FW_HL_BLOCK + FW_HL_BLOCK * p.obs_dim) * 4;
+}
+
+template <bool RANDOM_ACT, bool STD, bool FIELD>
+__global__ void __launch_bounds__(FW_HL_BLOCK, FW_HL_MIN_BLOCKS)
+fw_step_highlevel_kernel(const __grid_constant__ FwDev p, const FwPlanes pl, const FwTrk trk, const float4* __restrict__ act,
+                         float* __restrict__ obs, float* __restrict__ rew, uint8_t* __restrict__ flg,
+                         float* __restrict__ term_obs, int bulk_ok) {
+    extern __shared__ __align__(128) float smem[];
+    float* s_pi = smem;
+    float* s_mean = s_pi + TowerOff<FW_TRK_ACT, FW_TRK_DP>::SIZE;
+    float* s_istd = s_mean + FW_TRK_DP;
+    float* hbuf = s_istd + FW_TRK_DP;
+    float* stage = hbuf + PPO_H * FW_HL_BLOCK;
+    load_tower<FW_TRK_ACT, FW_TRK_DP>(s_pi, trk.params, FW_TRK_OBS);
+    stage_stats<FW_TRK_DP>(trk.stats, FW_TRK_OBS, s_mean, s_istd);
+    __syncthreads();
+
+    const int i = p.i_begin + blockIdx.x * FW_HL_BLOCK + threadIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int D = p.obs_dim;
+    float* stage_warp = stage + (size_t)warp * 32 * D;
+    float* trow = stage_warp + (size_t)lane * D;
+    float* row = obs != nullptr ? trow : nullptr;
+
+    if (i < p.i_end) {
+        const uint32_t gid = p.env_id0 + (uint32_t)i;
+        EnvState e;
+        fw_load(pl, i, e);
+        float4 w0 = make_float4(0.f, 0.f, 0.f, 0.f), w1 = w0;
+        if (p.wind_mode != 0) { w0 = pl.w0[i]; w1 = pl.w1[i]; }
+        float ep_ret = pl.ep_ret[i];
+        float prev[FW_TRK_ACT];
+#pragma unroll
+        for (int c = 0; c < FW_TRK_ACT; ++c) prev[c] = trk.prev[(size_t)c * p.n + i];
+        float a0, a1, a2, a3;
+        if (RANDOM_ACT) {
+            uint4 r = fw_philox(p.seed_lo, p.seed_hi, gid, e.episode, (uint32_t)e.step_count, FWD_STREAM_ACTION);
+            a0 = 2.0f * fw_u01(r.x) - 1.0f; a1 = 2.0f * fw_u01(r.y) - 1.0f;
+            a2 = 2.0f * fw_u01(r.z) - 1.0f; a3 = 2.0f * fw_u01(r.w) - 1.0f;
+        } else {
+            const float4 a = act[i];
+            a0 = a.x; a1 = a.y; a2 = a.z; a3 = a.w;
+        }
+        uint32_t bits = 0u;
+        int tidx_info = 0;
+        const float reward = fw_env_step_highlevel<STD, FIELD>(
+            p, pl, trk, s_pi, s_mean, s_istd, hbuf, trow, e, i, gid, a0, a1, a2, a3, prev, w0, w1, ep_ret, row,
+            (term_obs != nullptr && row != nullptr) ? term_obs + (size_t)i * D : nullptr, bits, tidx_info);
+#pragma unroll
+        for (int c = 0; c < FW_TRK_ACT; ++c) trk.prev[(size_t)c * p.n + i] = prev[c];
+        pl.ep_ret[i] = ep_ret;
+        fw_store(pl, i, e);
+        if (rew != nullptr) rew[i] = reward;
+        if (flg != nullptr) flg[i] = (uint8_t)bits;
+        if (!RANDOM_ACT && pl.tidx_out != nullptr) pl.tidx_out[i] = (uint8_t)tidx_info;
+    }
+    if (obs != nullptr) {
+        const int first_env = p.i_begin + blockIdx.x * FW_HL_BLOCK + warp * 32;
+        if (first_env < p.i_end)
+            fw_flush_obs(obs, stage_warp, D, first_env, p.i_end, lane, (bulk_ok & 1) != 0,
+                         (!RANDOM_ACT && pl.obs_acc != nullptr) ? pl.obs_acc + (size_t)(blockIdx.x & (FW_OBS_ACC_SLOTS - 1)) * 2 * D : nullptr);
+    }
+}
+
+__global__ void __launch_bounds__(256) fw_tracker_clear_kernel(const uint8_t* __restrict__ mask, float* __restrict__ prev, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || (mask != nullptr && mask[i] == 0)) return;
+#pragma unroll
+    for (int c = 0; c < FW_TRK_ACT; ++c) prev[(size_t)c * n + i] = 0.0f;
 }
 
 // ================================================================== K1p: two environments per thread (fw_pack.cuh)
@@ -1140,6 +1344,7 @@ static inline size_t stage_bytes(const FwDev& p) {
 static inline int grid_for(int n) { return (n + FW_BLOCK - 1) / FW_BLOCK; }
 
 typedef void (*fw_step_fn)(const FwDev, const FwPlanes, const float4*, float*, float*, uint8_t*, float*, int, int);
+typedef void (*fw_hl_fn)(const FwDev, const FwPlanes, const FwTrk, const float4*, float*, float*, uint8_t*, float*, int);
 
 // a step kernel with its launch geometry
 struct StepLaunch {
@@ -1214,8 +1419,30 @@ static bool smem_opt_in(const void* fn, size_t bytes) {
     return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess;
 }
 
+// the task-5 kernel of a handle: wind field or not, standard layout or not
+static fw_hl_fn hl_step_fn(const FwDev& p, bool random_act) {
+    const bool sg = p.std_geom != 0, r = random_act;
+    if (p.wind_mode == 3)
+        return sg ? (r ? fw_step_highlevel_kernel<true, true, true> : fw_step_highlevel_kernel<false, true, true>)
+                  : (r ? fw_step_highlevel_kernel<true, false, true> : fw_step_highlevel_kernel<false, false, true>);
+    return sg ? (r ? fw_step_highlevel_kernel<true, true, false> : fw_step_highlevel_kernel<false, true, false>)
+              : (r ? fw_step_highlevel_kernel<true, false, false> : fw_step_highlevel_kernel<false, false, false>);
+}
+
 cudaError_t fwk_launch_step(const FwDev& p, const FwPlanes& pl, const float* act, float* obs, float* rew, uint8_t* flg,
-                            float* term_obs, bool random_act, int spl, cudaStream_t st) {
+                            float* term_obs, bool random_act, int spl, cudaStream_t st, const FwTrk* trk) {
+    if (p.task == 5) {
+        if (trk == nullptr || trk->params == nullptr) return cudaErrorInvalidValue;
+        const fw_hl_fn fn = hl_step_fn(p, random_act);
+        const size_t smem = hl_smem_bytes(p);
+        if (!smem_opt_in((const void*)fn, smem)) return cudaErrorInvalidValue;
+        const int bulk_ok = (obs != nullptr) && ((reinterpret_cast<uintptr_t>(obs) & 15u) == 0) && ((p.obs_dim * 32 * 4) % 16 == 0) &&
+                            (((size_t)p.i_begin * p.obs_dim * 4) % 16 == 0);
+        const int n = p.i_end - p.i_begin;
+        fn<<<(n + FW_HL_BLOCK - 1) / FW_HL_BLOCK, FW_HL_BLOCK, smem, st>>>(p, pl, *trk, reinterpret_cast<const float4*>(act), obs, rew,
+                                                                       flg, term_obs, bulk_ok);
+        return cudaGetLastError();
+    }
     const StepLaunch L = step_launch(p, random_act);
     if (L.fn == nullptr) return cudaErrorNotSupported;
     // the bulk store of a warp's observation rows needs a 16-byte aligned destination and size
@@ -1325,6 +1552,11 @@ cudaError_t fwk_launch_reset(const FwDev& p, const FwPlanes& pl, const uint8_t* 
         auto fn = field ? fw_reset_kernel<true> : fw_reset_kernel<false>;
         fn<<<grid_for(p.n), FW_BLOCK, stage_bytes(p), st>>>(p, pl, mask, obs, bulk_ok, emit_only ? 1 : 0);
     }
+    return cudaGetLastError();
+}
+
+cudaError_t fwk_launch_tracker_clear(const uint8_t* mask, float* prev, int n, cudaStream_t st) {
+    fw_tracker_clear_kernel<<<(n + 255) / 256, 256, 0, st>>>(mask, prev, n);
     return cudaGetLastError();
 }
 

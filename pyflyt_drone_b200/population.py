@@ -189,7 +189,7 @@ class PPOPopulation:
     def _rollout_body(self) -> None:
         env, b, lib, P, n = self.env, self.buf, self.lib, self.P, self.n
         fwd = lib.ppo_pop_policy_forward_tc_a if self.tensor_core_forward else lib.ppo_pop_policy_forward_a
-        has_targets = env.cfg.task in (1, 2)
+        has_targets = env.cfg.task in (1, 2, 5)
         for t in range(self.n_steps):
             _lib.check(fwd(P, n, _p(self.seeds), _p(self.theta), self.d, self.a, _p(self._obs), self._stats_ptr(), self.clip_obs,
                            env.env_id0, t, _p(self._step_dev), 0, _p(b["obs"][t]), _p(self.act_env), _p(b["act"][t]),
@@ -318,7 +318,8 @@ class PPOPopulation:
         """A fresh env batch equal to member k's slice: the same config, wind field and env seed, env ids from env_id0 + k * n."""
         from .vec_env import FixedwingVecEnv
         return FixedwingVecEnv(self.n, config=self.env.cfg, device=self.env.device_index, seed=self.env._seed,
-                               env_id0=self.env.env_id0 + k * self.n, wind_field=getattr(self.env, "wind_field", None))
+                               env_id0=self.env.env_id0 + k * self.n, wind_field=getattr(self.env, "wind_field", None),
+                               tracker=getattr(self.env, "tracker", None))
 
     def member(self, k: int, env=None) -> PPO:
         """A standalone ``PPO`` holding copies of member k's state: hyper-parameters, parameters, Adam moments and step,

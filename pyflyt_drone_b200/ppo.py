@@ -260,7 +260,7 @@ class EvalResult:
 
     @property
     def has_targets(self) -> bool:
-        return self.task in (1, 2)
+        return self.task in (1, 2, 5)
 
     @property
     def n_episodes(self) -> int:
@@ -285,7 +285,7 @@ class EvalResult:
         lengths = np.asarray(lengths, np.int32)[order]
         targets_reached = np.asarray(targets_reached, np.uint8)[order]
         flags = np.asarray(flags, np.uint8)[order]
-        has_targets = task in (1, 2)
+        has_targets = task in (1, 2, 5)
         if not has_targets:
             targets_reached = np.zeros_like(targets_reached)
         nt = int(num_targets) if has_targets else 0
@@ -774,14 +774,15 @@ class PPO:
         if own:
             n = max(1, min(self.n_envs, int(n_eval_episodes)))
             env = FixedwingVecEnv(n, config=self.env.cfg, device=self.env.device_index, seed=self.seed + 7919,
-                                  env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None))
+                                  env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None),
+                                  tracker=getattr(self.env, "tracker", None))
         obs = env.reset_tensor()
         n = env.num_envs
         quota = torch.tensor(self.episode_quotas(n_eval_episodes, n), dtype=torch.int64, device=self.device)
         count = torch.zeros(n, dtype=torch.int64, device=self.device)
         ret = torch.zeros(n, dtype=torch.float64, device=self.device)
         length = torch.zeros(n, dtype=torch.int64, device=self.device)
-        has_targets = env.cfg.task in (1, 2)
+        has_targets = env.cfg.task in (1, 2, 5)
         done_ret, done_len, done_tr = [], [], []
         # every env needs at most quota episodes of at most max_steps + 2 steps
         limit = max_steps if max_steps is not None else (int(quota.max()) * (int(env.cfg.max_steps) + 2) + 8)
@@ -815,10 +816,12 @@ class PPO:
 
     def make_eval_env(self, n_eval_episodes: int) -> FixedwingVecEnv:
         """The batch ``evaluate`` builds when given no env: the training env's configuration (and wind field) on a fresh batch
-        of at most ``n_eval_episodes`` envs, seed ``seed + 7919``, env ids from ``env_id0 + 2**24`` -- ``evaluate_policy``'s."""
+        of at most ``n_eval_episodes`` envs, seed ``seed + 7919``, env ids from ``env_id0 + 2**24`` -- ``evaluate_policy``'s.
+        A high-level waypoint env (task 5) carries its tracker over as well."""
         n = max(1, min(self.n_envs, int(n_eval_episodes)))
         return FixedwingVecEnv(n, config=self.env.cfg, device=self.env.device_index, seed=self.seed + 7919,
-                               env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None))
+                               env_id0=self.env.env_id0 + (1 << 24), wind_field=getattr(self.env, "wind_field", None),
+                               tracker=getattr(self.env, "tracker", None))
 
     def evaluate(self, env=None, n_eval_episodes: int = 100, deterministic: bool = True,
                  max_steps: int | None = None) -> EvalResult:
@@ -907,7 +910,7 @@ class PPO:
                                                 self.vecnorm.clip_obs, n, seed, env.env_id0 & 0xFFFFFFFF, k, _p(s["step"]),
                                                 int(deterministic), None, _p(s["act"]), None, None, _p(s["val"]), _stream()))
             _, rew, flags = env.step_tensor(s["act"])
-            if env.cfg.task in (1, 2):
+            if env.cfg.task in (1, 2, 5):
                 tidx = env.targets_reached_tensor()
             _lib.check(lib.ppo_eval_ledger(_p(rew), _p(flags), _p(tidx), n, _p(s["ret"]), _p(s["len"]), _p(s["count"]),
                                            _p(s["quota"]), _p(s["offset"]), k, _p(s["step"]), limit, _p(s["remaining"]),
@@ -956,13 +959,11 @@ class PPO:
     def import_sb3(self, directory: str) -> "PPO":
         """Inverse of export_sb3.  Also takes what SB3 itself wrote: ``final_model.zip`` / ``best_model.zip`` (``model.save``)
         and ``vecnorm.pkl`` (``VecNormalize.save``) of the reference's training runs, or a bare ``policy.pth``."""
-        import os
         from . import sb3_io
-        zips = [f for f in ("final_model.zip", "best_model.zip", "model.zip") if os.path.exists(os.path.join(directory, f))]
-        if zips:
-            ck = sb3_io.read_model_zip(os.path.join(directory, zips[0]))
-            self.policy.load_state_dict(ck["policy"])
-            for i, st in ck.get("optimizer", {}).get("state", {}).items():          # Adam moments, SB3 parameter order
+        ck = sb3_io.read_directory(directory)
+        self.policy.load_state_dict(ck["policy"])
+        if "optimizer" in ck:
+            for i, st in ck["optimizer"].get("state", {}).items():                 # Adam moments, SB3 parameter order
                 key = sb3_io.SB3_PARAM_ORDER[int(i)]
                 base, _, leaf = key.rpartition(".")
                 m = {"mlp_extractor.policy_net.0": "pi.0", "mlp_extractor.policy_net.2": "pi.2",
@@ -971,14 +972,8 @@ class PPO:
                 self._adam_m[a:b] = st["exp_avg"].reshape(-1).to(self.device)
                 self._adam_v[a:b] = st["exp_avg_sq"].reshape(-1).to(self.device)
                 self._adam_t.fill_(int(float(st["step"])))
-        else:
-            sd = torch.load(os.path.join(directory, "policy.pth"), map_location="cpu", weights_only=True)
-            self.policy.load_state_dict(sd)
-        pkl, npz = os.path.join(directory, "vecnorm.pkl"), os.path.join(directory, "vecnorm.npz")
-        if os.path.exists(pkl):
-            self.vecnorm.load_state_dict(sb3_io.read_vecnorm_pkl(pkl))
-        elif os.path.exists(npz):
-            self.vecnorm.load_state_dict(import_vecnorm_npz(npz))
+        if "vecnorm" in ck:
+            self.vecnorm.load_state_dict(ck["vecnorm"])
         return self
 
     def get_parameters(self) -> dict:

@@ -232,3 +232,26 @@ def read_vecnorm_pkl(path: str) -> dict:
             "ret_rms.var": float(np.asarray(g["ret_rms"].var)), "ret_rms.count": float(g["ret_rms"].count),
             "clip_obs": float(g["clip_obs"]), "clip_reward": float(g["clip_reward"]), "gamma": float(g["gamma"]),
             "norm_obs": bool(g.get("norm_obs", True)), "norm_reward": bool(g.get("norm_reward", True))}
+
+
+def read_directory(directory: str) -> dict:
+    """What ``PPO.export_sb3`` writes, or what SB3 itself wrote: ``policy`` (state dict) and ``optimizer`` from the first of
+    ``final_model.zip`` / ``best_model.zip`` / ``model.zip`` (else ``policy`` from a bare ``policy.pth``), and ``vecnorm``
+    (``DeviceVecNormalize.load_state_dict`` layout) from ``vecnorm.pkl`` or ``vecnorm.npz`` when one exists."""
+    import os
+    out = {}
+    zips = [f for f in ("final_model.zip", "best_model.zip", "model.zip") if os.path.exists(os.path.join(directory, f))]
+    if zips:
+        ck = read_model_zip(os.path.join(directory, zips[0]))
+        out["policy"] = ck["policy"]
+        if "optimizer" in ck:
+            out["optimizer"] = ck["optimizer"]
+    else:
+        out["policy"] = torch.load(os.path.join(directory, "policy.pth"), map_location="cpu", weights_only=True)
+    pkl, npz = os.path.join(directory, "vecnorm.pkl"), os.path.join(directory, "vecnorm.npz")
+    if os.path.exists(pkl):
+        out["vecnorm"] = read_vecnorm_pkl(pkl)
+    elif os.path.exists(npz):
+        from .ppo import import_vecnorm_npz
+        out["vecnorm"] = import_vecnorm_npz(npz)
+    return out

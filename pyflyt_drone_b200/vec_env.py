@@ -24,6 +24,7 @@ from .compat import spaces
 from .compat.vec_env import VecEnv
 from .config import (EnvConfig, FLAG_COLLISION, FLAG_COMPLETE, FLAG_FAULT, FLAG_OOB, FLAG_STRIKE, FLAG_TERM, FLAG_TRUNC,
                      make_config)
+from .tracker import Tracker
 from .wind import WindField
 
 _STATE_FIELDS = {
@@ -51,7 +52,7 @@ class FixedwingVecEnv(VecEnv):
 
     def __init__(self, num_envs: int, preset: str = "waypoints_v3", config: EnvConfig | None = None,
                  device: int = 0, seed: int = 0, env_id0: int = 0, info_mode: str = "auto", wind_field: WindField | None = None,
-                 **overrides):
+                 tracker: Tracker | None = None, **overrides):
         self.cfg = config if config is not None else make_config(preset, **overrides)
         if config is not None and overrides:
             self.cfg = self.cfg.replace(**overrides)
@@ -63,6 +64,13 @@ class FixedwingVecEnv(VecEnv):
         elif self.cfg.wind_mode == 3:
             raise ValueError("wind_mode 3 (gridded field) needs wind_field=WindField(...)")
         self.wind_field = wind_field
+        # high-level waypoints (task 5): the frozen low-level tracker, installed by _open() like the wind field
+        if tracker is not None and not isinstance(tracker, Tracker):
+            raise TypeError("tracker must be a pyflyt_drone_b200.tracker.Tracker")
+        if (tracker is not None) != (self.cfg.task == 5):
+            raise ValueError("task 5 (high-level waypoints) needs tracker=Tracker(...), and only task 5 takes one")
+        self.tracker = tracker
+        self._trk_obs = None
         self.num_envs = int(num_envs)
         self.device_index = int(device)
         self._seed = int(seed)
@@ -89,6 +97,16 @@ class FixedwingVecEnv(VecEnv):
         if self.wind_field is not None:
             desc = self.wind_field.to_c()
             rc = self.lib.fw_set_wind_field(self._h, C.byref(desc))
+            if rc != 0:
+                msg = self.lib.fw_last_error()
+                self.lib.fw_destroy(self._h)
+                self._h = C.c_void_p()
+                raise _lib.FwError(f"libfwsim error {rc}: {msg.decode() if msg else '?'}")
+        if self.tracker is not None:
+            desc = self.tracker.to_c()
+            rc = self.lib.fw_set_tracker(self._h, C.byref(desc))
+            if rc == 0 and self._trk_obs is not None:
+                rc = self.lib.fw_set_tracker_obs_buffer(self._h, C.c_void_p(self._trk_obs.data_ptr()))
             if rc != 0:
                 msg = self.lib.fw_last_error()
                 self.lib.fw_destroy(self._h)
@@ -188,7 +206,7 @@ class FixedwingVecEnv(VecEnv):
         one WaypointEvalCallback._log_success_callback reads on every done (train_Fixedwing_Waypoints_v3.py:136-138).
         ``info_mode="lazy"`` (default above 4,096 envs) builds full dicts for finished envs only; the others share one
         blank dict, and the per-env values stay available as arrays (``last_flags``, ``last_targets_reached``)."""
-        has_t = self.cfg.task in (1, 2)
+        has_t = self.cfg.task in (1, 2, 5)
         tr = self._h_tidx
         idx = np.nonzero(dones)[0]
         if self.info_mode == "lazy":
@@ -344,6 +362,29 @@ class FixedwingVecEnv(VecEnv):
         if acc is not None and (acc.numel() != 64 * 2 * self.obs_dim or str(acc.dtype) != "torch.float64" or not acc.is_cuda):
             raise ValueError("accumulator must be a CUDA float64 tensor of 64 * 2 * obs_dim elements")
         _lib.check(self.lib.fw_set_obs_accumulator(self._h, C.c_void_p(acc.data_ptr()) if acc is not None else None))
+
+    # ------------------------------------------------------------------ high-level waypoints (task 5)
+    def get_tracker_state(self) -> np.ndarray:
+        """The tracker's previous action of every env, [num_envs, 6] float32 (synchronous)."""
+        out = np.zeros((self.num_envs, 6), np.float32)
+        _lib.check(self.lib.fw_get_tracker_state(self._h, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def set_tracker_state(self, prev: np.ndarray) -> None:
+        """Overwrite the tracker's previous action of every env ([num_envs, 6]; parity injection)."""
+        a = np.ascontiguousarray(np.asarray(prev, dtype=np.float32))
+        if a.shape != (self.num_envs, 6):
+            raise ValueError(f"tracker state must have shape ({self.num_envs}, 6), got {a.shape}")
+        _lib.check(self.lib.fw_set_tracker_state(self._h, a.ctypes.data_as(C.c_void_p)))
+
+    def set_tracker_obs_buffer(self, buf) -> None:
+        """CUDA float32 tensor [num_envs, 21] (or None): every step enqueued from now on writes the raw tracker observation of
+        each env's last tracker decision of the step into it (``fw_set_tracker_obs_buffer``).  Kept across ``seed()``."""
+        if buf is not None and (tuple(buf.shape) != (self.num_envs, 21) or str(buf.dtype) != "torch.float32" or not buf.is_cuda
+                                or not buf.is_contiguous()):
+            raise ValueError("tracker observation buffer must be a contiguous CUDA float32 tensor of shape (num_envs, 21)")
+        _lib.check(self.lib.fw_set_tracker_obs_buffer(self._h, C.c_void_p(buf.data_ptr()) if buf is not None else None))
+        self._trk_obs = buf
 
     def render_layers(self, env_index: int = 0, width: int | None = None, height: int | None = None) -> dict:
         """Debug / evaluation frame of one env (``fw_render``): ``rgba`` uint8 [H,W,4], ``seg`` int32 [H,W] (-1 sky, 0 ground,
